@@ -22,12 +22,17 @@ a single-GPU render of the same sample set on rank 0 (`parity_check`).
                host cores on a bounded sample of the same scene
 
 `--impl reference` times the reference's own CPU implementation instead (same metric / config keys).
+`--dump-outputs DIR` writes the per-pixel sums of the last timed step to DIR (fixed seed and scene: two builds run with
+the same arguments can be compared output for output).
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -68,15 +73,46 @@ def emit(obj):
         os.write(_RESULT_FD, line)
 
 
+_SCENE_DIR = None
+
+
 def scene_path(name):
-    """Deterministic synthetic scene, generated on first use (one private copy per rank: no write races)."""
+    """Deterministic synthetic scene, generated on first use into a temporary directory of this process (the tree
+    may be read-only; one private copy per rank: no write races), removed at exit."""
+    global _SCENE_DIR
     import gen_gltf
 
-    d = os.path.join(ROOT, "scenes", "cache", "rank" + os.environ.get("RANK", "0"))
-    p = os.path.join(d, name + ".gltf")
+    if _SCENE_DIR is None:
+        _SCENE_DIR = tempfile.mkdtemp(prefix="rt_b200_scenes_")
+        atexit.register(shutil.rmtree, _SCENE_DIR, ignore_errors=True)
+    p = os.path.join(_SCENE_DIR, name + ".gltf")
     if not os.path.exists(p):
-        gen_gltf.generate(name, d)
+        gen_gltf.generate(name, _SCENE_DIR)
     return p
+
+
+DUMP_BYTES = 64 * 10**6  # all files of the dump, .npy headers included
+NPY_HEADER_MAX = 4096  # room left per file for its .npy header (128 bytes in practice)
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, sums, w, h):
+    """The per-pixel float sums the timed path returned (W*H*4 float32: rgb + unused w) as accum_sums.npy [H, W, 4].
+    Above DUMP_BYTES a fixed, seeded sample of the pixels is written instead: accum_sums.npy [k, 4] and the row-major
+    pixel index of each row in accum_pixel_index.npy."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    sums = np.ascontiguousarray(sums, np.float32).reshape(h, w, 4)
+    if sums.nbytes + NPY_HEADER_MAX <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "accum_sums.npy"), sums)
+        log(f"dump-outputs: accum_sums.npy {sums.shape} -> {out_dir}")
+        return
+    k = (DUMP_BYTES - 2 * NPY_HEADER_MAX) // (sums.itemsize * 4 + 8)  # + one float64 pixel index per row
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(w * h, size=k, replace=False))
+    np.save(os.path.join(out_dir, "accum_sums.npy"), sums.reshape(-1, 4)[idx])
+    np.save(os.path.join(out_dir, "accum_pixel_index.npy"), idx.astype(np.float64))
+    log(f"dump-outputs: {k} of {w * h} pixels (seed {DUMP_SEED}) -> {out_dir}")
 
 
 class ClockSampler:
@@ -277,7 +313,7 @@ def run_gpu_arm(args, rank, world, local_rank):
     rays = [0, 0]
     e0.record()
     for i in range(args.steps):
-        step(i)
+        sums = step(i)
         st = rt.stats()
         launches += st["kernel_launches"] + (1 if world > 1 else 0)
         rays[0] += st["extension_rays"]
@@ -293,6 +329,8 @@ def run_gpu_arm(args, rank, world, local_rank):
     total_ms = float(ms.item())
     samples_all = float(w) * h * spp_total * args.steps
     value = samples_all / (total_ms * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:  # the reduced sums of the last timed step, before anything renders again
+        dump_outputs(args.dump_outputs, sums.cpu().numpy(), w, h)
 
     # the N-rank image of the last timed step, for the parity check below
     img_n = rt.readback()[0] if (rank == 0 and world > 1) else None
@@ -439,7 +477,13 @@ def main():
     ap.add_argument("--config", default="c4", choices=["c4", "c5"], help="BASELINE config 4 (default) or 5")
     ap.add_argument("--paths", type=int, default=0, help="paths in flight per batch (0 = library default)")
     ap.add_argument("--cpu-budget", type=float, default=15.0, help="seconds of CPU work for cpu_baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the per-pixel sums of the last timed step to DIR/*.npy (same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the GPU path (--impl b200)")
     if args.config == "c5":
         args.width, args.height = 3840, 2160
     if args.spp is None:

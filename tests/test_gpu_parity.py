@@ -369,9 +369,10 @@ def _read_ppm(path):
     return np.frombuffer(rest, np.uint8).reshape(h, w, 3)
 
 
-def test_cli_drop_in_matches_reference_binary(scene_dir, tmp_path):
+def test_cli_drop_in_matches_reference_binary(scene_dir, tmp_path, manifest):
     """Same CLI, same PPM: the reference-hosted drop-in (reference loader + BVH + Image, GPU integrator) and
-    the Python CLI against the unmodified reference binary on the same scene / size / spp."""
+    the Python CLI against the unmodified reference on the same scene / size: its tonemapped 16 384-spp render
+    (tests/golden/tiny_refhi_a.f32) and, where it was built, the reference binary at the same spp."""
     import subprocess
     from conftest import ROOT
     from rt_b200 import cli
@@ -379,6 +380,8 @@ def test_cli_drop_in_matches_reference_binary(scene_dir, tmp_path):
     exe = os.path.join(ROOT, "bin", "raytracer_b200")
     gltf_path = scene_dir("tiny")
     w, h, spp = 64, 48, 4096
+    assert (manifest["scenes"]["tiny"]["width"], manifest["scenes"]["tiny"]["height"]) == (w, h)
+    golden = host.tonemap_rgb8(golden_array("tiny_refhi_a.f32", np.float32, (h, w, 3)))
     outs = {}
     cli.main(["prog", gltf_path, str(w), str(h), str(spp), str(tmp_path / "py" / "o.ppm")])
     outs["python"] = _read_ppm(tmp_path / "py" / "o.ppm")
@@ -387,6 +390,10 @@ def test_cli_drop_in_matches_reference_binary(scene_dir, tmp_path):
         outs["cxx"] = _read_ppm(tmp_path / "cxx" / "o.ppm")
         # same Philox seed, same scene bits -> the two hosts differ only by the host that fed the C ABI
         assert np.abs(outs["cxx"].astype(int) - outs["python"].astype(int)).max() <= 1
+    for name, img in outs.items():
+        assert img.shape == golden.shape
+        mae = np.abs(img.astype(int) - golden.astype(int)).mean()
+        assert mae < 1.0, (name, mae)
     if os.path.exists(O.REF_BINARY):
         subprocess.run([O.REF_BINARY, gltf_path, str(w), str(h), str(spp), str(tmp_path / "ref" / "o.ppm")], check=True,
                        capture_output=True)

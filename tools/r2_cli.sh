@@ -5,13 +5,8 @@
 mkdir -p gpurun_out
 OUT=gpurun_out/r2_cli_times.log
 : > $OUT
-python - <<PY
-import sys, os
-sys.path[:0] = [os.getcwd(), os.path.join(os.getcwd(), "scenes")]
-import bench
-print(bench.scene_path("big_lights"))
-PY
-G=scenes/cache/rank0/big_lights.gltf
+SCENE_DIR=$(mktemp -d); trap 'rm -rf "$SCENE_DIR"' EXIT
+G=$(python scenes/gen_gltf.py big_lights "$SCENE_DIR") || exit 1
 t() { local s=$(date +%s%N); "$@" > /dev/null 2> gpurun_out/cli.err; local rc=$?; local e=$(date +%s%N); echo "$(( (e - s) / 1000000 )) ms  rc=$rc  : ${ENVDESC} $*" | tee -a $OUT; tail -1 gpurun_out/cli.err >> $OUT; }
 nproc | sed 's/^/host cores: /' | tee -a $OUT
 ENVDESC="" t bin/raytracer_b200 $G 1000 1000 1000 gpurun_out/cli_c4.ppm

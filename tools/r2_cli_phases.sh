@@ -1,12 +1,7 @@
 #!/bin/bash
 # phases of the drop-in CLI on config 4 (RT_TIMING=1)
-python - <<PY
-import sys, os
-sys.path[:0] = [os.getcwd(), os.path.join(os.getcwd(), "scenes")]
-import bench
-bench.scene_path("big_lights")
-PY
-G=scenes/cache/rank0/big_lights.gltf
+SCENE_DIR=$(mktemp -d); trap 'rm -rf "$SCENE_DIR"' EXIT
+G=$(python scenes/gen_gltf.py big_lights "$SCENE_DIR") || exit 1
 for spp in 1 1000 1000; do
   s=$(date +%s%N)
   RT_TIMING=1 bin/raytracer_b200 $G 1000 1000 $spp gpurun_out/t.ppm 2>&1 | grep "raytracer_b200:\|rt_gpu:"
