@@ -254,13 +254,45 @@ int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params);
 int rt_gpu_readback(rt_gpu_ctx *ctx, float *rgb_mean, int32_t *prim_ids, rt_stats *stats);
 
 /* Device pointer of device 0's per-pixel float sums (width*height*4 floats,
- * rgb + unused w) so that a one-process-per-GPU caller can hand it to its own
- * collective (e.g. torch.distributed.reduce over NCCL) before readback. */
+ * rgb + w) so that a one-process-per-GPU caller can hand it to its own
+ * collective (e.g. torch.distributed.reduce over NCCL) before readback.  w is 0
+ * after rt_gpu_render; after rt_gpu_render_adaptive it holds Q = sum of y^2 over
+ * the pixel's samples, y = (r + g + b) / 3 of each (NaN-scrubbed) sample, and the
+ * rgb sums are over per-pixel sample counts (rt_gpu_readback_adaptive). */
 int rt_gpu_accum_device_ptr(rt_gpu_ctx *ctx, void **dptr, size_t *n_floats);
 
 /* Device-side tonemap + quantise of the current sums (image.h:49-82):
  * rgb8 = width*height*3 bytes, ready to follow the "P6" header. */
 int rt_gpu_readback_rgb8(rt_gpu_ctx *ctx, uint8_t *rgb8);
+
+/* ---- adaptive sampling -------------------------------------------------------------------------------------
+ * rt_gpu_render_adaptive traces every pixel of [pixel_begin, pixel_end) until its noise reaches a target:
+ * params->samples is the MAXIMUM spp.  Round 0 gives every pixel min_samples samples; every later round gives
+ * step_samples more to each pixel that has not converged (the last round clipped at samples).  A pixel always has
+ * the sample prefix [0, n_p), so the image is, pixel by pixel, a fixed render truncated at that pixel's count.
+ * After n samples with S = sum y, Q = sum y^2 (y = (r + g + b) / 3 of each sample), in double precision:
+ *     m = S / n,  var = max(Q / n - m^2, 0) * n / (n - 1),  err = sqrt(var / n) / (m + abs_floor)
+ * and the pixel stops once err <= rel_error (rel_error = 0: never early; with min_samples == samples that is a
+ * fixed render that also yields the error map).  Afterwards rt_gpu_readback returns sum / n_p per pixel (0 where
+ * n_p = 0, i.e. outside the range), rt_gpu_readback_rgb8 tonemaps the same means and stats.samples = sum of n_p.
+ * RT_ERR_INVALID_ARG for sample_begin / sample_end != 0, RT_FLAG_ACCUMULATE, RT_MODE_PRIMARY_IDS, samples < 2,
+ * min_samples < 2, step_samples == 0, abs_floor <= 0, a text scene, or a (per-device) pixel range larger than one
+ * batch of max_paths_in_flight paths.  A multi-device handle splits the range into contiguous parts, one per
+ * device; the image equals the one-device image bit for bit.  RT_FLAG_ACCUMULATE on a render that follows an
+ * adaptive one fails with RT_ERR_INVALID_ARG (the sums have per-pixel counts); without it a render behaves as on a
+ * fresh handle. */
+typedef struct rt_adaptive_params {
+    uint32_t min_samples;   /* first round, every pixel of the range; >= 2 */
+    uint32_t step_samples;  /* added per later round to every pixel not yet converged; >= 1 */
+    float rel_error;        /* stop a pixel once err <= rel_error (0: never stop early) */
+    float abs_floor;        /* > 0: keeps near-black pixels from chasing relative noise */
+} rt_adaptive_params;
+
+int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_adaptive_params *ap);
+
+/* After rt_gpu_render_adaptive: per-pixel sample counts (width*height uint32) and the err each pixel last had
+ * (width*height float; 0 outside the range); either may be NULL.  RT_ERR_NO_RENDER after any other render. */
+int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error);
 
 /* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene.
  * which = 0: uint32[8] {n_tris, binary node slots, 4-wide nodes, root link, worst-case traversal stack need, depth of

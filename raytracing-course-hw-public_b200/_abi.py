@@ -79,6 +79,10 @@ class rt_render_params(C.Structure):
                 ("pixel_end", C.c_uint32)]
 
 
+class rt_adaptive_params(C.Structure):
+    _fields_ = [("min_samples", C.c_uint32), ("step_samples", C.c_uint32), ("rel_error", C.c_float), ("abs_floor", C.c_float)]
+
+
 class rt_stats(C.Structure):
     _fields_ = [("samples", C.c_uint64), ("extension_rays", C.c_uint64), ("light_pdf_rays", C.c_uint64),
                 ("shades", C.c_uint64), ("render_ms", C.c_double), ("reduce_ms", C.c_double),

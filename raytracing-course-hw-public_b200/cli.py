@@ -5,8 +5,14 @@ import os
 import sys
 
 
-def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1):
-    """Mirror of run_raytracer(scene, image) (src/raytracer.h:629): float means [H, W, 3] + stats."""
+def adaptive_steps(samples):
+    """min_samples = step_samples of the CLI's adaptive mode for a maximum of `samples` spp: 16 rounds at most."""
+    return max(2, -(-samples // 16))
+
+
+def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1, rel_error=None):
+    """Mirror of run_raytracer(scene, image) (src/raytracer.h:629): float means [H, W, 3] + stats.  With rel_error,
+    `samples` is the maximum spp of an adaptive render (rt_gpu_render_adaptive)."""
     from . import gpu, textscene
 
     with gpu.RtGpu(n_gpus, 0) as rt:
@@ -15,7 +21,12 @@ def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1):
         else:
             rt.upload_scene(scene)
         # one-shot command: 128 Mi paths per batch (17 GB of queues instead of 68 GB), see host/main_ref_host.cpp
-        rt.render(width, height, samples, seed=seed, max_paths_in_flight=int(os.environ.get("RT_PATHS", 128 << 20)))
+        paths = int(os.environ.get("RT_PATHS", 128 << 20))
+        if rel_error is None:
+            rt.render(width, height, samples, seed=seed, max_paths_in_flight=paths)
+        else:
+            step = adaptive_steps(samples)
+            rt.render_adaptive(width, height, samples, step, step, rel_error, seed=seed, max_paths_in_flight=paths)
         return rt.readback()
 
 
@@ -34,11 +45,18 @@ def main(argv=None):
             width, height, samples = width or scene.width, height or scene.height, samples or scene.samples
         else:
             scene = gltf.load_gltf(argv[1], width / height, env_map=os.environ.get("RT_ENV_MAP") or None)
+        # RT_ADAPTIVE=<rel_error>: `samples` is the maximum spp; every pixel stops once its relative error is reached
+        adaptive = os.environ.get("RT_ADAPTIVE")
+        rel_error = float(adaptive) if adaptive else None
         mean, stats = run_raytracer(scene, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
-                                    n_gpus=int(os.environ.get("RT_GPUS", "1")))
+                                    n_gpus=int(os.environ.get("RT_GPUS", "1")), rel_error=rel_error)
         host.write_ppm(argv[5], host.tonemap_rgb8(mean))
         ms = max(stats["render_ms"], 1e-9)
         print(f"rt_gpu: {ms:.1f} ms, {stats['samples'] / ms * 1e-3:.1f} Msamples/s", file=sys.stderr)
+        if rel_error is not None:
+            full = width * height * samples
+            print(f"rt_gpu adaptive (rel_error {rel_error:g}): {stats['samples']} samples traced, "
+                  f"{stats['samples'] / full:.3f} of {full}", file=sys.stderr)
     except RuntimeError as e:
         print(e, file=sys.stderr)
         return 1

@@ -116,32 +116,19 @@ constexpr uint32_t kCounterStride = RT_COUNTER_STRIDE;
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
 
-__global__ void __launch_bounds__(256) k_generate(Camera cam, BatchParams bp, Queues q) {
-    const uint32_t n = bp.npix * bp.k;
-    const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot == 0) {
-        q.count[0] = n;
-        atomicAdd(q.stats + 3, static_cast<unsigned long long>(n));
-    }
-    if (slot >= n) return;
-    const uint32_t j = slot / bp.npix;
-    const uint32_t pl = slot - j * bp.npix;
-    const uint32_t sample = bp.s0 + j;
-    // The order of queue 0 is free (a path's radiance slot follows from its pixel and sample, not from its queue
-    // position): with one 8 x 4 tile per warp instead of a 32 x 1 strip the camera rays of a warp share more of their
-    // traversal (bounce 0 is a quarter of k_extend's time).  Whole-image batches only (the host sets bp.tiled).
-    uint32_t pixel, px, py;
-    if (bp.tiled) {
-        const uint32_t tile = pl >> 5, in = pl & 31u, tiles_x = bp.width >> 3;
-        const uint32_t ty = tile / tiles_x, tx = tile - ty * tiles_x;
-        px = tx * 8u + (in & 7u);
-        py = ty * 4u + (in >> 3);
-        pixel = py * bp.width + px;
-    } else {
-        pixel = bp.pix0 + pl;
-        py = pixel / bp.width;
-        px = pixel - py * bp.width;
-    }
+// Position pl of a whole-image queue in 8 x 4 pixel tiles (one warp = one tile; width % 8 == 0, height % 4 == 0)
+__device__ __forceinline__ uint32_t tiled_pixel(uint32_t pl, uint32_t width) {
+    const uint32_t tile = pl >> 5, in = pl & 31u, tiles_x = width >> 3;
+    const uint32_t ty = tile / tiles_x, tx = tile - ty * tiles_x;
+    return (ty * 4u + (in >> 3)) * width + tx * 8u + (in & 7u);
+}
+
+// The camera ray of (pixel, sample) into queue position `slot`, its radiance slot `rad_slot` cleared.  k_generate and
+// the adaptive k_generate_active (adaptive.cuh) both go through here.
+__device__ __forceinline__ void emit_camera_ray(const Camera &cam, const BatchParams &bp, const Queues &q, uint32_t slot, uint32_t rad_slot,
+                                                uint32_t pixel, uint32_t sample) {
+    const uint32_t py = pixel / bp.width;
+    const uint32_t px = pixel - py * bp.width;
     const RngKey key{pixel, sample, bp.k0, bp.k1};
     float jx = 0.5f, jy = 0.5f;
     if (!bp.centre) {
@@ -153,7 +140,25 @@ __global__ void __launch_bounds__(256) k_generate(Camera cam, BatchParams bp, Qu
     q_store<2>(q.o_out + slot, make_float4(cam.pos.x, cam.pos.y, cam.pos.z, __uint_as_float(pixel)));
     q_store<2>(q.d_out + slot, make_float4(dir.x, dir.y, dir.z, __uint_as_float(sample)));
     q_store<2>(q.thr_out + slot, make_float4(1.0f, 1.0f, 1.0f, -1.0f));
-    q_store<3>(q.rad + slot, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+    q_store<3>(q.rad + rad_slot, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+}
+
+__global__ void __launch_bounds__(256) k_generate(Camera cam, BatchParams bp, Queues q) {
+    const uint32_t n = bp.npix * bp.k;
+    const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
+    if (slot == 0) {
+        q.count[0] = n;
+        atomicAdd(q.stats + 3, static_cast<unsigned long long>(n));
+    }
+    if (slot >= n) return;
+    const uint32_t j = slot / bp.npix;
+    const uint32_t pl = slot - j * bp.npix;
+    // The order of queue 0 is free (a path's radiance slot follows from its pixel and sample, not from its queue
+    // position): with one 8 x 4 tile per warp instead of a 32 x 1 strip the camera rays of a warp share more of their
+    // traversal (bounce 0 is a quarter of k_extend's time).  Whole-image batches only (the host sets bp.tiled).  The
+    // slots of the batch are a permutation of its queue positions, so clearing rad at `slot` clears all of them.
+    const uint32_t pixel = bp.tiled ? tiled_pixel(pl, bp.width) : bp.pix0 + pl;
+    emit_camera_ray(cam, bp, q, slot, slot, pixel, bp.s0 + j);
 }
 
 // one term of bvh_mix_dist::pdf: the light triangle `le` (normal, area) hit at distance t along d
@@ -835,15 +840,29 @@ __global__ void __launch_bounds__(256) k_split_nodes(const QNode4 *__restrict__ 
     *reinterpret_cast<uint4 *>(dst) = v;
 }
 
+// sum_j sanitize(rad[j * npix + p]) over the k samples of a batch, j ascending.  MOMENTS also returns in .w the sum of
+// y^2, y = (r + g + b) / 3 of each sanitised sample (the second moment of the adaptive stopping rule, adaptive.cuh).
+template <bool MOMENTS>
+__device__ __forceinline__ float4 sum_samples(const BatchParams &bp, const float4 *__restrict__ rad, uint32_t p) {
+    f3 sum = mk3(0, 0, 0);
+    float y2 = 0.0f;
+    for (uint32_t j = 0; j < bp.k; ++j) {
+        const float4 v = q_load<3>(rad + static_cast<size_t>(j) * bp.npix + p);
+        const f3 c = sanitize(mk3(v.x, v.y, v.z));
+        sum = sum + c;
+        if (MOMENTS) {
+            const float y = (c.x + c.y + c.z) / 3.0f;
+            y2 += y * y;
+        }
+    }
+    return make_float4(sum.x, sum.y, sum.z, y2);
+}
+
 // accum[pixel] += sum_j sanitize(rad[j * npix + p])  — fixed order, deterministic, no atomics
 __global__ void __launch_bounds__(256) k_accumulate(BatchParams bp, const float4 *__restrict__ rad, float4 *__restrict__ accum) {
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= bp.npix) return;
-    f3 sum = mk3(0, 0, 0);
-    for (uint32_t j = 0; j < bp.k; ++j) {
-        const float4 v = q_load<3>(rad + static_cast<size_t>(j) * bp.npix + p);
-        sum = sum + sanitize(mk3(v.x, v.y, v.z));
-    }
+    const float4 sum = sum_samples<false>(bp, rad, p);
     float4 a = accum[bp.pix0 + p];
     a.x += sum.x;
     a.y += sum.y;
@@ -871,11 +890,7 @@ __global__ void __launch_bounds__(256) k_means(const float4 *__restrict__ accum,
 }
 
 // Device-side Image::set_pixel (image.h:40-82): mean -> ACES -> gamma 1/2.2 -> x255 -> clamp -> round
-__global__ void __launch_bounds__(256) k_tonemap(const float4 *__restrict__ accum, float samples, uint32_t n_pixels,
-                                                 uint8_t *__restrict__ rgb8) {
-    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= n_pixels) return;
-    const float4 a = accum[p];
+__device__ __forceinline__ void tonemap_pixel(float4 a, float samples, uint8_t *__restrict__ out) {
     const float c[3] = {a.x / samples, a.y / samples, a.z / samples};  // `res / samples`, raytracer.h:626
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
@@ -883,8 +898,15 @@ __global__ void __launch_bounds__(256) k_tonemap(const float4 *__restrict__ accu
         const float m = (x * (2.51f * x + 0.03f)) / (x * (2.43f * x + 0.59f) + 0.14f);
         const float v = powf(m, 1.0f / 2.2f) * 255.0f;
         const float cl = fminf(fmaxf(v, 0.0f), 255.0f);  // NaN -> 0
-        rgb8[static_cast<size_t>(p) * 3 + k] = static_cast<uint8_t>(roundf(cl));
+        out[k] = static_cast<uint8_t>(roundf(cl));
     }
+}
+
+__global__ void __launch_bounds__(256) k_tonemap(const float4 *__restrict__ accum, float samples, uint32_t n_pixels,
+                                                 uint8_t *__restrict__ rgb8) {
+    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_pixels) return;
+    tonemap_pixel(accum[p], samples, rgb8 + static_cast<size_t>(p) * 3);
 }
 
 // FP32 roofline probe: 16 independent FFMA chains per thread, no memory traffic.

@@ -32,6 +32,7 @@
 #include "text_kernels.cuh"
 #include "repack.h"
 #include "gpu_build.cuh"
+#include "adaptive.cuh"
 #include "rt_gpu.h"
 
 namespace {
@@ -78,6 +79,7 @@ struct NcclApi {
     }
 };
 NcclApi g_nccl;
+constexpr int kNcclUint32 = 3;   // ncclUint32
 constexpr int kNcclFloat32 = 7;  // ncclFloat32
 constexpr int kNcclSum = 0;      // ncclSum
 
@@ -192,6 +194,14 @@ struct DeviceState {
         return RT_OK;
     }
     DevBuf<unsigned long long> stats;
+    // adaptive sampling (rt_gpu_render_adaptive, adaptive.cuh): two active lists (ping-pong), the flag words and their
+    // scan, per-pixel sample counts and errors (whole image, 0 outside this device's range), the active count of each
+    // list; each round's count travels behind ev_round[round & 1] into the pinned h_active[round & 1]
+    DevBuf<uint32_t> alist, awords, acounts, actr;
+    DevBuf<float> aerr;
+    uint32_t *h_active = nullptr;
+    cudaEvent_t ev_round[2] = {nullptr, nullptr};
+    size_t apix0 = 0, apix1 = 0;  // the pixel range this device adapted in the last adaptive render
     DevBuf<int32_t> prim_ids;
     DevBuf<uint8_t> rgb8;
     int extend_blocks = 0, shade_blocks = 0, light_blocks = 0;
@@ -218,6 +228,9 @@ struct rt_gpu_ctx {
     std::vector<ncclComm_t> comms;
     bool have_scene = false, have_render = false, profiling = false;
     bool text_scene = false;  // the uploaded scene is a course text scene
+    bool adaptive = false;       // the last render was rt_gpu_render_adaptive (rt_gpu_readback_adaptive has data)
+    bool adaptive_sums = false;  // the sums are an adaptive render's: per-pixel sample counts, Q in w
+    rt_adaptive_params last_adaptive{};
     rt_render_params last{};
     rt_stats stats{};
     uint32_t ray_depth = 0;
@@ -572,6 +585,118 @@ int enqueue_text_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt
     return RT_OK;
 }
 
+// Paths in flight per batch.  Every kernel of a batch ends with a tail in which the last warps finish
+// their rays while the other SMs idle, so throughput grows with the batch: 8 Mi / 16 / 32 / 64 / 128 /
+// 256 Mi paths -> 771 / 819 / 845 / 881 / 896 / 910 Msamples/s on config 4 (B200, measured; a later build: 128 / 256 /
+// 512 / 640 Mi -> 1149 / 1163 / 1169 / 1169).  The default is 512 Mi paths (140 B of queue state each = 75 GB of the
+// 180 GB), capped at half of the free memory.
+size_t batch_cap(const DeviceState &d, uint32_t max_paths_in_flight, size_t want_total) {
+    size_t max_paths = max_paths_in_flight;
+    if (max_paths == 0) {
+        max_paths = static_cast<size_t>(512) << 20;
+        // the memory query is a slow, jittery driver call (tens of ms with 50 GB allocated): only when the queues
+        // would have to grow beyond what this handle already holds
+        if (std::min(max_paths, want_total) > d.queue_cap) {
+            size_t free_b = 0, total_b = 0;
+            if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess)
+                max_paths = std::min(max_paths, std::max(d.queue_cap, (free_b + d.queue_cap * kBytesPerPath) / 2 / kBytesPerPath));
+        }
+    }
+    max_paths = std::max<size_t>(max_paths, 1024);
+    return std::min(max_paths, want_total);
+}
+
+size_t n_counters_of(uint32_t qdepth) { return (6 * static_cast<size_t>(qdepth) + 2) * rt::kCounterStride; }  // one 256-byte line each
+
+// Queues of bounce b: in = parity b & 1, out = the other one (k_generate fills queue 0 through `out` of b = -1)
+rt::Queues queues_of(DeviceState &d, uint32_t qdepth, int b) {
+    rt::Queues q;
+    const int in = b & 1, out = in ^ 1;
+    q.o_in = d.qo[in];
+    q.d_in = d.qd[in];
+    q.thr_in = d.qthr[in];
+    q.o_out = d.qo[out];
+    q.d_out = d.qd[out];
+    q.thr_out = d.qthr[out];
+    q.hit = d.hit;
+    q.rad = d.rad;
+    q.count = d.counters.p;
+    q.fetch_ext = d.counters.p + (qdepth + 1) * rt::kCounterStride;
+    q.fetch_shade = d.counters.p + (2 * qdepth + 1) * rt::kCounterStride;
+    q.stats = d.stats.p;
+    q.lpdf = d.lpdf[in];
+    q.lpdf_out = d.lpdf[out];
+    q.light_list = d.light_list;
+    q.light_count = d.counters.p + (3 * qdepth + 1) * rt::kCounterStride;
+    return q;
+}
+
+// The bounce loop of one batch whose queue 0 is filled (at most n paths): k_lightpdf_list / k_extend / k_shade per
+// bounce.  On return every kernel of the batch is ordered before the next work on d.stream.
+int enqueue_bounces(rt_gpu_ctx *ctx, DeviceState &d, const rt::BatchParams &bp, uint32_t n, bool split_allowed, uint64_t &launches) {
+    const uint32_t depth = d.scene.ray_depth, qdepth = std::max(depth, 1u);
+    const float inv_n_lights = d.scene.n_lights ? 1.0f / static_cast<float>(d.scene.n_lights) : 0.0f;
+#if !RT_EXT_WIDE8
+    // Batches below 256 Mi paths: two halves of every queue on two streams.  A persistent kernel ends with a drain
+    // (once its queue is empty every warp runs on with fewer and fewer live lanes and the SMs empty out), a fixed
+    // cost per launch.  With the halves in flight together the other half's next kernel moves into the freed
+    // slots: E(b, 0) | E(b, 1) over E(b, 0)'s drain | S(b, 0) over E(b, 1)'s drain | S(b, 1) over S(b, 0)'s; only
+    // the last shade of a bounce drains in the open (both halves of queue b + 1 need both shades of queue b).
+    // Measured on config 4: 92.05 -> 91.07 ms at 125 spp (the 8-GPU share of the image), 709.7 -> 711.6 ms at
+    // 1000 spp in 512 Mi-path batches, hence the bound.
+    const bool split = split_allowed && n < (256u << 20);
+    if (split) {
+        cudaStream_t sa = d.stream, sb = d.stream2;
+        CU_CHECK(cudaEventRecord(d.ev_a, sa));  // k_generate (and the counters' memset) done
+        CU_CHECK(cudaStreamWaitEvent(sb, d.ev_a, 0));
+        for (uint32_t b = 0; b < depth; ++b) {
+            rt::Queues q0 = queues_of(d, qdepth, static_cast<int>(b)), q1 = q0;
+            q1.fetch_ext = d.counters.p + (4 * qdepth + 2) * rt::kCounterStride;
+            q1.fetch_shade = d.counters.p + (5 * qdepth + 2) * rt::kCounterStride;
+            if (b > 0) {  // queue b is complete when both shades of queue b - 1 are
+                CU_CHECK(cudaStreamWaitEvent(sa, d.ev_b, 0));
+                CU_CHECK(cudaStreamWaitEvent(sb, d.ev_a, 0));
+            }
+            const bool light = RT_LIGHT_KERNEL && b > 0 && d.scene.n_lights > 0;
+            if (light) {
+                rt::k_lightpdf_list<<<d.light_blocks, rt::kLightThreads, 0, sa>>>(d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q0, b, 0x3F800000u);
+                CU_CHECK(cudaEventRecord(d.ev_light, sa));
+                ++launches;
+            }
+            rt::k_extend<<<d.extend_blocks, rt::kExtendThreads, 0, sa>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q0, b | rt::kPartFirst, 0x3F800000u);
+            rt::k_extend<<<d.extend_blocks, rt::kExtendThreads, 0, sb>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q1, b | rt::kPartSecond, 0x3F800000u);
+            rt::k_shade<<<d.shade_blocks, rt::kShadeThreads, 0, sa>>>(d.scene, d.lut.p, bp, q0, b | rt::kPartFirst, d.light_box);
+            if (light) CU_CHECK(cudaStreamWaitEvent(sb, d.ev_light, 0));  // the light pdfs of queue b
+            rt::k_shade<<<d.shade_blocks, rt::kShadeThreads, 0, sb>>>(d.scene, d.lut.p, bp, q1, b | rt::kPartSecond, d.light_box);
+            CU_CHECK(cudaEventRecord(d.ev_a, sa));
+            CU_CHECK(cudaEventRecord(d.ev_b, sb));
+        }
+        CU_CHECK(cudaStreamWaitEvent(sa, d.ev_b, 0));
+        launches += 4 * static_cast<uint64_t>(depth);
+        return RT_OK;
+    }
+#else
+    (void)split_allowed;
+    (void)n;
+#endif
+    for (uint32_t b = 0; b < depth; ++b) {
+        const rt::Queues q = queues_of(d, qdepth, static_cast<int>(b));
+#if RT_LIGHT_KERNEL
+        if (b > 0 && d.scene.n_lights > 0) {  // queue 0 holds camera rays: nothing is pending
+            rt::k_lightpdf_list<<<d.light_blocks, rt::kLightThreads, 0, d.stream>>>(d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q, b, 0x3F800000u);
+            mark(ctx, d, K_LIGHTPDF);
+            ++launches;
+        }
+#endif
+        RT_K_EXTEND<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q, b, 0x3F800000u);
+        mark(ctx, d, K_EXTEND);
+        rt::k_shade<<<d.shade_blocks, rt::kShadeThreads, 0, d.stream>>>(d.scene, d.lut.p, bp, q, b, d.light_box);
+        mark(ctx, d, K_SHADE);
+    }
+    launches += 2 * static_cast<uint64_t>(depth);
+    return RT_OK;
+}
+
 // Enqueue the whole render of samples [s_begin, s_end) on device d (asynchronous).
 int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_render_params &rp, uint32_t s_begin, uint32_t s_end,
                    uint64_t &launches) {
@@ -602,55 +727,14 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
         s_begin = 0;
         s_end = 1;
     }
-    // Paths in flight per batch.  Every kernel of a batch ends with a tail in which the last warps finish
-    // their rays while the other SMs idle, so throughput grows with the batch: 8 Mi / 16 / 32 / 64 / 128 /
-    // 256 Mi paths -> 771 / 819 / 845 / 881 / 896 / 910 Msamples/s on config 4 (B200, measured; a later build: 128 / 256 /
-    // 512 / 640 Mi -> 1149 / 1163 / 1169 / 1169).  The default is 512 Mi paths (140 B of queue state each = 75 GB of the
-    // 180 GB), capped at half of the free memory.
     const size_t px_begin = ids_mode ? 0 : rp.pixel_begin, px_end = ids_mode || rp.pixel_end == 0 ? n_pix : rp.pixel_end;
     const size_t n_render = px_end - px_begin;  // image-tile split: only this pixel range is rendered
-    const size_t want_total = n_render * static_cast<size_t>(s_end - s_begin);
-    size_t max_paths = rp.max_paths_in_flight;
-    if (max_paths == 0) {
-        max_paths = static_cast<size_t>(512) << 20;
-        // the memory query is a slow, jittery driver call (tens of ms with 50 GB allocated): only when the queues
-        // would have to grow beyond what this handle already holds
-        if (std::min(max_paths, want_total) > d.queue_cap) {
-            size_t free_b = 0, total_b = 0;
-            if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess)
-                max_paths = std::min(max_paths, std::max(d.queue_cap, (free_b + d.queue_cap * kBytesPerPath) / 2 / kBytesPerPath));
-        }
-    }
-    max_paths = std::max<size_t>(max_paths, 1024);
-    const size_t cap = std::min(max_paths, want_total);
+    const size_t cap = batch_cap(d, rp.max_paths_in_flight, n_render * static_cast<size_t>(s_end - s_begin));
     if (int rc = d.alloc_queues(cap)) return rc;
     const uint32_t qdepth = std::max(depth, 1u);
-    const size_t n_counters = (6 * static_cast<size_t>(qdepth) + 2) * rt::kCounterStride;  // one 256-byte line each
+    const size_t n_counters = n_counters_of(qdepth);
     if (int rc = d.counters.alloc(n_counters)) return rc;
-
-    // Queues of bounce b: in = parity b & 1, out = the other one (k_generate fills queue 0 through `out` of b = -1)
-    auto queues_of = [&](int b) {
-        rt::Queues q;
-        const int in = b & 1, out = in ^ 1;
-        q.o_in = d.qo[in];
-        q.d_in = d.qd[in];
-        q.thr_in = d.qthr[in];
-        q.o_out = d.qo[out];
-        q.d_out = d.qd[out];
-        q.thr_out = d.qthr[out];
-        q.hit = d.hit;
-        q.rad = d.rad;
-        q.count = d.counters.p;
-        q.fetch_ext = d.counters.p + (qdepth + 1) * rt::kCounterStride;
-        q.fetch_shade = d.counters.p + (2 * qdepth + 1) * rt::kCounterStride;
-        q.stats = d.stats.p;
-        q.lpdf = d.lpdf[in];
-        q.lpdf_out = d.lpdf[out];
-        q.light_list = d.light_list;
-        q.light_count = d.counters.p + (3 * qdepth + 1) * rt::kCounterStride;
-        return q;
-    };
-    const rt::Queues q_gen = queues_of(-1);
+    const rt::Queues q_gen = queues_of(d, qdepth, -1);
     // per-kernel profiling needs the kernels one after the other on one stream
     const bool split_allowed = !ids_mode && !ctx->profiling && !std::getenv("RT_NO_SPLIT");
 
@@ -678,75 +762,167 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
             rt::k_generate<<<(n + 255) / 256, 256, 0, d.stream>>>(cam, bp, q_gen);
             mark(ctx, d, K_GENERATE);
             if (ids_mode) {  // pixel-centre rays through the same traversal kernel, then hit -> scene.objects id
-                RT_K_EXTEND<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, queues_of(0), 0, 0x3F800000u);
+                RT_K_EXTEND<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, queues_of(d, qdepth, 0), 0, 0x3F800000u);
                 mark(ctx, d, K_EXTEND);
                 rt::k_ids_from_hits<<<(bp.npix + 255) / 256, 256, 0, d.stream>>>(bp, d.hit, d.scene.scene.tris, d.prim_ids.p);
                 mark(ctx, d, K_IDS);
                 launches += 3;
                 continue;
             }
-#if !RT_EXT_WIDE8
-            // Batches below 256 Mi paths: two halves of every queue on two streams.  A persistent kernel ends with a drain
-            // (once its queue is empty every warp runs on with fewer and fewer live lanes and the SMs empty out), a fixed
-            // cost per launch.  With the halves in flight together the other half's next kernel moves into the freed
-            // slots: E(b, 0) | E(b, 1) over E(b, 0)'s drain | S(b, 0) over E(b, 1)'s drain | S(b, 1) over S(b, 0)'s; only
-            // the last shade of a bounce drains in the open (both halves of queue b + 1 need both shades of queue b).
-            // Measured on config 4: 92.05 -> 91.07 ms at 125 spp (the 8-GPU share of the image), 709.7 -> 711.6 ms at
-            // 1000 spp in 512 Mi-path batches, hence the bound.
-            const bool split = split_allowed && n < (256u << 20);
-            if (split) {
-                cudaStream_t sa = d.stream, sb = d.stream2;
-                CU_CHECK(cudaEventRecord(d.ev_a, sa));  // k_generate (and the counters' memset) done
-                CU_CHECK(cudaStreamWaitEvent(sb, d.ev_a, 0));
-                for (uint32_t b = 0; b < depth; ++b) {
-                    rt::Queues q0 = queues_of(static_cast<int>(b)), q1 = q0;
-                    q1.fetch_ext = d.counters.p + (4 * qdepth + 2) * rt::kCounterStride;
-                    q1.fetch_shade = d.counters.p + (5 * qdepth + 2) * rt::kCounterStride;
-                    if (b > 0) {  // queue b is complete when both shades of queue b - 1 are
-                        CU_CHECK(cudaStreamWaitEvent(sa, d.ev_b, 0));
-                        CU_CHECK(cudaStreamWaitEvent(sb, d.ev_a, 0));
-                    }
-                    const bool light = RT_LIGHT_KERNEL && b > 0 && d.scene.n_lights > 0;
-                    if (light) {
-                        rt::k_lightpdf_list<<<d.light_blocks, rt::kLightThreads, 0, sa>>>(d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q0, b, 0x3F800000u);
-                        CU_CHECK(cudaEventRecord(d.ev_light, sa));
-                        ++launches;
-                    }
-                    rt::k_extend<<<d.extend_blocks, rt::kExtendThreads, 0, sa>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q0, b | rt::kPartFirst, 0x3F800000u);
-                    rt::k_extend<<<d.extend_blocks, rt::kExtendThreads, 0, sb>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q1, b | rt::kPartSecond, 0x3F800000u);
-                    rt::k_shade<<<d.shade_blocks, rt::kShadeThreads, 0, sa>>>(d.scene, d.lut.p, bp, q0, b | rt::kPartFirst, d.light_box);
-                    if (light) CU_CHECK(cudaStreamWaitEvent(sb, d.ev_light, 0));  // the light pdfs of queue b
-                    rt::k_shade<<<d.shade_blocks, rt::kShadeThreads, 0, sb>>>(d.scene, d.lut.p, bp, q1, b | rt::kPartSecond, d.light_box);
-                    CU_CHECK(cudaEventRecord(d.ev_a, sa));
-                    CU_CHECK(cudaEventRecord(d.ev_b, sb));
-                }
-                CU_CHECK(cudaStreamWaitEvent(sa, d.ev_b, 0));
-                rt::k_accumulate<<<(bp.npix + 255) / 256, 256, 0, sa>>>(bp, d.rad, d.accum.p);
-                launches += 2 + 4 * static_cast<uint64_t>(depth);
-                continue;
-            }
-#endif
-            for (uint32_t b = 0; b < depth; ++b) {
-                const rt::Queues q = queues_of(static_cast<int>(b));
-#if RT_LIGHT_KERNEL
-                if (b > 0 && d.scene.n_lights > 0) {  // queue 0 holds camera rays: nothing is pending
-                    rt::k_lightpdf_list<<<d.light_blocks, rt::kLightThreads, 0, d.stream>>>(d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q, b, 0x3F800000u);
-                    mark(ctx, d, K_LIGHTPDF);
-                    ++launches;
-                }
-#endif
-                RT_K_EXTEND<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q, b, 0x3F800000u);
-                mark(ctx, d, K_EXTEND);
-                rt::k_shade<<<d.shade_blocks, rt::kShadeThreads, 0, d.stream>>>(d.scene, d.lut.p, bp, q, b, d.light_box);
-                mark(ctx, d, K_SHADE);
-            }
+            if (int rc = enqueue_bounces(ctx, d, bp, n, split_allowed, launches)) return rc;
             rt::k_accumulate<<<(bp.npix + 255) / 256, 256, 0, d.stream>>>(bp, d.rad, d.accum.p);
             mark(ctx, d, K_ACCUMULATE);
-            launches += 2 + 2 * static_cast<uint64_t>(depth);
+            launches += 2;
         }
     }
     CU_CHECK(cudaGetLastError());
     CU_CHECK(cudaEventRecord(d.ev_end, d.stream));
+    return RT_OK;
+}
+
+// One device's part of an adaptive render (rt_gpu_render_adaptive): the pixel range it adapts and where its rounds are.
+struct AdaptiveRun {
+    DeviceState *d = nullptr;
+    size_t pix0 = 0, n_render = 0;
+    uint32_t k_max = 0, n_words = 0, done = 0;  // samples per pixel and batch; flag words; samples every active pixel has
+    int cur = 0;                                 // the list of the active pixels: alist + cur * n_render
+    bool finished = false;
+    rt::BatchParams bp{};
+    rt::Camera cam{};
+};
+
+// Sizes the queues and the adaptive buffers of run.d for the pixel range [pix0, pix1) and clears its sums, counts and
+// errors; no kernel runs yet.  RT_ERR_INVALID_ARG when the range does not fit one batch at one sample.
+int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp, size_t pix0, size_t pix1) {
+    DeviceState &d = *run.d;
+    CU_CHECK(cudaSetDevice(d.device));
+    const size_t n_pix = static_cast<size_t>(rp.width) * rp.height;
+    run.pix0 = pix0;
+    run.n_render = pix1 - pix0;
+    const size_t cap = batch_cap(d, rp.max_paths_in_flight, std::max<size_t>(run.n_render, 1) * rp.samples);
+    if (run.n_render > cap)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: the pixel range (" + std::to_string(run.n_render) +
+                                            " pixels) does not fit one batch of " + std::to_string(cap) + " paths");
+    run.k_max = static_cast<uint32_t>(cap / std::max<size_t>(run.n_render, 1));
+    run.n_words = static_cast<uint32_t>((run.n_render + 31) / 32);
+    run.cur = 0;
+    run.done = 0;
+    run.finished = run.n_render == 0 || d.scene.ray_depth == 0;  // run_raytracer returns early for ray_depth == 0
+    if (int rc = d.accum.alloc(n_pix)) return rc;
+    if (int rc = d.stats.alloc(4)) return rc;
+    if (int rc = d.acounts.alloc(n_pix)) return rc;
+    if (int rc = d.aerr.alloc(n_pix)) return rc;
+    if (int rc = d.actr.alloc(2)) return rc;
+    if (!run.finished) {
+        if (int rc = d.alloc_queues(cap)) return rc;
+        if (int rc = d.counters.alloc(n_counters_of(std::max(d.scene.ray_depth, 1u)))) return rc;
+        if (int rc = d.alist.alloc(2 * run.n_render)) return rc;
+        if (int rc = d.awords.alloc(2 * static_cast<size_t>(run.n_words))) return rc;
+    }
+    d.apix0 = pix0;
+    d.apix1 = pix1;
+    CU_CHECK(cudaMemsetAsync(d.stats.p, 0, 4 * sizeof(unsigned long long), d.stream));
+    CU_CHECK(cudaMemsetAsync(d.accum.p, 0, n_pix * sizeof(float4), d.stream));
+    CU_CHECK(cudaMemsetAsync(d.acounts.p, 0, n_pix * sizeof(uint32_t), d.stream));
+    CU_CHECK(cudaMemsetAsync(d.aerr.p, 0, n_pix * sizeof(float), d.stream));
+    CU_CHECK(cudaMemsetAsync(d.actr.p, 0, 2 * sizeof(uint32_t), d.stream));
+    rt::BatchParams &bp = run.bp;
+    bp.pix0 = static_cast<uint32_t>(pix0);
+    bp.npix = static_cast<uint32_t>(run.n_render);  // the whole range: k_shade's radiance slots stay those of a fixed render
+    bp.width = rp.width;
+    bp.height = rp.height;
+    bp.k0 = static_cast<uint32_t>(rp.seed);
+    bp.k1 = static_cast<uint32_t>(rp.seed >> 32);
+    bp.centre = 0;
+    bp.tiled = 0;  // queue 0 follows the active list, whose first form is already in tiles where that applies
+    run.cam = make_camera(d.scene, rp.width, rp.height);
+    d.marks.clear();
+    d.events_used = 0;
+    CU_CHECK(cudaEventRecord(d.ev_begin, d.stream));
+    mark(ctx, d, -1);
+    return RT_OK;
+}
+
+// Round `round` of run.d (k samples for every pixel of the active list), asynchronous: batches of k_max samples, then
+// the rule, the flag scan and the compaction into the other list, whose device-side length goes to h_active[round & 1]
+// behind ev_round[round & 1].
+int enqueue_adaptive_round(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp, const rt_adaptive_params &ap, uint32_t round,
+                           uint32_t k, uint64_t &launches) {
+    DeviceState &d = *run.d;
+    CU_CHECK(cudaSetDevice(d.device));
+    const uint32_t qdepth = std::max(d.scene.ray_depth, 1u), npix = run.bp.npix;
+    uint32_t *list = d.alist.p + run.cur * run.n_render, *next = d.alist.p + (run.cur ^ 1) * run.n_render;
+    uint32_t *active = d.actr.p + run.cur, *next_active = d.actr.p + (run.cur ^ 1);
+    uint32_t *words = d.awords.p, *wscan = d.awords.p + run.n_words;
+    if (round == 0) {
+        const bool tiled = run.pix0 == 0 && npix == static_cast<size_t>(rp.width) * rp.height && rp.width % 8 == 0 && rp.height % 4 == 0 &&
+                           !std::getenv("RT_NO_TILES");
+        rt::k_adapt_init<<<(npix + 255) / 256, 256, 0, d.stream>>>(list, run.bp.pix0, npix, rp.width, tiled ? 1u : 0u, active);
+        ++launches;
+    }
+    const rt::Queues q_gen = queues_of(d, qdepth, -1);
+    const bool split_allowed = !ctx->profiling && !std::getenv("RT_NO_SPLIT");
+    for (uint32_t j0 = 0; j0 < k; j0 += run.k_max) {
+        rt::BatchParams bp = run.bp;
+        bp.s0 = run.done + j0;
+        bp.k = std::min(run.k_max, k - j0);
+        const uint32_t n = npix * bp.k;  // the grid of k_generate_active; the queue holds n_active * k paths
+        CU_CHECK(cudaMemsetAsync(d.counters.p, 0, n_counters_of(qdepth) * sizeof(uint32_t), d.stream));
+        rt::k_generate_active<<<(n + 255) / 256, 256, 0, d.stream>>>(run.cam, bp, q_gen, list, active);
+        mark(ctx, d, K_GENERATE);
+        if (int rc = enqueue_bounces(ctx, d, bp, n, split_allowed, launches)) return rc;
+        rt::k_accumulate_active<<<(npix + 255) / 256, 256, 0, d.stream>>>(bp, d.rad, d.accum.p, d.acounts.p, list, active);
+        mark(ctx, d, K_ACCUMULATE);
+        launches += 2;
+    }
+    run.done += k;
+    rt::k_adapt_flags<<<(run.n_words * 32 + 255) / 256, 256, 0, d.stream>>>(list, active, d.accum.p, d.acounts.p, d.aerr.p, rp.samples,
+                                                                               ap.rel_error, ap.abs_floor, words, run.n_words);
+    rtb::kb_scan<<<1, 1024, 0, d.stream>>>(words, wscan, run.n_words, next_active, nullptr);
+    rt::k_adapt_scatter<<<(npix + 255) / 256, 256, 0, d.stream>>>(list, next, active, words, wscan);
+    launches += 3;
+    CU_CHECK(cudaMemcpyAsync(d.h_active + (round & 1), next_active, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
+    CU_CHECK(cudaEventRecord(d.ev_round[round & 1], d.stream));
+    run.cur ^= 1;
+    CU_CHECK(cudaGetLastError());
+    return RT_OK;
+}
+
+// The rounds of every device, interleaved so that no device waits for another.  The host never waits for the round it
+// has just enqueued: before round r + 2 it waits for round r's active count (one round of lookahead) and stops a device
+// whose count was 0, so at most one empty round is launched and the GPU does not idle on the host.
+int enqueue_render_adaptive(rt_gpu_ctx *ctx, std::vector<AdaptiveRun> &runs, const rt_render_params &rp, const rt_adaptive_params &ap,
+                            uint64_t &launches) {
+    const uint32_t first = std::min(ap.min_samples, rp.samples);
+    for (uint32_t round = 0;; ++round) {
+        bool any = false;
+        for (AdaptiveRun &run : runs) {
+            if (run.finished) continue;
+            if (run.done >= rp.samples) {
+                run.finished = true;
+                continue;
+            }
+            DeviceState &d = *run.d;
+            if (round >= 2) {
+                CU_CHECK(cudaSetDevice(d.device));
+                CU_CHECK(cudaEventSynchronize(d.ev_round[round & 1]));  // round - 2's survivors
+                if (d.h_active[round & 1] == 0) {
+                    run.finished = true;
+                    continue;
+                }
+            }
+            const uint32_t k = round == 0 ? first : std::min(ap.step_samples, rp.samples - run.done);
+            if (int rc = enqueue_adaptive_round(ctx, run, rp, ap, round, k, launches)) return rc;
+            any = true;
+        }
+        if (!any) break;
+    }
+    for (AdaptiveRun &run : runs) {
+        DeviceState &d = *run.d;
+        CU_CHECK(cudaSetDevice(d.device));
+        CU_CHECK(cudaEventRecord(d.ev_end, d.stream));
+        CU_CHECK(cudaMemcpyAsync(d.h_stats, d.stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
+    }
     return RT_OK;
 }
 
@@ -793,6 +969,8 @@ int create_devices(rt_gpu_ctx *ctx, int n_gpus, int first_device) {
         CU_CHECK(cudaMallocHost(reinterpret_cast<void **>(&d->h_stats), 4 * sizeof(unsigned long long)));
         std::memset(d->h_stats, 0, 4 * sizeof(unsigned long long));
         CU_CHECK(cudaMallocHost(reinterpret_cast<void **>(&d->h_counters), sizeof(rtb::Counters)));
+        CU_CHECK(cudaMallocHost(reinterpret_cast<void **>(&d->h_active), 2 * sizeof(uint32_t)));
+        for (cudaEvent_t &e : d->ev_round) CU_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         int occ_e = 0, occ_s = 0;
         // experiment knob: shared-memory carve-out of k_extend in percent of the maximum (the rest of the 256 KB is L1)
         if (const char *e = std::getenv("RT_EXT_CARVEOUT"))
@@ -865,11 +1043,13 @@ void rt_gpu_destroy(rt_gpu_ctx *ctx) {
         if (d.h_means) cudaFreeHost(d.h_means);
         if (d.h_stage) cudaFreeHost(d.h_stage);
         if (d.h_counters) cudaFreeHost(d.h_counters);
+        if (d.h_active) cudaFreeHost(d.h_active);
+        d.alist.release(); d.awords.release(); d.acounts.release(); d.actr.release(); d.aerr.release();
         d.in_pos.release(); d.in_nrm.release(); d.in_uv.release(); d.in_tan.release(); d.in_mat.release(); d.build_scratch.release();
         d.counters.release(); d.stats.release();
         d.prim_ids.release(); d.rgb8.release();
         for (cudaEvent_t e : d.event_pool) cudaEventDestroy(e);
-        for (cudaEvent_t e : {d.ev_begin, d.ev_end, d.ev_red0, d.ev_red1, d.ev_a, d.ev_b, d.ev_light})
+        for (cudaEvent_t e : {d.ev_begin, d.ev_end, d.ev_red0, d.ev_red1, d.ev_a, d.ev_b, d.ev_light, d.ev_round[0], d.ev_round[1]})
             if (e) cudaEventDestroy(e);
         if (d.stream2) cudaStreamDestroy(d.stream2);
         if (d.ev_copied) cudaEventDestroy(d.ev_copied);
@@ -958,6 +1138,7 @@ int rt_gpu_upload_scene(rt_gpu_ctx *ctx, const rt_scene_desc *scene) {
     ctx->ray_depth = scene->ray_depth;
     ctx->have_scene = true;
     ctx->have_render = false;
+    ctx->adaptive = ctx->adaptive_sums = false;
     ctx->text_scene = false;
     return RT_OK;
 }
@@ -1003,72 +1184,42 @@ int rt_gpu_upload_text_scene(rt_gpu_ctx *ctx, const rt_text_scene *scene) {
     ctx->ray_depth = scene->ray_depth;
     ctx->have_scene = true;
     ctx->have_render = false;
+    ctx->adaptive = ctx->adaptive_sums = false;
     ctx->text_scene = true;
     return RT_OK;
 }
 
-int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
-    if (!ctx || !params) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: null argument");
-    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render: no scene uploaded");
-    rt_render_params rp = *params;
-    if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull)
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal image size");
-    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: samples == 0");
-    if (rp.sample_end == 0) rp.sample_end = rp.samples;
-    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: sample_begin > sample_end");
-    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height;
-    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
-    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal pixel range");
+namespace {
+
+// The per-pixel sums of every device reduced (sum) to device 0 in one NCCL group; with_counts adds the adaptive
+// render's per-pixel sample counts (each device's are 0 outside its pixel range).
+int reduce_to_device0(rt_gpu_ctx *ctx, size_t n_pix, bool with_counts) {
     const int n = static_cast<int>(ctx->devs.size());
-    const uint32_t total = rp.sample_end - rp.sample_begin;
-    uint64_t launches = 0;
-    // sample-split: device g renders [begin + g*total/n, begin + (g+1)*total/n) of every pixel.  With fewer samples
-    // than devices the image is split instead: device g renders all samples of a contiguous range of the pixels
-    // (the other pixels of its buffer stay 0, so the same reduce(sum) merges the tiles).
-    const bool tile_split = n > 1 && total < static_cast<uint32_t>(n) && rp.mode == RT_MODE_BEAUTY;
-    const uint64_t n_px = rp.pixel_end - rp.pixel_begin;
+    for (auto &d : ctx->devs) {
+        CU_CHECK(cudaSetDevice(d->device));
+        CU_CHECK(cudaEventRecord(d->ev_red0, d->stream));
+    }
+    g_nccl.GroupStart();
     for (int g = 0; g < n; ++g) {
-        uint32_t sb = rp.sample_begin + static_cast<uint32_t>(static_cast<uint64_t>(total) * g / n);
-        uint32_t se = rp.sample_begin + static_cast<uint32_t>(static_cast<uint64_t>(total) * (g + 1) / n);
-        rt_render_params local = rp;
-        if (tile_split) {
-            sb = rp.sample_begin;
-            se = rp.sample_end;
-            local.pixel_begin = rp.pixel_begin + static_cast<uint32_t>(n_px * g / n);
-            local.pixel_end = rp.pixel_begin + static_cast<uint32_t>(n_px * (g + 1) / n);
-            if (local.pixel_end == local.pixel_begin) se = sb;  // nothing for this device: zero buffer only
-        }
-        if (rp.mode == RT_MODE_PRIMARY_IDS && g > 0) continue;  // ids: device 0 only
-        DeviceState &dg = *ctx->devs[g];
-        if (ctx->text_scene) {
-            if (int rc = enqueue_text_render(ctx, dg, g, local, sb, se, launches)) return rc;
-        } else if (int rc = enqueue_render(ctx, dg, g, local, sb, se, launches)) {
-            return rc;
-        }
-        // the work counters travel on the stream into pinned memory: no second synchronising copy after the render
-        CU_CHECK(cudaMemcpyAsync(dg.h_stats, dg.stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, dg.stream));
-    }
-    const size_t n_floats = static_cast<size_t>(rp.width) * rp.height * 4;
-    if (n > 1 && rp.mode == RT_MODE_BEAUTY) {
-        for (auto &d : ctx->devs) {
-            CU_CHECK(cudaSetDevice(d->device));
-            CU_CHECK(cudaEventRecord(d->ev_red0, d->stream));
-        }
-        g_nccl.GroupStart();
-        for (int g = 0; g < n; ++g) {
-            DeviceState &d = *ctx->devs[g];
-            const int rc = g_nccl.Reduce(d.accum.p, d.accum.p, n_floats, kNcclFloat32, kNcclSum, 0, ctx->comms[g], d.stream);
-            if (rc != 0) {
-                g_nccl.GroupEnd();
-                return fail(RT_ERR_NCCL, std::string("ncclReduce: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"));
-            }
-        }
-        if (int rc = g_nccl.GroupEnd()) return fail(RT_ERR_NCCL, std::string("ncclGroupEnd: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"));
-        for (auto &d : ctx->devs) {
-            CU_CHECK(cudaSetDevice(d->device));
-            CU_CHECK(cudaEventRecord(d->ev_red1, d->stream));
+        DeviceState &d = *ctx->devs[g];
+        int rc = g_nccl.Reduce(d.accum.p, d.accum.p, n_pix * 4, kNcclFloat32, kNcclSum, 0, ctx->comms[g], d.stream);
+        if (rc == 0 && with_counts) rc = g_nccl.Reduce(d.acounts.p, d.acounts.p, n_pix, kNcclUint32, kNcclSum, 0, ctx->comms[g], d.stream);
+        if (rc != 0) {
+            g_nccl.GroupEnd();
+            return fail(RT_ERR_NCCL, std::string("ncclReduce: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"));
         }
     }
+    if (int rc = g_nccl.GroupEnd()) return fail(RT_ERR_NCCL, std::string("ncclGroupEnd: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"));
+    for (auto &d : ctx->devs) {
+        CU_CHECK(cudaSetDevice(d->device));
+        CU_CHECK(cudaEventRecord(d->ev_red1, d->stream));
+    }
+    return RT_OK;
+}
+
+// Waits for every device, gathers the work counters and timings of the render into ctx->stats.
+int finish_render(rt_gpu_ctx *ctx, const rt_render_params &rp, uint64_t launches) {
+    const int n = static_cast<int>(ctx->devs.size());
     rt_stats st;
     std::memset(&st, 0, sizeof st);
     for (int g = 0; g < n; ++g) {
@@ -1109,8 +1260,129 @@ int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
     }
     st.kernel_launches = launches;
     ctx->stats = st;
+    return RT_OK;
+}
+
+}  // namespace
+
+int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
+    if (!ctx || !params) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render: no scene uploaded");
+    rt_render_params rp = *params;
+    if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal image size");
+    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: samples == 0");
+    if (rp.sample_end == 0) rp.sample_end = rp.samples;
+    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: sample_begin > sample_end");
+    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height;
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal pixel range");
+    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY && ctx->adaptive_sums)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: RT_FLAG_ACCUMULATE onto the sums of an adaptive render (per-pixel sample counts)");
+    const int n = static_cast<int>(ctx->devs.size());
+    const uint32_t total = rp.sample_end - rp.sample_begin;
+    uint64_t launches = 0;
+    // sample-split: device g renders [begin + g*total/n, begin + (g+1)*total/n) of every pixel.  With fewer samples
+    // than devices the image is split instead: device g renders all samples of a contiguous range of the pixels
+    // (the other pixels of its buffer stay 0, so the same reduce(sum) merges the tiles).
+    const bool tile_split = n > 1 && total < static_cast<uint32_t>(n) && rp.mode == RT_MODE_BEAUTY;
+    const uint64_t n_px = rp.pixel_end - rp.pixel_begin;
+    for (int g = 0; g < n; ++g) {
+        uint32_t sb = rp.sample_begin + static_cast<uint32_t>(static_cast<uint64_t>(total) * g / n);
+        uint32_t se = rp.sample_begin + static_cast<uint32_t>(static_cast<uint64_t>(total) * (g + 1) / n);
+        rt_render_params local = rp;
+        if (tile_split) {
+            sb = rp.sample_begin;
+            se = rp.sample_end;
+            local.pixel_begin = rp.pixel_begin + static_cast<uint32_t>(n_px * g / n);
+            local.pixel_end = rp.pixel_begin + static_cast<uint32_t>(n_px * (g + 1) / n);
+            if (local.pixel_end == local.pixel_begin) se = sb;  // nothing for this device: zero buffer only
+        }
+        if (rp.mode == RT_MODE_PRIMARY_IDS && g > 0) continue;  // ids: device 0 only
+        DeviceState &dg = *ctx->devs[g];
+        if (ctx->text_scene) {
+            if (int rc = enqueue_text_render(ctx, dg, g, local, sb, se, launches)) return rc;
+        } else if (int rc = enqueue_render(ctx, dg, g, local, sb, se, launches)) {
+            return rc;
+        }
+        // the work counters travel on the stream into pinned memory: no second synchronising copy after the render
+        CU_CHECK(cudaMemcpyAsync(dg.h_stats, dg.stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, dg.stream));
+    }
+    if (n > 1 && rp.mode == RT_MODE_BEAUTY)
+        if (int rc = reduce_to_device0(ctx, static_cast<size_t>(rp.width) * rp.height, false)) return rc;
+    if (int rc = finish_render(ctx, rp, launches)) return rc;
     ctx->last = rp;
     ctx->have_render = true;
+    ctx->adaptive = false;
+    if (rp.mode == RT_MODE_BEAUTY) ctx->adaptive_sums = false;
+    return RT_OK;
+}
+
+int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_adaptive_params *ap) {
+    if (!ctx || !params || !ap) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render_adaptive: no scene uploaded");
+    rt_render_params rp = *params;
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: not available for course text scenes");
+    if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: illegal image size");
+    if (rp.mode != RT_MODE_BEAUTY) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: beauty renders only");
+    if (rp.samples < 2) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: samples (the maximum spp) < 2");
+    if (rp.sample_begin != 0 || rp.sample_end != 0)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: every pixel starts at sample 0 (sample_begin / sample_end must be 0)");
+    if (rp.flags & RT_FLAG_ACCUMULATE) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: RT_FLAG_ACCUMULATE is not supported");
+    if (ap->min_samples < 2 || ap->step_samples == 0 || !(ap->abs_floor > 0.0f) || !(ap->rel_error >= 0.0f))
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: needs min_samples >= 2, step_samples >= 1, abs_floor > 0, rel_error >= 0");
+    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height;
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: illegal pixel range");
+    // every device adapts a contiguous part of the range (a pixel's decisions depend on its own sums only)
+    const int n = static_cast<int>(ctx->devs.size());
+    const uint64_t n_px = rp.pixel_end - rp.pixel_begin;
+    std::vector<AdaptiveRun> runs(n);
+    ctx->have_render = false;  // the sums are being replaced
+    for (int g = 0; g < n; ++g) {
+        runs[g].d = ctx->devs[g].get();
+        const size_t b = rp.pixel_begin + n_px * g / n, e = rp.pixel_begin + n_px * (g + 1) / n;
+        if (int rc = setup_adaptive(ctx, runs[g], rp, b, e)) return rc;
+    }
+    uint64_t launches = 0;
+    if (int rc = enqueue_render_adaptive(ctx, runs, rp, *ap, launches)) return rc;
+    if (n > 1)
+        if (int rc = reduce_to_device0(ctx, static_cast<size_t>(n_pixels), true)) return rc;
+    if (int rc = finish_render(ctx, rp, launches)) return rc;
+    if (std::getenv("RT_TIMING")) {  // contiguous tiles are not load-balanced: the per-device times show by how much
+        for (int g = 0; g < n; ++g) {
+            float ms = 0.0f;
+            cudaEventElapsedTime(&ms, runs[g].d->ev_begin, runs[g].d->ev_end);
+            std::fprintf(stderr, "rt_gpu adaptive: device %d pixels [%zu, %zu) %.2f ms, %llu samples\n", runs[g].d->device, runs[g].pix0,
+                         runs[g].pix0 + runs[g].n_render, ms, static_cast<unsigned long long>(runs[g].d->h_stats[3]));
+        }
+    }
+    ctx->last = rp;
+    ctx->last_adaptive = *ap;
+    ctx->have_render = true;
+    ctx->adaptive = ctx->adaptive_sums = true;
+    return RT_OK;
+}
+
+int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error) {
+    if (!ctx) return fail(RT_ERR_INVALID_ARG, "rt_gpu_readback_adaptive: null handle");
+    if (!ctx->have_render || !ctx->adaptive) return fail(RT_ERR_NO_RENDER, "rt_gpu_readback_adaptive: the last render was not adaptive");
+    const size_t n_pix = static_cast<size_t>(ctx->last.width) * ctx->last.height;
+    if (sample_counts) {  // reduced to device 0
+        DeviceState &d = *ctx->devs[0];
+        CU_CHECK(cudaSetDevice(d.device));
+        CU_CHECK(cudaMemcpy(sample_counts, d.acounts.p, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    }
+    if (rel_error) {  // gathered from every device's own range
+        std::memset(rel_error, 0, n_pix * sizeof(float));
+        for (auto &dp : ctx->devs) {
+            DeviceState &d = *dp;
+            if (d.apix1 <= d.apix0) continue;
+            CU_CHECK(cudaSetDevice(d.device));
+            CU_CHECK(cudaMemcpy(rel_error + d.apix0, d.aerr.p + d.apix0, (d.apix1 - d.apix0) * sizeof(float), cudaMemcpyDeviceToHost));
+        }
+    }
     return RT_OK;
 }
 
@@ -1128,7 +1400,10 @@ int rt_gpu_readback(rt_gpu_ctx *ctx, float *rgb_mean, int32_t *prim_ids, rt_stat
         const size_t n_f = n_pix * 3;
         if (int rc = d.means.alloc(n_f)) return rc;
         const uint32_t np32 = static_cast<uint32_t>(n_pix);
-        rt::k_means<<<(np32 + 255) / 256, 256, 0, d.stream>>>(d.accum.p, static_cast<float>(ctx->last.samples), np32, d.means.p);
+        if (ctx->adaptive_sums)
+            rt::k_means_counts<<<(np32 + 255) / 256, 256, 0, d.stream>>>(d.accum.p, d.acounts.p, np32, d.means.p);
+        else
+            rt::k_means<<<(np32 + 255) / 256, 256, 0, d.stream>>>(d.accum.p, static_cast<float>(ctx->last.samples), np32, d.means.p);
         CU_CHECK(cudaGetLastError());
         cudaPointerAttributes attr;
         const bool pinned = cudaPointerGetAttributes(&attr, rgb_mean) == cudaSuccess && attr.type == cudaMemoryTypeHost;
@@ -1182,7 +1457,10 @@ int rt_gpu_readback_rgb8(rt_gpu_ctx *ctx, uint8_t *rgb8) {
     CU_CHECK(cudaSetDevice(d.device));
     const uint32_t n_pix = ctx->last.width * ctx->last.height;
     if (int rc = d.rgb8.alloc(static_cast<size_t>(n_pix) * 3)) return rc;
-    rt::k_tonemap<<<(n_pix + 255) / 256, 256, 0, d.stream>>>(d.accum.p, static_cast<float>(ctx->last.samples), n_pix, d.rgb8.p);
+    if (ctx->adaptive_sums)
+        rt::k_tonemap_counts<<<(n_pix + 255) / 256, 256, 0, d.stream>>>(d.accum.p, d.acounts.p, n_pix, d.rgb8.p);
+    else
+        rt::k_tonemap<<<(n_pix + 255) / 256, 256, 0, d.stream>>>(d.accum.p, static_cast<float>(ctx->last.samples), n_pix, d.rgb8.p);
     CU_CHECK(cudaGetLastError());
     CU_CHECK(cudaMemcpyAsync(rgb8, d.rgb8.p, static_cast<size_t>(n_pix) * 3, cudaMemcpyDeviceToHost, d.stream));
     CU_CHECK(cudaStreamSynchronize(d.stream));

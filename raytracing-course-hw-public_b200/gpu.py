@@ -6,7 +6,8 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_render_params, rt_scene_desc, rt_stats)
+from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_render_params, rt_scene_desc,
+                   rt_stats)
 
 # RT_GPU_LIB selects another build of the same C ABI (kernel A/B experiments, tools/build_variants.sh)
 LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu.so")
@@ -14,7 +15,7 @@ LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu
 # every symbol include/rt_gpu.h declares
 SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upload_text_scene", "rt_gpu_render", "rt_gpu_readback",
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
-           "rt_gpu_device_count", "rt_gpu_abi_version"]
+           "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive"]
 
 _lib = None
 
@@ -30,6 +31,8 @@ def lib():
         L.rt_gpu_upload_text_scene.argtypes = [C.c_void_p, C.c_void_p]
         L.rt_gpu_render.argtypes = [C.c_void_p, C.POINTER(rt_render_params)]
         L.rt_gpu_readback.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+        L.rt_gpu_render_adaptive.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params)]
+        L.rt_gpu_readback_adaptive.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.rt_gpu_accum_device_ptr.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
         L.rt_gpu_readback_rgb8.argtypes = [C.c_void_p, C.c_void_p]
         L.rt_gpu_set_profiling.argtypes = [C.c_void_p, C.c_int]
@@ -101,6 +104,26 @@ class RtGpu:
                              RT_FLAG_ACCUMULATE if accumulate else 0, pixel_begin, pixel_end)
         _check(lib().rt_gpu_render(self._h, C.byref(p)), "rt_gpu_render")
         self._last = (width, height, mode)
+
+    def render_adaptive(self, width, height, max_samples, min_samples, step_samples, rel_error, abs_floor=1e-3, seed=0,
+                        max_paths_in_flight=0, pixel_begin=0, pixel_end=0):
+        """Adaptive render (rt_gpu_render_adaptive): every pixel of the range traces min_samples, then step_samples more
+        per round until its relative standard error is <= rel_error or it has max_samples.  readback() then returns
+        the per-pixel means, readback_adaptive() the sample counts and errors."""
+        p = rt_render_params(width, height, max_samples, 0, 0, RT_MODE_BEAUTY, seed, max_paths_in_flight, 0, pixel_begin,
+                             pixel_end)
+        a = rt_adaptive_params(min_samples, step_samples, rel_error, abs_floor)
+        _check(lib().rt_gpu_render_adaptive(self._h, C.byref(p), C.byref(a)), "rt_gpu_render_adaptive")
+        self._last = (width, height, RT_MODE_BEAUTY)
+
+    def readback_adaptive(self):
+        """(sample counts uint32 [H, W], err float32 [H, W]) of the last adaptive render."""
+        w, h, _ = self._last
+        counts = np.empty((h, w), np.uint32)
+        err = np.empty((h, w), np.float32)
+        _check(lib().rt_gpu_readback_adaptive(self._h, counts.ctypes.data_as(C.c_void_p), err.ctypes.data_as(C.c_void_p)),
+               "rt_gpu_readback_adaptive")
+        return counts, err
 
     def readback(self):
         """(rgb_mean float32 [H, W, 3], stats dict) of the last beauty render."""

@@ -21,8 +21,11 @@
 //   RT_ADD_LIGHT_TRIANGLE  1: the extra light source of the reference's compile-time ADD_LIGHT_TRIANGLE (config.h:39-47)
 //   RT_ENV_MAP  image file used as the equirectangular environment map Scene::bg (the run-time form of the
 //             reference's compile-time USE_ENV_MAP / ENV_MAP_PATH, src/config.h:35-37)
+//   RT_ADAPTIVE  relative-error target of an adaptive render (rt_gpu_render_adaptive, glTF scenes): <samples> becomes
+//             the maximum spp, min_samples = step_samples = max(2, ceil(samples / 16)); the samples traced on stderr
 #define STB_IMAGE_IMPLEMENTATION
 
+#include <algorithm>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -73,7 +76,16 @@ void render_into(rt_gpu_ctx *gpu, unsigned width, unsigned height, unsigned samp
     // A one-shot command pays for allocating and freeing the path queues: 128 Mi paths per batch (17 GB) instead of the
     // library's 512 Mi (68 GB) cost 1.7 % of the render and save ~0.15 s of cudaMalloc / cudaFree (RT_PATHS overrides).
     params.max_paths_in_flight = env_uint("RT_PATHS", 128u << 20);
-    check(rt_gpu_render(gpu, &params), "rt_gpu_render");
+    const char *adaptive = std::getenv("RT_ADAPTIVE");
+    if (adaptive && *adaptive) {
+        rt_adaptive_params ap{};
+        ap.min_samples = ap.step_samples = std::max(2u, (samples + 15) / 16);
+        ap.rel_error = std::strtof(adaptive, nullptr);
+        ap.abs_floor = 1e-3f;
+        check(rt_gpu_render_adaptive(gpu, &params, &ap), "rt_gpu_render_adaptive");
+    } else {
+        check(rt_gpu_render(gpu, &params), "rt_gpu_render");
+    }
     std::vector<float> mean(static_cast<size_t>(width) * height * 3);
     rt_stats stats{};
     check(rt_gpu_readback(gpu, mean.data(), nullptr, &stats), "rt_gpu_readback");
@@ -82,6 +94,11 @@ void render_into(rt_gpu_ctx *gpu, unsigned width, unsigned height, unsigned samp
     std::fprintf(stderr, "rt_gpu: %.1f ms, %.1f Msamples/s, %.1f Mrays/s (extension) + %.1f Mrays/s (light pdf)\n", stats.render_ms,
                  stats.samples / stats.render_ms * 1e-3, stats.extension_rays / stats.render_ms * 1e-3,
                  stats.light_pdf_rays / stats.render_ms * 1e-3);
+    if (adaptive && *adaptive) {
+        const double full = static_cast<double>(width) * height * samples;
+        std::fprintf(stderr, "rt_gpu adaptive (rel_error %s): %llu samples traced, %.3f of %.0f\n", adaptive,
+                     static_cast<unsigned long long>(stats.samples), stats.samples / full, full);
+    }
 }
 
 void write_image(Image &img, const char *path) {
