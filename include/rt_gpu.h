@@ -294,6 +294,31 @@ int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, cons
  * (width*height float; 0 outside the range); either may be NULL.  RT_ERR_NO_RENDER after any other render. */
 int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error);
 
+/* ---- multi-view rendering ----------------------------------------------------------------------------------
+ * rt_gpu_render_views traces n_views cameras over the uploaded triangle scene in one render.  The views of
+ * width x height are stacked into one image of width x (n_views * height): pixel v * width * height + y * width + x
+ * is pixel (x, y) of view v.  Afterwards rt_gpu_readback returns n_views * width * height * 3 floats (view-major)
+ * and, after RT_MODE_PRIMARY_IDS, n_views * width * height ids; rt_gpu_readback_rgb8 returns
+ * n_views * width * height * 3 bytes; rt_gpu_accum_device_ptr reports n_views * width * height * 4 floats;
+ * stats.samples counts every view.  rt_render_params keep their meaning; pixel_begin / pixel_end index the stacked
+ * image [0, n_views * width * height), and a multi-device handle splits it like any image.
+ * Pixel p of view v is keyed (Philox) as pixel (view_base + v) * width * height + p, so:
+ *   - one view with the scene's own camera and view_base = 0 is rt_gpu_render, bit for bit;
+ *   - view v of a call is a one-view call with view_base = v (bit for bit when both run in the same batches),
+ * and how a camera path is split into calls does not change a frame.
+ * RT_ERR_INVALID_ARG for n_views == 0, cameras == NULL, a non-finite camera value, (view_base + n_views) * width *
+ * height > 2^32, a stacked image of more than 2^31 - 1 pixels, a text scene, and RT_FLAG_ACCUMULATE unless the
+ * previous render had the same width, height and n_views (rt_gpu_render counts as one view; this holds in both
+ * directions).  Without the flag, a render behaves as on a fresh handle.  Adaptive sampling over views is not
+ * offered: rt_gpu_readback_adaptive returns RT_ERR_NO_RENDER after this call. */
+typedef struct rt_views {
+    uint32_t n_views;          /* >= 1 */
+    uint32_t view_base;        /* Philox pixel key of pixel p of view v = (view_base + v) * width * height + p */
+    const rt_camera *cameras;  /* n_views cameras; same convention as rt_scene_desc.camera (fov_y from width / height) */
+} rt_views;
+
+int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views);
+
 /* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene.
  * which = 0: uint32[8] {n_tris, binary node slots, 4-wide nodes, root link, worst-case traversal stack need, depth of
  * the binary tree, 1 if built on the device, levels of the top-down phase}; 1: rt_bvh_node[slots] (the binary tree in the

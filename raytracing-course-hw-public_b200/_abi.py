@@ -60,6 +60,44 @@ class rt_camera(C.Structure):
                 ("forward", C.c_float * 3), ("fov_x", C.c_float)]
 
 
+class rt_views(C.Structure):
+    _fields_ = [("n_views", C.c_uint32), ("view_base", C.c_uint32), ("cameras", C.POINTER(rt_camera))]
+
+
+class Camera:
+    """A camera of a scene (rt_camera): position, the right / up / forward axes and the horizontal field of view fov_x
+    in radians, all float32.  Two cameras are equal when every value is equal bit for bit."""
+
+    __slots__ = ("position", "right", "up", "forward", "fov_x")
+
+    def __init__(self, position, right, up, forward, fov_x):
+        self.position = np.array(position, np.float32).reshape(3)
+        self.right = np.array(right, np.float32).reshape(3)
+        self.up = np.array(up, np.float32).reshape(3)
+        self.forward = np.array(forward, np.float32).reshape(3)
+        self.fov_x = np.float32(fov_x)
+
+    def to_c(self):
+        c = rt_camera()
+        for k in range(3):
+            c.position[k], c.right[k] = float(self.position[k]), float(self.right[k])
+            c.up[k], c.forward[k] = float(self.up[k]), float(self.forward[k])
+        c.fov_x = float(self.fov_x)
+        return c
+
+    def _bits(self):
+        return np.concatenate([self.position, self.right, self.up, self.forward, [self.fov_x]]).astype(np.float32).view(np.uint32)
+
+    def __eq__(self, other):
+        return isinstance(other, Camera) and np.array_equal(self._bits(), other._bits())
+
+    __hash__ = None
+
+    def __repr__(self):
+        return (f"Camera(position={self.position.tolist()}, right={self.right.tolist()}, up={self.up.tolist()}, "
+                f"forward={self.forward.tolist()}, fov_x={float(self.fov_x)!r})")
+
+
 class rt_scene_desc(C.Structure):
     _fields_ = [
         ("abi_version", C.c_uint32), ("n_tris", C.c_uint32), ("camera", rt_camera), ("bg_color", C.c_float * 3),
@@ -145,6 +183,12 @@ class SceneData:
         self.texels = np.zeros(0, np.uint8)
         self.scene_bvh = BvhData(np.zeros(0, NODE_DTYPE), np.zeros(0, np.uint32), RT_NO_CHILD)
         self.light_bvh = BvhData(np.zeros(0, NODE_DTYPE), np.zeros(0, np.uint32), RT_NO_CHILD)
+        self.cameras = []  # every camera node of the source glTF in traversal order (gltf.load_gltf); the scene's own
+                           # camera is the last of them
+
+    def camera(self):
+        """The scene's own camera (the one rt_gpu_render uses) as a Camera."""
+        return Camera(self.camera_position, self.camera_right, self.camera_up, self.camera_forward, self.fov_x)
 
     @property
     def n_tris(self):

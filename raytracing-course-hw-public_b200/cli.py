@@ -30,6 +30,22 @@ def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1, rel_error=Non
         return rt.readback()
 
 
+def run_views(scene, cameras, width, height, samples, seed=0, n_gpus=1):
+    """Every camera of `cameras` in one rt_gpu_render_views call: float means [V, H, W, 3] + stats."""
+    from . import gpu
+
+    with gpu.RtGpu(n_gpus, 0) as rt:
+        rt.upload_scene(scene)
+        rt.render_views(cameras, width, height, samples, seed=seed, max_paths_in_flight=int(os.environ.get("RT_PATHS", 128 << 20)))
+        return rt.readback()
+
+
+def view_paths(out, n):
+    """<stem>_<i><ext> for the n views of RT_CAMERAS=all"""
+    stem, ext = os.path.splitext(out)
+    return [f"{stem}_{i}{ext}" for i in range(n)]
+
+
 def main(argv=None):
     argv = sys.argv if argv is None else argv
     if len(argv) < 6:
@@ -48,6 +64,24 @@ def main(argv=None):
         # RT_ADAPTIVE=<rel_error>: `samples` is the maximum spp; every pixel stops once its relative error is reached
         adaptive = os.environ.get("RT_ADAPTIVE")
         rel_error = float(adaptive) if adaptive else None
+        # RT_CAMERAS=all: every camera node of the glTF in one multi-view render, view i to <stem>_<i><ext>
+        cameras = os.environ.get("RT_CAMERAS")
+        if cameras is not None:
+            if cameras != "all":
+                print(f"RT_CAMERAS={cameras}: the only value is 'all'", file=sys.stderr)
+                return 1
+            if rel_error is not None or textscene.is_text_scene(argv[1]):
+                print("RT_CAMERAS=all renders glTF scenes at a fixed spp: it cannot be combined with RT_ADAPTIVE or a "
+                      "text scene", file=sys.stderr)
+                return 1
+            cams = scene.cameras or [scene.camera()]  # no camera node: the scene's default camera
+            means, stats = run_views(scene, cams, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
+                                     n_gpus=int(os.environ.get("RT_GPUS", "1")))
+            for path, mean in zip(view_paths(argv[5], len(cams)), means):
+                host.write_ppm(path, host.tonemap_rgb8(mean))
+            ms = max(stats["render_ms"], 1e-9)
+            print(f"rt_gpu: {len(cams)} views, {ms:.1f} ms, {stats['samples'] / ms * 1e-3:.1f} Msamples/s", file=sys.stderr)
+            return 0
         mean, stats = run_raytracer(scene, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
                                     n_gpus=int(os.environ.get("RT_GPUS", "1")), rel_error=rel_error)
         host.write_ppm(argv[5], host.tonemap_rgb8(mean))

@@ -123,12 +123,10 @@ __device__ __forceinline__ uint32_t tiled_pixel(uint32_t pl, uint32_t width) {
     return (ty * 4u + (in >> 3)) * width + tx * 8u + (in & 7u);
 }
 
-// The camera ray of (pixel, sample) into queue position `slot`, its radiance slot `rad_slot` cleared.  k_generate and
-// the adaptive k_generate_active (adaptive.cuh) both go through here.
-__device__ __forceinline__ void emit_camera_ray(const Camera &cam, const BatchParams &bp, const Queues &q, uint32_t slot, uint32_t rad_slot,
-                                                uint32_t pixel, uint32_t sample) {
-    const uint32_t py = pixel / bp.width;
-    const uint32_t px = pixel - py * bp.width;
+// The camera ray through pixel (px, py) of `cam` for Philox key (pixel, sample) into queue position `slot`, its radiance
+// slot `rad_slot` cleared.  The multi-view k_generate_views (views.cuh) keys a view's pixel apart from its (px, py).
+__device__ __forceinline__ void emit_camera_ray_at(const Camera &cam, const BatchParams &bp, const Queues &q, uint32_t slot, uint32_t rad_slot,
+                                                   uint32_t pixel, uint32_t px, uint32_t py, uint32_t sample) {
     const RngKey key{pixel, sample, bp.k0, bp.k1};
     float jx = 0.5f, jy = 0.5f;
     if (!bp.centre) {
@@ -141,6 +139,15 @@ __device__ __forceinline__ void emit_camera_ray(const Camera &cam, const BatchPa
     q_store<2>(q.d_out + slot, make_float4(dir.x, dir.y, dir.z, __uint_as_float(sample)));
     q_store<2>(q.thr_out + slot, make_float4(1.0f, 1.0f, 1.0f, -1.0f));
     q_store<3>(q.rad + rad_slot, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+}
+
+// The camera ray of row-major (pixel, sample).  k_generate and the adaptive k_generate_active (adaptive.cuh) both go
+// through here.
+__device__ __forceinline__ void emit_camera_ray(const Camera &cam, const BatchParams &bp, const Queues &q, uint32_t slot, uint32_t rad_slot,
+                                                uint32_t pixel, uint32_t sample) {
+    const uint32_t py = pixel / bp.width;
+    const uint32_t px = pixel - py * bp.width;
+    emit_camera_ray_at(cam, bp, q, slot, rad_slot, pixel, px, py, sample);
 }
 
 __global__ void __launch_bounds__(256) k_generate(Camera cam, BatchParams bp, Queues q) {

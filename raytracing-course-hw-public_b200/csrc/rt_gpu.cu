@@ -33,6 +33,7 @@
 #include "repack.h"
 #include "gpu_build.cuh"
 #include "adaptive.cuh"
+#include "views.cuh"
 #include "rt_gpu.h"
 
 namespace {
@@ -204,6 +205,7 @@ struct DeviceState {
     size_t apix0 = 0, apix1 = 0;  // the pixel range this device adapted in the last adaptive render
     DevBuf<int32_t> prim_ids;
     DevBuf<uint8_t> rgb8;
+    DevBuf<rt::Camera> cams;  // the cameras of the last multi-view render (rt_gpu_render_views), one per view
     int extend_blocks = 0, shade_blocks = 0, light_blocks = 0;
     rt::LightBox light_box{};  // box of all light triangles (k_shade tests the rays it queues against it)
     // profiling
@@ -232,6 +234,7 @@ struct rt_gpu_ctx {
     bool adaptive_sums = false;  // the sums are an adaptive render's: per-pixel sample counts, Q in w
     rt_adaptive_params last_adaptive{};
     rt_render_params last{};
+    uint32_t last_views = 0;  // views of the last render: 0 = not rt_gpu_render_views (one image, the scene's camera)
     rt_stats stats{};
     uint32_t ray_depth = 0;
     rt::PackedScene packed;  // staging of the last upload, kept so that the next one re-uses its (already touched) memory
@@ -509,12 +512,12 @@ int upload_to_device(DeviceState &d, const rt_scene_desc &sc, const rt::PackedSc
     return RT_OK;
 }
 
-rt::Camera make_camera(const DScene &s, uint32_t w, uint32_t h) {
+rt::Camera make_camera(const rt_camera &s, uint32_t w, uint32_t h) {
     rt::Camera c;
-    c.pos = rt::mk3(s.cam_pos[0], s.cam_pos[1], s.cam_pos[2]);
-    c.right = rt::mk3(s.cam_right[0], s.cam_right[1], s.cam_right[2]);
-    c.up = rt::mk3(s.cam_up[0], s.cam_up[1], s.cam_up[2]);
-    c.fwd = rt::mk3(s.cam_fwd[0], s.cam_fwd[1], s.cam_fwd[2]);
+    c.pos = rt::mk3(s.position[0], s.position[1], s.position[2]);
+    c.right = rt::mk3(s.right[0], s.right[1], s.right[2]);
+    c.up = rt::mk3(s.up[0], s.up[1], s.up[2]);
+    c.fwd = rt::mk3(s.forward[0], s.forward[1], s.forward[2]);
     // tan(fov_x / 2) and Camera::fov_y (scene.h:69-71), evaluated on the host exactly like the reference
     c.tan_half_x = std::tan(s.fov_x / 2);
     const float fov_y = std::atan(std::tan(s.fov_x / 2) * static_cast<float>(h) / static_cast<float>(w)) * 2;
@@ -523,6 +526,25 @@ rt::Camera make_camera(const DScene &s, uint32_t w, uint32_t h) {
     c.inv_h2 = 2.0f / static_cast<float>(h);
     return c;
 }
+
+// The camera of the uploaded triangle scene (rt_scene_desc.camera)
+rt_camera scene_camera(const DScene &s) {
+    rt_camera c;
+    for (int k = 0; k < 3; ++k) {
+        c.position[k] = s.cam_pos[k];
+        c.right[k] = s.cam_right[k];
+        c.up[k] = s.cam_up[k];
+        c.forward[k] = s.cam_fwd[k];
+    }
+    c.fov_x = s.fov_x;
+    return c;
+}
+
+// The cameras of a multi-view render (rt_gpu_render_views), one per view, and the Philox key of its first view
+struct ViewSet {
+    std::vector<rt::Camera> cams;
+    uint32_t view_base = 0;
+};
 
 void mark(rt_gpu_ctx *ctx, DeviceState &d, int kind) {
     if (!ctx->profiling) return;
@@ -555,17 +577,7 @@ int enqueue_text_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt
     const unsigned long long hs[4] = {0, 0, 0, ids_mode ? 0ull : static_cast<unsigned long long>(n_render) * (s_end - s_begin)};
     CU_CHECK(cudaMemcpyAsync(d.stats.p, hs, sizeof hs, cudaMemcpyHostToDevice, d.stream));
     if (n_render > 0 && (ids_mode || (s_end > s_begin && d.tscene.ray_depth > 0))) {
-        rt::Camera cam;
-        DScene tmp;
-        std::memset(&tmp, 0, sizeof tmp);
-        for (int k = 0; k < 3; ++k) {
-            tmp.cam_pos[k] = d.tcamera.position[k];
-            tmp.cam_right[k] = d.tcamera.right[k];
-            tmp.cam_up[k] = d.tcamera.up[k];
-            tmp.cam_fwd[k] = d.tcamera.forward[k];
-        }
-        tmp.fov_x = d.tcamera.fov_x;
-        cam = make_camera(tmp, W, H);
+        const rt::Camera cam = make_camera(d.tcamera, W, H);
         rtt::TextParams tp;
         tp.width = W;
         tp.height = H;
@@ -697,13 +709,17 @@ int enqueue_bounces(rt_gpu_ctx *ctx, DeviceState &d, const rt::BatchParams &bp, 
     return RT_OK;
 }
 
-// Enqueue the whole render of samples [s_begin, s_end) on device d (asynchronous).
+// Enqueue the whole render of samples [s_begin, s_end) on device d (asynchronous).  views != nullptr: the stacked image
+// of its views (views.cuh), rp's pixel range indexing it.
 int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_render_params &rp, uint32_t s_begin, uint32_t s_end,
-                   uint64_t &launches) {
+                   const ViewSet *views, uint64_t &launches) {
     CU_CHECK(cudaSetDevice(d.device));
     const uint32_t W = rp.width, H = rp.height, depth = d.scene.ray_depth;
-    const size_t n_pix = static_cast<size_t>(W) * H;
-    const rt::Camera cam = make_camera(d.scene, W, H);
+    const uint32_t n_views = views ? static_cast<uint32_t>(views->cams.size()) : 1u;
+    const size_t n_pix = static_cast<size_t>(W) * H * n_views;
+    const rt::Camera cam = make_camera(scene_camera(d.scene), W, H);
+    // stacked pixel + key_offset = Philox pixel key; fits 32 bits (rt_gpu_render_views checks (view_base + V) * W * H)
+    const uint32_t key_offset = views ? static_cast<uint32_t>(static_cast<uint64_t>(views->view_base) * W * H) : 0u;
     if (int rc = d.accum.alloc(n_pix)) return rc;
     if (int rc = d.stats.alloc(4)) return rc;
     CU_CHECK(cudaMemsetAsync(d.stats.p, 0, 4 * sizeof(unsigned long long), d.stream));
@@ -735,6 +751,8 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
     const size_t n_counters = n_counters_of(qdepth);
     if (int rc = d.counters.alloc(n_counters)) return rc;
     const rt::Queues q_gen = queues_of(d, qdepth, -1);
+    if (views)
+        if (int rc = d.cams.upload(views->cams, d.stream)) return rc;
     // per-kernel profiling needs the kernels one after the other on one stream
     const bool split_allowed = !ids_mode && !ctx->profiling && !std::getenv("RT_NO_SPLIT");
 
@@ -756,10 +774,13 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
             bp.npix = npix;
             bp.s0 = s0;
             bp.k = std::min(k_max, s_end - s0);
-            bp.tiled = !ids_mode && pix0 == 0 && npix == n_pix && W % 8 == 0 && H % 4 == 0 && !std::getenv("RT_NO_TILES");
+            bp.tiled = !ids_mode && pix0 == 0 && npix == n_pix && W % 8 == 0 && (H * n_views) % 4 == 0 && !std::getenv("RT_NO_TILES");
             const uint32_t n = bp.npix * bp.k;
             CU_CHECK(cudaMemsetAsync(d.counters.p, 0, n_counters * sizeof(uint32_t), d.stream));
-            rt::k_generate<<<(n + 255) / 256, 256, 0, d.stream>>>(cam, bp, q_gen);
+            if (views)
+                rt::k_generate_views<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, bp, q_gen, key_offset);
+            else
+                rt::k_generate<<<(n + 255) / 256, 256, 0, d.stream>>>(cam, bp, q_gen);
             mark(ctx, d, K_GENERATE);
             if (ids_mode) {  // pixel-centre rays through the same traversal kernel, then hit -> scene.objects id
                 RT_K_EXTEND<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, queues_of(d, qdepth, 0), 0, 0x3F800000u);
@@ -769,7 +790,9 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
                 launches += 3;
                 continue;
             }
-            if (int rc = enqueue_bounces(ctx, d, bp, n, split_allowed, launches)) return rc;
+            rt::BatchParams bp_key = bp;  // k_shade's radiance slot: (sample - s0) * npix + (key - pix0)
+            bp_key.pix0 += key_offset;
+            if (int rc = enqueue_bounces(ctx, d, bp_key, n, split_allowed, launches)) return rc;
             rt::k_accumulate<<<(bp.npix + 255) / 256, 256, 0, d.stream>>>(bp, d.rad, d.accum.p);
             mark(ctx, d, K_ACCUMULATE);
             launches += 2;
@@ -835,7 +858,7 @@ int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp
     bp.k1 = static_cast<uint32_t>(rp.seed >> 32);
     bp.centre = 0;
     bp.tiled = 0;  // queue 0 follows the active list, whose first form is already in tiles where that applies
-    run.cam = make_camera(d.scene, rp.width, rp.height);
+    run.cam = make_camera(scene_camera(d.scene), rp.width, rp.height);
     d.marks.clear();
     d.events_used = 0;
     CU_CHECK(cudaEventRecord(d.ev_begin, d.stream));
@@ -1047,7 +1070,7 @@ void rt_gpu_destroy(rt_gpu_ctx *ctx) {
         d.alist.release(); d.awords.release(); d.acounts.release(); d.actr.release(); d.aerr.release();
         d.in_pos.release(); d.in_nrm.release(); d.in_uv.release(); d.in_tan.release(); d.in_mat.release(); d.build_scratch.release();
         d.counters.release(); d.stats.release();
-        d.prim_ids.release(); d.rgb8.release();
+        d.prim_ids.release(); d.rgb8.release(); d.cams.release();
         for (cudaEvent_t e : d.event_pool) cudaEventDestroy(e);
         for (cudaEvent_t e : {d.ev_begin, d.ev_end, d.ev_red0, d.ev_red1, d.ev_a, d.ev_b, d.ev_light, d.ev_round[0], d.ev_round[1]})
             if (e) cudaEventDestroy(e);
@@ -1263,22 +1286,14 @@ int finish_render(rt_gpu_ctx *ctx, const rt_render_params &rp, uint64_t launches
     return RT_OK;
 }
 
-}  // namespace
+// Pixels of the last render's image: width * height, times the views of a multi-view render
+size_t last_pixels(const rt_gpu_ctx *ctx) {
+    return static_cast<size_t>(ctx->last.width) * ctx->last.height * std::max(ctx->last_views, 1u);
+}
 
-int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
-    if (!ctx || !params) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: null argument");
-    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render: no scene uploaded");
-    rt_render_params rp = *params;
-    if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull)
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal image size");
-    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: samples == 0");
-    if (rp.sample_end == 0) rp.sample_end = rp.samples;
-    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: sample_begin > sample_end");
-    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height;
-    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
-    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal pixel range");
-    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY && ctx->adaptive_sums)
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: RT_FLAG_ACCUMULATE onto the sums of an adaptive render (per-pixel sample counts)");
+// The render of rt_gpu_render (views == nullptr) and rt_gpu_render_views over every device of the handle; rp is
+// validated and its sample_end / pixel_end resolved.
+int render_on_devices(rt_gpu_ctx *ctx, const rt_render_params &rp, const ViewSet *views) {
     const int n = static_cast<int>(ctx->devs.size());
     const uint32_t total = rp.sample_end - rp.sample_begin;
     uint64_t launches = 0;
@@ -1302,20 +1317,78 @@ int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
         DeviceState &dg = *ctx->devs[g];
         if (ctx->text_scene) {
             if (int rc = enqueue_text_render(ctx, dg, g, local, sb, se, launches)) return rc;
-        } else if (int rc = enqueue_render(ctx, dg, g, local, sb, se, launches)) {
+        } else if (int rc = enqueue_render(ctx, dg, g, local, sb, se, views, launches)) {
             return rc;
         }
         // the work counters travel on the stream into pinned memory: no second synchronising copy after the render
         CU_CHECK(cudaMemcpyAsync(dg.h_stats, dg.stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, dg.stream));
     }
+    const size_t n_pix = static_cast<size_t>(rp.width) * rp.height * (views ? views->cams.size() : 1);
     if (n > 1 && rp.mode == RT_MODE_BEAUTY)
-        if (int rc = reduce_to_device0(ctx, static_cast<size_t>(rp.width) * rp.height, false)) return rc;
+        if (int rc = reduce_to_device0(ctx, n_pix, false)) return rc;
     if (int rc = finish_render(ctx, rp, launches)) return rc;
     ctx->last = rp;
+    ctx->last_views = views ? static_cast<uint32_t>(views->cams.size()) : 0u;
     ctx->have_render = true;
     ctx->adaptive = false;
     if (rp.mode == RT_MODE_BEAUTY) ctx->adaptive_sums = false;
     return RT_OK;
+}
+
+}  // namespace
+
+int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
+    if (!ctx || !params) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render: no scene uploaded");
+    rt_render_params rp = *params;
+    if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal image size");
+    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: samples == 0");
+    if (rp.sample_end == 0) rp.sample_end = rp.samples;
+    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: sample_begin > sample_end");
+    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height;
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: illegal pixel range");
+    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY && ctx->adaptive_sums)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: RT_FLAG_ACCUMULATE onto the sums of an adaptive render (per-pixel sample counts)");
+    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY && ctx->have_render && ctx->last_views != 0 &&
+        (ctx->last_views != 1 || ctx->last.width != rp.width || ctx->last.height != rp.height))
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render: RT_FLAG_ACCUMULATE onto the sums of a multi-view render of another shape");
+    return render_on_devices(ctx, rp, nullptr);
+}
+
+int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views) {
+    if (!ctx || !params || !views) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render_views: no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: not available for course text scenes");
+    if (views->n_views == 0 || !views->cameras) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: no views / null cameras");
+    rt_render_params rp = *params;
+    const uint64_t per_view = static_cast<uint64_t>(rp.width) * rp.height, V = views->n_views;
+    if (per_view == 0 || per_view > 0x7FFFFFFFull || per_view * V > 0x7FFFFFFFull)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: illegal image size (the stacked image has n_views * width * height pixels)");
+    if ((views->view_base + V) * per_view > (1ull << 32))
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: (view_base + n_views) * width * height exceeds the 32-bit pixel key");
+    for (uint32_t v = 0; v < views->n_views; ++v) {
+        const rt_camera &c = views->cameras[v];
+        bool finite = std::isfinite(c.fov_x);
+        for (int k = 0; k < 3; ++k)
+            finite = finite && std::isfinite(c.position[k]) && std::isfinite(c.right[k]) && std::isfinite(c.up[k]) && std::isfinite(c.forward[k]);
+        if (!finite) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: camera " + std::to_string(v) + " has a non-finite value");
+    }
+    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: samples == 0");
+    if (rp.sample_end == 0) rp.sample_end = rp.samples;
+    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: sample_begin > sample_end");
+    const uint64_t n_pixels = per_view * V;
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: illegal pixel range");
+    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY &&
+        (!ctx->have_render || ctx->adaptive_sums || ctx->last.width != rp.width || ctx->last.height != rp.height ||
+         std::max(ctx->last_views, 1u) != views->n_views))
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: RT_FLAG_ACCUMULATE needs a previous render of the same width, height and n_views");
+    ViewSet vs;
+    vs.view_base = views->view_base;
+    for (uint32_t v = 0; v < views->n_views; ++v) vs.cams.push_back(make_camera(views->cameras[v], rp.width, rp.height));
+    return render_on_devices(ctx, rp, &vs);
 }
 
 int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_adaptive_params *ap) {
@@ -1359,6 +1432,7 @@ int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, cons
         }
     }
     ctx->last = rp;
+    ctx->last_views = 0;
     ctx->last_adaptive = *ap;
     ctx->have_render = true;
     ctx->adaptive = ctx->adaptive_sums = true;
@@ -1391,7 +1465,7 @@ int rt_gpu_readback(rt_gpu_ctx *ctx, float *rgb_mean, int32_t *prim_ids, rt_stat
     if (!ctx->have_render) return fail(RT_ERR_NO_RENDER, "rt_gpu_readback: nothing rendered");
     DeviceState &d = *ctx->devs[0];
     CU_CHECK(cudaSetDevice(d.device));
-    const size_t n_pix = static_cast<size_t>(ctx->last.width) * ctx->last.height;
+    const size_t n_pix = last_pixels(ctx);
     if (rgb_mean) {
         if (ctx->last.mode != RT_MODE_BEAUTY) return fail(RT_ERR_NO_RENDER, "rt_gpu_readback: last render was not a beauty render");
         // the division and the float4 -> rgb packing run on the device (12 B per pixel cross the bus instead of 16);
@@ -1446,7 +1520,7 @@ int rt_gpu_accum_device_ptr(rt_gpu_ctx *ctx, void **dptr, size_t *n_floats) {
     if (!ctx || !dptr) return fail(RT_ERR_INVALID_ARG, "rt_gpu_accum_device_ptr: null argument");
     if (!ctx->have_render || ctx->last.mode != RT_MODE_BEAUTY) return fail(RT_ERR_NO_RENDER, "rt_gpu_accum_device_ptr: no beauty render");
     *dptr = ctx->devs[0]->accum.p;
-    if (n_floats) *n_floats = static_cast<size_t>(ctx->last.width) * ctx->last.height * 4;
+    if (n_floats) *n_floats = last_pixels(ctx) * 4;
     return RT_OK;
 }
 
@@ -1455,7 +1529,7 @@ int rt_gpu_readback_rgb8(rt_gpu_ctx *ctx, uint8_t *rgb8) {
     if (!ctx->have_render || ctx->last.mode != RT_MODE_BEAUTY) return fail(RT_ERR_NO_RENDER, "rt_gpu_readback_rgb8: no beauty render");
     DeviceState &d = *ctx->devs[0];
     CU_CHECK(cudaSetDevice(d.device));
-    const uint32_t n_pix = ctx->last.width * ctx->last.height;
+    const uint32_t n_pix = static_cast<uint32_t>(last_pixels(ctx));
     if (int rc = d.rgb8.alloc(static_cast<size_t>(n_pix) * 3)) return rc;
     if (ctx->adaptive_sums)
         rt::k_tonemap_counts<<<(n_pix + 255) / 256, 256, 0, d.stream>>>(d.accum.p, d.acounts.p, n_pix, d.rgb8.p);

@@ -22,7 +22,7 @@ import os
 import numpy as np
 
 from . import host
-from ._abi import MATERIAL_DTYPE, TEXTURE_DTYPE, SceneData
+from ._abi import MATERIAL_DTYPE, TEXTURE_DTYPE, Camera, SceneData
 
 F = np.float32
 _libm = ctypes.CDLL(ctypes.util.find_library("m") or "libm.so.6")
@@ -177,6 +177,7 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
         return buffers[int(view["buffer"])][off:off + count * dt.itemsize].view(dt).astype(np.int64)
 
     cam = {}
+    cameras = []  # every camera node, in traversal order; the reference keeps only the last (cam)
     pos_chunks, nrm_chunks, uv_chunks, tan_chunks, mat_chunks = [], [], [], [], []
     materials = []
     mat_index = {}
@@ -243,6 +244,7 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
             cam["up"] = col_dir(np.array([0, 1, 0], F))
             cam["right"] = col_dir(np.array([1, 0, 0], F))
             cam["fov_x"] = F(atanf(F(tanf(F(fov_y / F(2))) * ar)) * F(2))
+            cameras.append(Camera(cam["position"], cam["right"], cam["up"], cam["forward"], cam["fov_x"]))
 
         if "mesh" in node:
             for prim in doc["meshes"][int(node["mesh"])]["primitives"]:
@@ -295,6 +297,7 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
         handle_node(int(n), np.eye(4, dtype=F))
 
     s = SceneData()
+    s.cameras = cameras
     if cam:
         s.camera_position, s.camera_right = cam["position"], cam["right"]
         s.camera_up, s.camera_forward, s.fov_x = cam["up"], cam["forward"], cam["fov_x"]

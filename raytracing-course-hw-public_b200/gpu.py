@@ -6,8 +6,8 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_render_params, rt_scene_desc,
-                   rt_stats)
+from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_camera, rt_render_params,
+                   rt_scene_desc, rt_stats, rt_views)
 
 # RT_GPU_LIB selects another build of the same C ABI (kernel A/B experiments, tools/build_variants.sh)
 LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu.so")
@@ -15,7 +15,8 @@ LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu
 # every symbol include/rt_gpu.h declares
 SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upload_text_scene", "rt_gpu_render", "rt_gpu_readback",
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
-           "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive"]
+           "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive",
+           "rt_gpu_render_views"]
 
 _lib = None
 
@@ -32,6 +33,7 @@ def lib():
         L.rt_gpu_render.argtypes = [C.c_void_p, C.POINTER(rt_render_params)]
         L.rt_gpu_readback.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_gpu_render_adaptive.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params)]
+        L.rt_gpu_render_views.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views)]
         L.rt_gpu_readback_adaptive.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.rt_gpu_accum_device_ptr.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
         L.rt_gpu_readback_rgb8.argtypes = [C.c_void_p, C.c_void_p]
@@ -66,6 +68,7 @@ class RtGpu:
         self.n_gpus = n_gpus
         self._scene = None
         self._last = None
+        self._views = None  # views of the last render when it was render_views: readbacks are [V, H, W, ...]
 
     def close(self):
         if self._h:
@@ -104,6 +107,25 @@ class RtGpu:
                              RT_FLAG_ACCUMULATE if accumulate else 0, pixel_begin, pixel_end)
         _check(lib().rt_gpu_render(self._h, C.byref(p)), "rt_gpu_render")
         self._last = (width, height, mode)
+        self._views = None
+
+    def render_views(self, cameras, width, height, samples, seed=0, view_base=0, sample_begin=0, sample_end=0,
+                     mode=RT_MODE_BEAUTY, max_paths_in_flight=0, accumulate=False, pixel_begin=0, pixel_end=0):
+        """Multi-view render (rt_gpu_render_views): every Camera of `cameras` over the uploaded scene in one call, the
+        views stacked into one image of W x (V * H) pixels (pixel_begin / pixel_end index it).  Pixel p of view v is
+        keyed (view_base + v) * W * H + p, so view v equals a one-view call with view_base = v.  readback() and
+        readback_rgb8() then return [V, H, W, 3]."""
+        cams = (rt_camera * max(len(cameras), 1))(*[c.to_c() for c in cameras])
+        v = rt_views(len(cameras), view_base, cams)
+        p = rt_render_params(width, height, samples, sample_begin, sample_end, mode, seed, max_paths_in_flight,
+                             RT_FLAG_ACCUMULATE if accumulate else 0, pixel_begin, pixel_end)
+        _check(lib().rt_gpu_render_views(self._h, C.byref(p), C.byref(v)), "rt_gpu_render_views")
+        self._last = (width, height, mode)
+        self._views = len(cameras)
+
+    def _shape(self, *tail):
+        w, h, _ = self._last
+        return ((self._views,) if self._views is not None else ()) + (h, w) + tail
 
     def render_adaptive(self, width, height, max_samples, min_samples, step_samples, rel_error, abs_floor=1e-3, seed=0,
                         max_paths_in_flight=0, pixel_begin=0, pixel_end=0):
@@ -115,6 +137,7 @@ class RtGpu:
         a = rt_adaptive_params(min_samples, step_samples, rel_error, abs_floor)
         _check(lib().rt_gpu_render_adaptive(self._h, C.byref(p), C.byref(a)), "rt_gpu_render_adaptive")
         self._last = (width, height, RT_MODE_BEAUTY)
+        self._views = None
 
     def readback_adaptive(self):
         """(sample counts uint32 [H, W], err float32 [H, W]) of the last adaptive render."""
@@ -126,9 +149,8 @@ class RtGpu:
         return counts, err
 
     def readback(self):
-        """(rgb_mean float32 [H, W, 3], stats dict) of the last beauty render."""
-        w, h, _ = self._last
-        out = np.empty((h, w, 3), np.float32)
+        """(rgb_mean float32 [H, W, 3], or [V, H, W, 3] after render_views; stats dict) of the last beauty render."""
+        out = np.empty(self._shape(3), np.float32)
         st = rt_stats()
         _check(lib().rt_gpu_readback(self._h, out.ctypes.data_as(C.c_void_p), None, C.byref(st)), "rt_gpu_readback")
         return out, st.as_dict()
@@ -145,14 +167,17 @@ class RtGpu:
         return st.as_dict()
 
     def readback_rgb8(self):
-        w, h, _ = self._last
-        out = np.empty((h, w, 3), np.uint8)
+        out = np.empty(self._shape(3), np.uint8)
         _check(lib().rt_gpu_readback_rgb8(self._h, out.ctypes.data_as(C.c_void_p)), "rt_gpu_readback_rgb8")
         return out
 
-    def primary_ids(self, width, height):
-        self.render(width, height, 1, mode=RT_MODE_PRIMARY_IDS)
-        ids = np.empty((height, width), np.int32)
+    def primary_ids(self, width, height, cameras=None, view_base=0):
+        """Primary-hit ids [H, W] of the scene's camera, or [V, H, W] of `cameras` (render_views)."""
+        if cameras is None:
+            self.render(width, height, 1, mode=RT_MODE_PRIMARY_IDS)
+        else:
+            self.render_views(cameras, width, height, 1, view_base=view_base, mode=RT_MODE_PRIMARY_IDS)
+        ids = np.empty(self._shape(), np.int32)
         _check(lib().rt_gpu_readback(self._h, None, ids.ctypes.data_as(C.c_void_p), None), "rt_gpu_readback")
         return ids
 
