@@ -59,7 +59,7 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT8_MINB)
     uint32_t gx = kDone8, gy = 0;  // current group
     uint32_t tx = 0, ty = 0;       // postponed triangle group
     uint32_t ray = kNoRay;         // bit 31: pending (its light pdf is wanted)
-    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 1), idir = mk3(0, 0, 1), ood = mk3(0, 0, 0);
+    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 1), idir = mk3(0, 0, 1);
     uint32_t octinv = 0;
     float best_t = INFINITY, best_b = 0.0f, best_c = 0.0f;
     int32_t best_tri = -1;
@@ -112,7 +112,6 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT8_MINB)
                 o = mk3(o4.x, o4.y, o4.z);
                 d = mk3(d4.x, d4.y, d4.z);
                 idir = mk3(rcp_rn(d.x), rcp_rn(d.y), rcp_rn(d.z));
-                ood = mk3(o.x * idir.x, o.y * idir.y, o.z * idir.z);
                 octinv = (idir.x < 0.0f ? 0u : 1u) | (idir.y < 0.0f ? 0u : 2u) | (idir.z < 0.0f ? 0u : 4u);
                 best_t = INFINITY;
                 best_b = best_c = 0.0f;
@@ -184,7 +183,7 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT8_MINB)
                     if (gy >> 24) push(gx, gy);
                     const char *np = reinterpret_cast<const char *>(node_base + child);
                     const f8 h = ld8(np), ga = ld8(np + 32), gb = ld8(np + 64);
-                    const Grid3 g = qgrid(f2u(h.a), f2u(h.b), f2u(h.c), idir, ood);
+                    const Grid3 g = qgrid(f2u(h.a), f2u(h.b), f2u(h.c), idir, o);
                     const bool px = !(idir.x < 0.0f), py = !(idir.y < 0.0f), pz = !(idir.z < 0.0f);
                     const uint32_t hs =
                         q8_group_hits(f2u(ga.a), f2u(ga.b), f2u(ga.c), f2u(ga.d), f2u(ga.e), f2u(ga.f), g, px, py, pz, one, eps, best_t) |

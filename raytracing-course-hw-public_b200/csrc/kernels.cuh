@@ -316,7 +316,7 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT_MINB)
     int32_t link = kLinkDone;  // >= 0 inner node, kLinkPop / kLinkDone, otherwise a leaf (~first triangle)
     int32_t leaf = 0;          // postponed leaf link (always < 0) or 0 = none
     uint32_t ray = kNoRay;     // queue index; bit 31: pending (its light pdf is wanted)
-    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 1), idir = mk3(0, 0, 1), ood = mk3(0, 0, 0);
+    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 1), idir = mk3(0, 0, 1);
     float best_t = INFINITY, best_b = 0.0f, best_c = 0.0f;
     int32_t best_tri = -1;
 #if RT_LIGHT_KERNEL
@@ -370,7 +370,6 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT_MINB)
                 o = mk3(o4.x, o4.y, o4.z);
                 d = mk3(d4.x, d4.y, d4.z);
                 idir = mk3(rcp_rn(d.x), rcp_rn(d.y), rcp_rn(d.z));
-                ood = mk3(o.x * idir.x, o.y * idir.y, o.z * idir.z);
                 best_t = INFINITY;
                 best_b = best_c = 0.0f;
                 best_tri = -1;
@@ -459,7 +458,7 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT_MINB)
                     const f8 na = ld8h<RT_EXT_NODE_L1>(np), nb = ld8h<RT_EXT_NODE_L1>(np + 32);  // 64 B node: grid, 6 plane words, 4 links
 #endif
                     const Node4Test nt = qnode4_test(f2u(na.a), f2u(na.b), f2u(na.c), f2u(na.d), f2u(na.e), f2u(na.f), f2u(na.g),
-                                                     f2u(na.h), f2u(nb.a), idir, ood, one, eps, best_t);
+                                                     f2u(na.h), f2u(nb.a), idir, o, one, eps, best_t);
                     float d0 = nt.d[0], d1 = nt.d[1], d2 = nt.d[2], d3 = nt.d[3];
                     int32_t l0 = static_cast<int32_t>(f2u(nb.b)), l1 = static_cast<int32_t>(f2u(nb.c));
                     int32_t l2 = static_cast<int32_t>(f2u(nb.d)), l3 = static_cast<int32_t>(f2u(nb.e));
@@ -564,7 +563,7 @@ struct LightBox {
 };
 constexpr int kLightThreads = 256;
 
-__device__ __forceinline__ float light_traverse(const DBvh &lbvh, const DLight *__restrict__ light_extra, f3 o, f3 d, f3 idir, f3 ood,
+__device__ __forceinline__ float light_traverse(const DBvh &lbvh, const DLight *__restrict__ light_extra, f3 o, f3 d, f3 idir,
                                                 float eps, uint32_t one) {
     int32_t stack[RT_EXT_STACK_CAP];  // the upload bounds the need of an unordered traversal as well (stack_need4)
     int sp = 0;
@@ -575,7 +574,7 @@ __device__ __forceinline__ float light_traverse(const DBvh &lbvh, const DLight *
             const char *np = reinterpret_cast<const char *>(lbvh.qnodes4 + link);
             const f8 na = ld8(np), nb = ld8(np + 32);
             const Node4Test nt = qnode4_test(f2u(na.a), f2u(na.b), f2u(na.c), f2u(na.d), f2u(na.e), f2u(na.f), f2u(na.g), f2u(na.h),
-                                             f2u(nb.a), idir, ood, one, eps, INFINITY);
+                                             f2u(nb.a), idir, o, one, eps, INFINITY);
             const int32_t l[4] = {static_cast<int32_t>(f2u(nb.b)), static_cast<int32_t>(f2u(nb.c)), static_cast<int32_t>(f2u(nb.d)),
                                   static_cast<int32_t>(f2u(nb.e))};
             link = kLinkPop;
@@ -636,8 +635,7 @@ __global__ void __launch_bounds__(kLightThreads) k_lightpdf_list(DBvh lbvh, cons
         }
         const f3 o = mk3(o4.x, o4.y, o4.z), d = mk3(d4.x, d4.y, d4.z);
         const f3 idir = mk3(rcp_rn(d.x), rcp_rn(d.y), rcp_rn(d.z));
-        const f3 ood = mk3(o.x * idir.x, o.y * idir.y, o.z * idir.z);
-        q_store<0>(q.lpdf + i_cur, light_traverse(lbvh, light_extra, o, d, idir, ood, eps, one) * inv_n_lights);
+        q_store<0>(q.lpdf + i_cur, light_traverse(lbvh, light_extra, o, d, idir, eps, one) * inv_n_lights);
         if (!more) break;
         j += stride;
         i_cur = i_nxt;

@@ -263,10 +263,11 @@ RT_HD uint32_t swz(uint32_t w, uint32_t sel) {
 }
 
 RT_HD NodeTest qnode_test(const uint32_t ox, const uint32_t oy, const uint32_t oz, const uint32_t q0, const uint32_t q1,
-                          const uint32_t q2, f3 idir, f3 ood, RaySwz sw, uint32_t one, float eps, float best_t) {
-    const float ax = u2f((ox << 23) + 0x08000000u) * idir.x, bx = fmaf(u2f(ox), idir.x, -ood.x) - ax;
-    const float ay = u2f((oy << 23) + 0x08000000u) * idir.y, by = fmaf(u2f(oy), idir.y, -ood.y) - ay;
-    const float az = u2f((oz << 23) + 0x08000000u) * idir.z, bz = fmaf(u2f(oz), idir.z, -ood.z) - az;
+                          const uint32_t q2, f3 idir, f3 o, RaySwz sw, uint32_t one, float eps, float best_t) {
+    // ray-space planes as in qnode4_test: subtract the ray origin before the multiply
+    const float ax = u2f((ox << 23) + 0x08000000u) * idir.x, bx = fmaf(u2f(ox) - o.x, idir.x, -ax);
+    const float ay = u2f((oy << 23) + 0x08000000u) * idir.y, by = fmaf(u2f(oy) - o.y, idir.y, -ay);
+    const float az = u2f((oz << 23) + 0x08000000u) * idir.z, bz = fmaf(u2f(oz) - o.z, idir.z, -az);
     const uint32_t wx = swz(q0, sw.x), wy = swz(q1, sw.y), wz = swz(q2, sw.z);
     // slab test of both children (bvh.h:137-152): entry = max of the three near planes, exit = min of the three far
     // planes, interval clipped to [eps, best_t] (hit <=> entry <= exit): visits the boxes
@@ -291,7 +292,6 @@ RT_HD Hit closest_hit_q(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *st
     best.tri = -1;
     if (bvh.root == RT_LINK_NONE) return best;
     const f3 idir = mk3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
-    const f3 ood = mk3(o.x * idir.x, o.y * idir.y, o.z * idir.z);
     const RaySwz sw = ray_swizzle(idir);
     int32_t stack_link[RT_STACK_SIZE];
     float stack_t[RT_STACK_SIZE];
@@ -301,7 +301,7 @@ RT_HD Hit closest_hit_q(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *st
         if (link >= 0) {
             if (steps) ++*steps;
             const f8 nq = ld8(bvh.qnodes + link);
-            const NodeTest nt = qnode_test(f2u(nq.a), f2u(nq.b), f2u(nq.c), f2u(nq.d), f2u(nq.e), f2u(nq.f), idir, ood, sw,
+            const NodeTest nt = qnode_test(f2u(nq.a), f2u(nq.b), f2u(nq.c), f2u(nq.d), f2u(nq.e), f2u(nq.f), idir, o, sw,
                                            qnode_one(), min_dst, best.t);
             const int32_t ll = static_cast<int32_t>(f2u(nq.g)), lr = static_cast<int32_t>(f2u(nq.h));
             if (nt.hl || nt.hr) {
@@ -375,11 +375,16 @@ RT_HD void q4_axis(uint32_t w, float a, float b, uint32_t one, float t[4]) {
 #endif
 }
 RT_HD Node4Test qnode4_test(const uint32_t ox, const uint32_t oy, const uint32_t oz, const uint32_t lox, const uint32_t loy,
-                            const uint32_t loz, const uint32_t hix, const uint32_t hiy, const uint32_t hiz, f3 idir, f3 ood,
+                            const uint32_t loz, const uint32_t hix, const uint32_t hiy, const uint32_t hiz, f3 idir, f3 o,
                             uint32_t one, float eps, float best_t) {
-    const float ax = u2f((ox << 23) + 0x08000000u) * idir.x, bx = fmaf(u2f(ox), idir.x, -ood.x) - ax;
-    const float ay = u2f((oy << 23) + 0x08000000u) * idir.y, by = fmaf(u2f(oy), idir.y, -ood.y) - ay;
-    const float az = u2f((oz << 23) + 0x08000000u) * idir.z, bz = fmaf(u2f(oz), idir.z, -ood.z) - az;
+    // plane t = (org + q * cell - o) / d = fma(1 + q * 2^-16, ax, bx).  The grid origin is subtracted from the ray origin
+    // BEFORE the multiply (bvh.h:137-152 does the same), so the rounding error of bx is relative to |org - o|, the
+    // ray's distance to the node.  The former fma(org, 1/d, -o * (1/d)) rounded o * (1/d) first: an error relative to
+    // |o| itself, which outgrew the packer's 1/64-cell margin for small nodes ~1e3 of their extent away from the world
+    // origin, and those nodes lost hits.  Same instruction count (FADD + FFMA instead of FFMA + FADD per axis).
+    const float ax = u2f((ox << 23) + 0x08000000u) * idir.x, bx = fmaf(u2f(ox) - o.x, idir.x, -ax);
+    const float ay = u2f((oy << 23) + 0x08000000u) * idir.y, by = fmaf(u2f(oy) - o.y, idir.y, -ay);
+    const float az = u2f((oz << 23) + 0x08000000u) * idir.z, bz = fmaf(u2f(oz) - o.z, idir.z, -az);
     const bool px = !(idir.x < 0.0f), py = !(idir.y < 0.0f), pz = !(idir.z < 0.0f);
     const uint32_t nx = px ? lox : hix, fx = px ? hix : lox;
     const uint32_t ny = py ? loy : hiy, fy = py ? hiy : loy;
@@ -419,7 +424,6 @@ RT_HD Hit closest_hit_q4(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *s
     best.tri = -1;
     if (bvh.root4 == RT_LINK_NONE) return best;
     const f3 idir = mk3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
-    const f3 ood = mk3(o.x * idir.x, o.y * idir.y, o.z * idir.z);
     int32_t stack_link[RT_STACK_SIZE * 2];
     float stack_t[RT_STACK_SIZE * 2];
     int sp = 0;
@@ -430,7 +434,7 @@ RT_HD Hit closest_hit_q4(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *s
             const char *p = reinterpret_cast<const char *>(bvh.qnodes4 + link);
             const f8 na = ld8(p), nb = ld8(p + 32);
             const Node4Test nt = qnode4_test(f2u(na.a), f2u(na.b), f2u(na.c), f2u(na.d), f2u(na.e), f2u(na.f), f2u(na.g),
-                                             f2u(na.h), f2u(nb.a), idir, ood, qnode_one(), min_dst, best.t);
+                                             f2u(na.h), f2u(nb.a), idir, o, qnode_one(), min_dst, best.t);
             float d0 = nt.d[0], d1 = nt.d[1], d2 = nt.d[2], d3 = nt.d[3];
             int32_t l0 = static_cast<int32_t>(f2u(nb.b)), l1 = static_cast<int32_t>(f2u(nb.c));
             int32_t l2 = static_cast<int32_t>(f2u(nb.d)), l3 = static_cast<int32_t>(f2u(nb.e));
@@ -503,11 +507,11 @@ RT_HD uint32_t oct_permute(uint32_t m, uint32_t octinv) {
 struct Grid3 {
     float ax, bx, ay, by, az, bz;
 };
-RT_HD Grid3 qgrid(uint32_t ox, uint32_t oy, uint32_t oz, f3 idir, f3 ood) {
+RT_HD Grid3 qgrid(uint32_t ox, uint32_t oy, uint32_t oz, f3 idir, f3 o) {  // ray-space grid as in qnode4_test
     Grid3 g;
-    g.ax = u2f((ox << 23) + 0x08000000u) * idir.x, g.bx = fmaf(u2f(ox), idir.x, -ood.x) - g.ax;
-    g.ay = u2f((oy << 23) + 0x08000000u) * idir.y, g.by = fmaf(u2f(oy), idir.y, -ood.y) - g.ay;
-    g.az = u2f((oz << 23) + 0x08000000u) * idir.z, g.bz = fmaf(u2f(oz), idir.z, -ood.z) - g.az;
+    g.ax = u2f((ox << 23) + 0x08000000u) * idir.x, g.bx = fmaf(u2f(ox) - o.x, idir.x, -g.ax);
+    g.ay = u2f((oy << 23) + 0x08000000u) * idir.y, g.by = fmaf(u2f(oy) - o.y, idir.y, -g.ay);
+    g.az = u2f((oz << 23) + 0x08000000u) * idir.z, g.bz = fmaf(u2f(oz) - o.z, idir.z, -g.az);
     return g;
 }
 // slab test of child C of a plane group: entry (max of the near planes, eps) <= exit (min of the far planes, best_t)
@@ -543,7 +547,6 @@ RT_HD Hit closest_hit_q8(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *s
     best.tri = -1;
     if (bvh.n_nodes8 == 0) return best;
     const f3 idir = mk3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
-    const f3 ood = mk3(o.x * idir.x, o.y * idir.y, o.z * idir.z);
     const bool px = !(idir.x < 0.0f), py = !(idir.y < 0.0f), pz = !(idir.z < 0.0f);
     const uint32_t octinv = (px ? 1u : 0u) | (py ? 2u : 0u) | (pz ? 4u : 0u);
     uint32_t sx[RT_STACK_SIZE], sy[RT_STACK_SIZE];
@@ -562,7 +565,7 @@ RT_HD Hit closest_hit_q8(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *s
             if (steps) ++*steps;
             const char *np = reinterpret_cast<const char *>(bvh.qnodes8 + child);
             const f8 h = ld8(np), a = ld8(np + 32), b = ld8(np + 64);
-            const Grid3 g = qgrid(f2u(h.a), f2u(h.b), f2u(h.c), idir, ood);
+            const Grid3 g = qgrid(f2u(h.a), f2u(h.b), f2u(h.c), idir, o);
             const uint32_t hs = q8_group_hits(f2u(a.a), f2u(a.b), f2u(a.c), f2u(a.d), f2u(a.e), f2u(a.f), g, px, py, pz, qnode_one(), min_dst, best.t) |
                                 q8_group_hits(f2u(b.a), f2u(b.b), f2u(b.c), f2u(b.d), f2u(b.e), f2u(b.f), g, px, py, pz, qnode_one(), min_dst, best.t) << 4;
             const uint32_t imask = f2u(h.d), counts = f2u(h.g);
@@ -673,7 +676,6 @@ RT_HD Hit closest_hit(const DBvh &bvh, f3 o, f3 d, float min_dst) {
 RT_HD float light_pdf_q8(const DScene &s, f3 x, f3 dir) {
     const DBvh &bvh = s.light;
     const f3 idir = mk3(1.0f / dir.x, 1.0f / dir.y, 1.0f / dir.z);
-    const f3 ood = mk3(x.x * idir.x, x.y * idir.y, x.z * idir.z);
     const bool px = !(idir.x < 0.0f), py = !(idir.y < 0.0f), pz = !(idir.z < 0.0f);
     uint32_t sx[RT_STACK_SIZE], sy[RT_STACK_SIZE];
     int sp = 0;
@@ -691,7 +693,7 @@ RT_HD float light_pdf_q8(const DScene &s, f3 x, f3 dir) {
             }
             const char *np = reinterpret_cast<const char *>(bvh.qnodes8 + child);
             const f8 h = ld8(np), a = ld8(np + 32), b = ld8(np + 64);
-            const Grid3 g = qgrid(f2u(h.a), f2u(h.b), f2u(h.c), idir, ood);
+            const Grid3 g = qgrid(f2u(h.a), f2u(h.b), f2u(h.c), idir, x);
             const uint32_t hs = q8_group_hits(f2u(a.a), f2u(a.b), f2u(a.c), f2u(a.d), f2u(a.e), f2u(a.f), g, px, py, pz, qnode_one(), s.eps, INFINITY) |
                                 q8_group_hits(f2u(b.a), f2u(b.b), f2u(b.c), f2u(b.d), f2u(b.e), f2u(b.f), g, px, py, pz, qnode_one(), s.eps, INFINITY) << 4;
             const uint32_t imask = f2u(h.d), counts = f2u(h.g);

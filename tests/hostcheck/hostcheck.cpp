@@ -7,6 +7,7 @@
 #include <chrono>
 #include <cmath>
 #include <cstring>
+#include <thread>
 #include <vector>
 
 #include "pt_core.cuh"
@@ -401,19 +402,109 @@ int hc_primary_ids_q4(const rt_scene_desc *sc, uint32_t w, uint32_t h, int32_t *
 }
 
 // Arbitrary rays (n x 6 floats: origin, direction) through the exact binary tree and through the quantised 4-wide nodes
-// in the kernel's arithmetic: tri_exact / tri_q4 = BVH-order triangle or -1, t_exact / t_q4 = hit distance (inf: miss).
+// in the kernel's arithmetic: tri_exact / tri_q4 = the scene's triangle id or -1, t_exact / t_q4 = hit distance (inf: miss).
 int hc_trace_rays(const rt_scene_desc *sc, uint64_t n, const float *rays, int32_t *tri_exact, float *t_exact, int32_t *tri_q4, float *t_q4) {
     HostScene hs;
     if (int rc = build(sc, hs)) return rc;
+    auto id = [&](int32_t k) { return k < 0 ? -1 : (int32_t)(hs.p.scene.tris[k].id_last & ~RT_LAST_BIT); };
     for (uint64_t i = 0; i < n; ++i) {
         const f3 o = mk3(rays[6 * i], rays[6 * i + 1], rays[6 * i + 2]), d = mk3(rays[6 * i + 3], rays[6 * i + 4], rays[6 * i + 5]);
         const Hit a = closest_hit(hs.d.scene, o, d, hs.d.eps);
         const Hit b = closest_hit_q4(hs.d.scene, o, d, hs.d.eps, nullptr);
-        tri_exact[i] = a.tri;
+        tri_exact[i] = id(a.tri);
         t_exact[i] = a.t;
-        tri_q4[i] = b.tri;
+        tri_q4[i] = id(b.tri);
         t_q4[i] = b.t;
     }
+    return 0;
+}
+
+// ---- independent closest-hit reference ----------------------------------------------------------------------------------
+// Brute force over every (ray, triangle) pair in double precision, on the float32 inputs widened exactly.  It calls
+// nothing from pt_core.cuh, so a defect in the shared device math cannot hide in it.  Each pair is classified against a
+// LOCAL tolerance: s = c_tol * 2^-23 * (max_i |v_i - o|_inf + |t|), w = s / |cos(d, n)|.  s bounds the float32
+// triangle test's rounding (relative to the magnitudes it subtracts: vertices relative to the origin, and t); dividing
+// by |cos| turns it into a distance along the plane, where a grazing ray's hit point moves by error / |cos|.  s has no
+// |o| term on purpose: a float32 box or triangle test whose error grows with the distance from the WORLD origin is a
+// defect this reference must expose.  The tests use c_tol = 16 (tests/hit_scenarios.py); at that value the exact host
+// traversal has no mismatch on any scenario.
+//   clear hit:  the plane point is inside by more than w (world distance to every edge line: barycentric x altitude),
+//               t > eps + w and |cos| > 1e-4;
+//   clear miss: outside by more than w, or t < eps - w, or a determinant of exactly 0 (parallel ray, zero area);
+//   borderline: anything else.
+// Per ray: k_star = nearest clear hit (triangle index) or -1, t_star its distance, ties = clear hits with
+// |t - t_star| <= w + w_star (k_star included), decidable = 1 when no borderline triangle can be closer than
+// t_star + w_star (t_b - w_b < t_star + w_star) — for a ray without a clear hit: when there is no borderline pair at all.
+int hc_brute_hits(const float *tri, uint64_t n_tris, const float *rays, uint64_t n_rays, double eps, double c_tol, int32_t *k_star,
+                  double *t_star, int32_t *ties, uint8_t *decidable) {
+    struct T {
+        double v[3][3], e1[3], e2[3], n[3], area2, alt[3];
+    };
+    std::vector<T> tr(n_tris);
+    auto len = [](const double *a) { return std::sqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]); };
+    for (uint64_t k = 0; k < n_tris; ++k) {
+        T &t = tr[k];
+        for (int i = 0; i < 3; ++i)
+            for (int a = 0; a < 3; ++a) t.v[i][a] = tri[9 * k + 3 * i + a];
+        double e12[3];
+        for (int a = 0; a < 3; ++a) t.e1[a] = t.v[1][a] - t.v[0][a], t.e2[a] = t.v[2][a] - t.v[0][a], e12[a] = t.v[2][a] - t.v[1][a];
+        t.n[0] = t.e1[1] * t.e2[2] - t.e1[2] * t.e2[1];
+        t.n[1] = t.e1[2] * t.e2[0] - t.e1[0] * t.e2[2];
+        t.n[2] = t.e1[0] * t.e2[1] - t.e1[1] * t.e2[0];
+        t.area2 = len(t.n);
+        // altitude onto the edge opposite vertex i: the world distance of barycentric 1 from that edge
+        const double l[3] = {len(e12), len(t.e2), len(t.e1)};
+        for (int i = 0; i < 3; ++i) t.alt[i] = l[i] > 0 ? t.area2 / l[i] : 0.0;
+    }
+    auto work = [&](uint64_t r0, uint64_t r1) {
+        std::vector<std::pair<double, double>> clear;  // (t, w) of the ray's clear hits
+        for (uint64_t r = r0; r < r1; ++r) {
+            const double o[3] = {rays[6 * r], rays[6 * r + 1], rays[6 * r + 2]}, d[3] = {rays[6 * r + 3], rays[6 * r + 4], rays[6 * r + 5]};
+            const double dl = len(d);
+            clear.clear();
+            int32_t best = -1;
+            double bt = INFINITY, bw = 0, border_lo = INFINITY;  // border_lo: min over borderline pairs of t - w
+            bool any_border = false;
+            for (uint64_t k = 0; k < n_tris; ++k) {
+                const T &t = tr[k];
+                const double det = -(d[0] * t.n[0] + d[1] * t.n[1] + d[2] * t.n[2]);
+                if (det == 0.0 || t.area2 == 0.0) continue;  // clear miss
+                const double y[3] = {o[0] - t.v[0][0], o[1] - t.v[0][1], o[2] - t.v[0][2]};
+                const double rr[3] = {d[1] * y[2] - d[2] * y[1], d[2] * y[0] - d[0] * y[2], d[0] * y[1] - d[1] * y[0]};
+                const double beta = -(t.e2[0] * rr[0] + t.e2[1] * rr[1] + t.e2[2] * rr[2]) / det;
+                const double gamma = (t.e1[0] * rr[0] + t.e1[1] * rr[1] + t.e1[2] * rr[2]) / det;
+                const double tt = (y[0] * t.n[0] + y[1] * t.n[1] + y[2] * t.n[2]) / det;
+                double m = 0;
+                for (int i = 0; i < 3; ++i)
+                    for (int a = 0; a < 3; ++a) m = std::max(m, std::fabs(t.v[i][a] - o[a]));
+                const double cosg = std::fabs(det) / (dl * t.area2);
+                const double w = c_tol * std::ldexp(1.0, -23) * (m + std::fabs(tt)) / cosg;
+                const double dist = std::min({(1.0 - beta - gamma) * t.alt[0], beta * t.alt[1], gamma * t.alt[2]});
+                if (dist < -w || tt < eps - w) continue;  // clear miss
+                if (dist > w && tt > eps + w && cosg > 1e-4) {
+                    clear.emplace_back(tt, w);
+                    if (tt < bt) bt = tt, bw = w, best = (int32_t)k;
+                } else {
+                    any_border = true;
+                    border_lo = std::min(border_lo, tt - w);
+                }
+            }
+            int32_t n_ties = 0;
+            for (const auto &c : clear) n_ties += std::fabs(c.first - bt) <= c.second + bw ? 1 : 0;
+            k_star[r] = best;
+            t_star[r] = bt;
+            ties[r] = n_ties;
+            decidable[r] = best < 0 ? !any_border : !(border_lo < bt + bw);
+        }
+    };
+    const unsigned n_threads = std::max(1u, std::min(64u, std::thread::hardware_concurrency()));
+    std::vector<std::thread> pool;
+    const uint64_t chunk = (n_rays + n_threads - 1) / n_threads;
+    for (unsigned i = 0; i < n_threads; ++i) {
+        const uint64_t a = std::min<uint64_t>(n_rays, i * chunk), b = std::min<uint64_t>(n_rays, a + chunk);
+        if (a < b) pool.emplace_back(work, a, b);
+    }
+    for (auto &th : pool) th.join();
     return 0;
 }
 

@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, golden_array
+from hit_scenarios import check_tree, triangles_scene
 
 import rt_b200
 from rt_b200 import _abi, gpu
@@ -34,33 +35,11 @@ def _download(rt):
     return info, rt.debug_bvh(1, _abi.NODE_DTYPE), rt.debug_bvh(2, np.uint32), rt.debug_bvh(3, np.uint8), rt.debug_bvh(4, np.uint8)
 
 
-def _check_tree(hc, sc, info, nodes, objects, qn, tris):
-    n = sc.n_tris
-    assert info[0] == n and info[6] == 1, info  # built on the device
-    assert sorted(objects.tolist()) == list(range(n))
-    d = sc.desc()
-    out = np.zeros(8)
-    rc = hc.hc_tree_stats(C.byref(d), nodes.ctypes.data_as(C.c_void_p), C.c_uint64(len(nodes)), objects.ctypes.data_as(C.c_void_p),
-                          C.c_uint64(len(objects)), out.ctypes.data_as(C.c_void_p))
-    assert rc == 0, rc
-    _, inner, leaves, max_leaf, depth, ok, cost, layout = out
-    assert ok == 1.0, "triangle coverage / exact boxes"
-    assert layout == 1.0 and inner == leaves - 1 and max_leaf <= 8 and depth == info[5] and depth < 62
-    res = np.zeros(4)
-    root4 = C.c_int32(int(np.int32(np.uint32(info[3]))))
-    rc = hc.hc_wide_containment_arrays(qn.ctypes.data_as(C.c_void_p), C.c_uint64(len(qn) // 64), root4, tris.ctypes.data_as(C.c_void_p),
-                                       C.c_uint64(len(tris) // 64), res.ctypes.data_as(C.c_void_p))
-    assert rc == 0, rc
-    assert res[1] == 0 and res[2] == n  # no quantised plane cuts into a triangle below it; every triangle reached once
-    assert res[3] == info[4] <= 96  # the traversal-stack need computed on the device is the host's figure
-    return cost, depth, inner
-
-
 @pytest.mark.parametrize("name", ["tiny", "texall", "small_lights"])
 def test_device_built_tree_small_scenes(name, rt, hc, manifest, golden_scene):
     sc = golden_scene(name)
     rt.upload_scene(sc)
-    cost, depth, inner = _check_tree(hc, sc, *_download(rt))
+    cost, depth, inner = check_tree(hc, sc, *_download(rt))
     m = manifest["scenes"][name]
     ids = rt.primary_ids(m["width"], m["height"])
     ref = golden_array(f"{name}_ids.i32", np.int32, (m["height"], m["width"]))
@@ -72,7 +51,7 @@ def test_device_built_tree_260k_scene(rt, hc, manifest, big_scene):
     inside a node differs, so the trees are not identical), and the images do not depend on the tree."""
     rt.upload_scene(big_scene)
     info, nodes, objects, qn, tris = _download(rt)
-    cost, depth, inner = _check_tree(hc, big_scene, info, nodes, objects, qn, tris)
+    cost, depth, inner = check_tree(hc, big_scene, info, nodes, objects, qn, tris)
     d = big_scene.desc()
     host = np.zeros(8)
     assert hc.hc_sah_stats(C.byref(d), host.ctypes.data_as(C.c_void_p)) == 0
@@ -120,29 +99,12 @@ def test_device_build_is_deterministic(rt, big_scene):
     assert a[1][used].tobytes() == b[1][used].tobytes()
 
 
-def _triangles_scene(tri):
-    sc = rt_b200.SceneData.load(os.path.join(ROOT, "tests", "golden", "tiny.rtsc"))
-    n = len(tri)
-    sc.tri_pos = np.asarray(tri, np.float32).reshape(n, 3, 3)
-    sc.tri_normals = np.tile(np.array([0, 0, 1], np.float32), (n, 3, 1))
-    sc.tri_uv = np.zeros((n, 3, 2), np.float32)
-    sc.tri_tangents = None
-    sc.tri_material = np.zeros(n, np.uint32)
-    sc.scene_bvh = _abi.BvhData(np.zeros(0, _abi.NODE_DTYPE), np.zeros(0, np.uint32), _abi.RT_NO_CHILD)
-    sc.light_bvh = _abi.BvhData(np.zeros(0, _abi.NODE_DTYPE), np.zeros(0, np.uint32), _abi.RT_NO_CHILD)
-    sc.camera_position = np.array([0, 0, 5], np.float32)
-    sc.camera_forward = np.array([0, 0, -1], np.float32)
-    sc.camera_right = np.array([1, 0, 0], np.float32)
-    sc.camera_up = np.array([0, 1, 0], np.float32)
-    return sc
-
-
 @pytest.mark.parametrize("n", [1, 2, 9, 33, 1000])
 def test_device_build_edge_cases(n, rt, hc):
     """One triangle, a handful, and n copies of the SAME triangle (all centroids coincide: binning cannot separate them,
     the builder splits by position until the leaves hold <= 8)."""
     one = [[-1, -1, 0], [1, -1, 0], [0, 1, 0]]
-    sc = _triangles_scene([one] * n)
+    sc = triangles_scene([one] * n)
     rt.upload_scene(sc)
     info, nodes, objects, qn, tris = _download(rt)
     assert info[0] == n and sorted(objects.tolist()) == list(range(n))
@@ -154,26 +116,29 @@ def test_device_build_edge_cases(n, rt, hc):
     ids = rt.primary_ids(32, 32)
     assert ids[16, 16] >= 0 and ids[0, 0] == -1
     # distinct triangles in a row: every one is found
-    row = [[[x - 0.4, -0.4, 0], [x + 0.4, -0.4, 0], [x, 0.4, 0]] for x in np.linspace(-2, 2, n)] if n > 1 else [one]
-    sc = _triangles_scene(row)
+    s = min(1.0, 4.0 / max(n - 1, 1))  # side scaled so that neighbours do not overlap: each centroid has one answer
+    row = [[[x - 0.4 * s, -0.4 * s, 0], [x + 0.4 * s, -0.4 * s, 0], [x, 0.4 * s, 0]] for x in np.linspace(-2, 2, n)] if n > 1 else [one]
+    sc = triangles_scene(row)
     rt.upload_scene(sc)
     info = rt.debug_bvh(0, np.uint32)
     assert info[0] == n and info[4] <= 96
-    ids = rt.primary_ids(256, 64)
-    assert (ids >= 0).any()
+    # one 1x1 view straight down onto each centroid (the pixel centre's camera term is 0: the ray is the camera's axis)
+    centroids = np.asarray(row, np.float32).astype(np.float64).mean(axis=1)
+    cams = [rt_b200.Camera((c[0], c[1], 5), (1, 0, 0), (0, 1, 0), (0, 0, -1), 1.0) for c in centroids]
+    assert rt.primary_ids(1, 1, cameras=cams).reshape(-1).tolist() == list(range(n))
 
 
 def test_device_build_rejects_non_finite_geometry(rt):
     tri = np.array([[[-1, -1, 0], [1, -1, 0], [0, 1, 0]]] * 40, np.float32)
     tri[7, 1, 0] = np.inf
-    sc = _triangles_scene(tri)
+    sc = triangles_scene(tri)
     with pytest.raises(gpu.RtGpuError, match="RT_ERR_BAD_SCENE"):
         rt.upload_scene(sc)
-    rt.upload_scene(_triangles_scene(tri[:7]))  # the handle stays usable
+    rt.upload_scene(triangles_scene(tri[:7]))  # the handle stays usable
 
 
 def test_empty_scene_through_the_device_build(rt):
-    sc = _triangles_scene(np.zeros((0, 3, 3), np.float32))
+    sc = triangles_scene(np.zeros((0, 3, 3), np.float32))
     rt.upload_scene(sc)
     ids = rt.primary_ids(8, 8)
     assert (ids == -1).all()

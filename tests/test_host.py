@@ -297,8 +297,8 @@ def test_four_wide_collapse_gives_reference_ids(name, rebuild, hc, manifest, gol
 
 def test_rays_inside_the_plane_of_a_flat_node_keep_their_hits(hc, big_scene):
     """Light-sampled directions from one emissive panel to the next run INSIDE the panels' common plane (|d.y| ~ 1e-7,
-    origin one ulp above it): the ray-space offset fma(org, 1/d, -o/d) of the quantised slab test then carries an
-    error of several units of t, and a flat node's box has to absorb it.  The power-of-two grid does (its origin is
+    origin one ulp above it): the ray-space offset of the quantised slab test then carries an error of several units of
+    t (it did with fma(org, 1/d, -o/d); (org - o)/d shrinks it), and a flat node's box has to absorb it.  The power-of-two grid does (its origin is
     rounded down to 14 mantissa bits, which leaves every flat box ~2e-6 of slack); an exact-cell variant tried in round 2
     lost 33 of 15 176 path-traced rays exactly here (DESIGN.md, k_extend).  Every hit the exact boxes find must be
     found through the quantised 4-wide nodes as well."""
