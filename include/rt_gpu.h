@@ -291,7 +291,8 @@ typedef struct rt_adaptive_params {
 int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_adaptive_params *ap);
 
 /* After rt_gpu_render_adaptive: per-pixel sample counts (width*height uint32) and the err each pixel last had
- * (width*height float; 0 outside the range); either may be NULL.  RT_ERR_NO_RENDER after any other render. */
+ * (width*height float; 0 outside the range); either may be NULL.  After rt_gpu_render_views_adaptive: the same for
+ * the stacked image (n_views*width*height each).  RT_ERR_NO_RENDER after any other render. */
 int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error);
 
 /* ---- multi-view rendering ----------------------------------------------------------------------------------
@@ -310,7 +311,8 @@ int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *re
  * height > 2^32, a stacked image of more than 2^31 - 1 pixels, a text scene, and RT_FLAG_ACCUMULATE unless the
  * previous render had the same width, height and n_views (rt_gpu_render counts as one view; this holds in both
  * directions).  Without the flag, a render behaves as on a fresh handle.  Adaptive sampling over views is not
- * offered: rt_gpu_readback_adaptive returns RT_ERR_NO_RENDER after this call. */
+ * offered by this call: rt_gpu_readback_adaptive returns RT_ERR_NO_RENDER after it (rt_gpu_render_views_adaptive
+ * below is the adaptive form). */
 typedef struct rt_views {
     uint32_t n_views;          /* >= 1 */
     uint32_t view_base;        /* Philox pixel key of pixel p of view v = (view_base + v) * width * height + p */
@@ -318,6 +320,27 @@ typedef struct rt_views {
 } rt_views;
 
 int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views);
+
+/* Adaptive multi-view rendering: rt_gpu_render_adaptive over the stacked image of rt_gpu_render_views.  The image,
+ * pixel range and keys are rt_gpu_render_views' (pixel_begin / pixel_end index [0, n_views * width * height); pixel p
+ * of view v is keyed (view_base + v) * width * height + p); the rounds, the rule, params->samples as the maximum spp
+ * and the sample prefix [0, n_p) of every pixel are rt_gpu_render_adaptive's.  So:
+ *   - one view with the scene's own camera and view_base = 0 is rt_gpu_render_adaptive, bit for bit;
+ *   - view v of a call is a one-view call with view_base = v (bit for bit when both run in the same batches);
+ *   - a pixel with count n equals rt_gpu_render_views of samples [0, n) summed in the same sample ranges.
+ * Afterwards rt_gpu_readback returns n_views * width * height * 3 means (sum / n_p, view-major), rt_gpu_readback_rgb8
+ * n_views * width * height * 3 bytes, rt_gpu_readback_adaptive n_views * width * height counts and errors,
+ * rt_gpu_accum_device_ptr reports n_views * width * height * 4 floats, and stats.samples = sum of n_p.
+ * RT_ERR_INVALID_ARG for everything either call refuses: a null argument, a text scene, n_views == 0, cameras == NULL,
+ * a non-finite camera value, (view_base + n_views) * width * height > 2^32, a stacked image of more than 2^31 - 1
+ * pixels, RT_MODE_PRIMARY_IDS, samples < 2, sample_begin / sample_end != 0, RT_FLAG_ACCUMULATE, bad
+ * rt_adaptive_params, an illegal pixel range, or a (per-device) range larger than one batch of max_paths_in_flight
+ * paths.  A multi-device handle splits the stacked range into contiguous parts, as rt_gpu_render_adaptive does.  The
+ * sums have per-pixel counts afterwards: RT_FLAG_ACCUMULATE on the next rt_gpu_render / rt_gpu_render_views fails with
+ * RT_ERR_INVALID_ARG; without it a render behaves as on a fresh handle.  A round of k samples runs in ceil(k / k_max)
+ * batches, k_max = paths per batch / pixels of the (per-device) range: more views mean more batches per round. */
+int rt_gpu_render_views_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views,
+                                 const rt_adaptive_params *ap);
 
 /* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene.
  * which = 0: uint32[8] {n_tris, binary node slots, 4-wide nodes, root link, worst-case traversal stack need, depth of

@@ -803,7 +803,8 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
     return RT_OK;
 }
 
-// One device's part of an adaptive render (rt_gpu_render_adaptive): the pixel range it adapts and where its rounds are.
+// One device's part of an adaptive render (rt_gpu_render_adaptive, rt_gpu_render_views_adaptive): the pixel range it
+// adapts and where its rounds are.
 struct AdaptiveRun {
     DeviceState *d = nullptr;
     size_t pix0 = 0, n_render = 0;
@@ -812,20 +813,24 @@ struct AdaptiveRun {
     bool finished = false;
     rt::BatchParams bp{};
     rt::Camera cam{};
+    uint32_t key_offset = 0;  // views: stacked pixel + key_offset = Philox pixel key (view_base * W * H)
 };
 
 // Sizes the queues and the adaptive buffers of run.d for the pixel range [pix0, pix1) and clears its sums, counts and
-// errors; no kernel runs yet.  RT_ERR_INVALID_ARG when the range does not fit one batch at one sample.
-int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp, size_t pix0, size_t pix1) {
+// errors; no kernel runs yet.  RT_ERR_INVALID_ARG when the range does not fit one batch at one sample.  views != nullptr:
+// the stacked image of its views (views.cuh), [pix0, pix1) indexing it, and its cameras go to d.cams.
+int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp, size_t pix0, size_t pix1, const ViewSet *views) {
     DeviceState &d = *run.d;
     CU_CHECK(cudaSetDevice(d.device));
-    const size_t n_pix = static_cast<size_t>(rp.width) * rp.height;
+    const uint32_t n_views = views ? static_cast<uint32_t>(views->cams.size()) : 1u;
+    const size_t n_pix = static_cast<size_t>(rp.width) * rp.height * n_views;
     run.pix0 = pix0;
     run.n_render = pix1 - pix0;
     const size_t cap = batch_cap(d, rp.max_paths_in_flight, std::max<size_t>(run.n_render, 1) * rp.samples);
     if (run.n_render > cap)
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: the pixel range (" + std::to_string(run.n_render) +
-                                            " pixels) does not fit one batch of " + std::to_string(cap) + " paths");
+        return fail(RT_ERR_INVALID_ARG, std::string(views ? "rt_gpu_render_views_adaptive" : "rt_gpu_render_adaptive") +
+                                            ": the pixel range (" + std::to_string(run.n_render) + " pixels) does not fit one batch of " +
+                                            std::to_string(cap) + " paths");
     run.k_max = static_cast<uint32_t>(cap / std::max<size_t>(run.n_render, 1));
     run.n_words = static_cast<uint32_t>((run.n_render + 31) / 32);
     run.cur = 0;
@@ -842,6 +847,8 @@ int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp
         if (int rc = d.alist.alloc(2 * run.n_render)) return rc;
         if (int rc = d.awords.alloc(2 * static_cast<size_t>(run.n_words))) return rc;
     }
+    if (views)
+        if (int rc = d.cams.upload(views->cams, d.stream)) return rc;
     d.apix0 = pix0;
     d.apix1 = pix1;
     CU_CHECK(cudaMemsetAsync(d.stats.p, 0, 4 * sizeof(unsigned long long), d.stream));
@@ -853,12 +860,14 @@ int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp
     bp.pix0 = static_cast<uint32_t>(pix0);
     bp.npix = static_cast<uint32_t>(run.n_render);  // the whole range: k_shade's radiance slots stay those of a fixed render
     bp.width = rp.width;
-    bp.height = rp.height;
+    bp.height = rp.height;  // views: the height of one view (split_view_pixel)
     bp.k0 = static_cast<uint32_t>(rp.seed);
     bp.k1 = static_cast<uint32_t>(rp.seed >> 32);
     bp.centre = 0;
     bp.tiled = 0;  // queue 0 follows the active list, whose first form is already in tiles where that applies
     run.cam = make_camera(scene_camera(d.scene), rp.width, rp.height);
+    // fits 32 bits: rt_gpu_render_views_adaptive checks (view_base + V) * W * H
+    run.key_offset = views ? static_cast<uint32_t>(static_cast<uint64_t>(views->view_base) * rp.width * rp.height) : 0u;
     d.marks.clear();
     d.events_used = 0;
     CU_CHECK(cudaEventRecord(d.ev_begin, d.stream));
@@ -870,16 +879,17 @@ int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp
 // the rule, the flag scan and the compaction into the other list, whose device-side length goes to h_active[round & 1]
 // behind ev_round[round & 1].
 int enqueue_adaptive_round(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp, const rt_adaptive_params &ap, uint32_t round,
-                           uint32_t k, uint64_t &launches) {
+                           uint32_t k, const ViewSet *views, uint64_t &launches) {
     DeviceState &d = *run.d;
     CU_CHECK(cudaSetDevice(d.device));
     const uint32_t qdepth = std::max(d.scene.ray_depth, 1u), npix = run.bp.npix;
     uint32_t *list = d.alist.p + run.cur * run.n_render, *next = d.alist.p + (run.cur ^ 1) * run.n_render;
     uint32_t *active = d.actr.p + run.cur, *next_active = d.actr.p + (run.cur ^ 1);
     uint32_t *words = d.awords.p, *wscan = d.awords.p + run.n_words;
-    if (round == 0) {
-        const bool tiled = run.pix0 == 0 && npix == static_cast<size_t>(rp.width) * rp.height && rp.width % 8 == 0 && rp.height % 4 == 0 &&
-                           !std::getenv("RT_NO_TILES");
+    if (round == 0) {  // tiles over the stacked image of W x (V * H), as in k_generate_views
+        const uint32_t n_views = views ? static_cast<uint32_t>(views->cams.size()) : 1u;
+        const bool tiled = run.pix0 == 0 && npix == static_cast<size_t>(rp.width) * rp.height * n_views && rp.width % 8 == 0 &&
+                           (rp.height * n_views) % 4 == 0 && !std::getenv("RT_NO_TILES");
         rt::k_adapt_init<<<(npix + 255) / 256, 256, 0, d.stream>>>(list, run.bp.pix0, npix, rp.width, tiled ? 1u : 0u, active);
         ++launches;
     }
@@ -891,9 +901,14 @@ int enqueue_adaptive_round(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_pa
         bp.k = std::min(run.k_max, k - j0);
         const uint32_t n = npix * bp.k;  // the grid of k_generate_active; the queue holds n_active * k paths
         CU_CHECK(cudaMemsetAsync(d.counters.p, 0, n_counters_of(qdepth) * sizeof(uint32_t), d.stream));
-        rt::k_generate_active<<<(n + 255) / 256, 256, 0, d.stream>>>(run.cam, bp, q_gen, list, active);
+        if (views)
+            rt::k_generate_active_views<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, bp, q_gen, list, active, run.key_offset);
+        else
+            rt::k_generate_active<<<(n + 255) / 256, 256, 0, d.stream>>>(run.cam, bp, q_gen, list, active);
         mark(ctx, d, K_GENERATE);
-        if (int rc = enqueue_bounces(ctx, d, bp, n, split_allowed, launches)) return rc;
+        rt::BatchParams bp_key = bp;  // k_shade's radiance slot: (sample - s0) * npix + (key - pix0)
+        bp_key.pix0 += run.key_offset;
+        if (int rc = enqueue_bounces(ctx, d, bp_key, n, split_allowed, launches)) return rc;
         rt::k_accumulate_active<<<(npix + 255) / 256, 256, 0, d.stream>>>(bp, d.rad, d.accum.p, d.acounts.p, list, active);
         mark(ctx, d, K_ACCUMULATE);
         launches += 2;
@@ -915,7 +930,7 @@ int enqueue_adaptive_round(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_pa
 // has just enqueued: before round r + 2 it waits for round r's active count (one round of lookahead) and stops a device
 // whose count was 0, so at most one empty round is launched and the GPU does not idle on the host.
 int enqueue_render_adaptive(rt_gpu_ctx *ctx, std::vector<AdaptiveRun> &runs, const rt_render_params &rp, const rt_adaptive_params &ap,
-                            uint64_t &launches) {
+                            const ViewSet *views, uint64_t &launches) {
     const uint32_t first = std::min(ap.min_samples, rp.samples);
     for (uint32_t round = 0;; ++round) {
         bool any = false;
@@ -935,7 +950,7 @@ int enqueue_render_adaptive(rt_gpu_ctx *ctx, std::vector<AdaptiveRun> &runs, con
                 }
             }
             const uint32_t k = round == 0 ? first : std::min(ap.step_samples, rp.samples - run.done);
-            if (int rc = enqueue_adaptive_round(ctx, run, rp, ap, round, k, launches)) return rc;
+            if (int rc = enqueue_adaptive_round(ctx, run, rp, ap, round, k, views, launches)) return rc;
             any = true;
         }
         if (!any) break;
@@ -1335,6 +1350,78 @@ int render_on_devices(rt_gpu_ctx *ctx, const rt_render_params &rp, const ViewSet
     return RT_OK;
 }
 
+// The checks of the views of rt_gpu_render_views (and rt_gpu_render_views_adaptive): views, stacked image size, the
+// 32-bit key and finite cameras.  Fills vs with the device cameras.
+int check_views(const rt_render_params &rp, const rt_views &views, const std::string &who, ViewSet &vs) {
+    if (views.n_views == 0 || !views.cameras) return fail(RT_ERR_INVALID_ARG, who + ": no views / null cameras");
+    const uint64_t per_view = static_cast<uint64_t>(rp.width) * rp.height, V = views.n_views;
+    if (per_view == 0 || per_view > 0x7FFFFFFFull || per_view * V > 0x7FFFFFFFull)
+        return fail(RT_ERR_INVALID_ARG, who + ": illegal image size (the stacked image has n_views * width * height pixels)");
+    if ((views.view_base + V) * per_view > (1ull << 32))
+        return fail(RT_ERR_INVALID_ARG, who + ": (view_base + n_views) * width * height exceeds the 32-bit pixel key");
+    for (uint32_t v = 0; v < views.n_views; ++v) {
+        const rt_camera &c = views.cameras[v];
+        bool finite = std::isfinite(c.fov_x);
+        for (int k = 0; k < 3; ++k)
+            finite = finite && std::isfinite(c.position[k]) && std::isfinite(c.right[k]) && std::isfinite(c.up[k]) && std::isfinite(c.forward[k]);
+        if (!finite) return fail(RT_ERR_INVALID_ARG, who + ": camera " + std::to_string(v) + " has a non-finite value");
+    }
+    vs.view_base = views.view_base;
+    vs.cams.clear();
+    for (uint32_t v = 0; v < views.n_views; ++v) vs.cams.push_back(make_camera(views.cameras[v], rp.width, rp.height));
+    return RT_OK;
+}
+
+// The checks of an adaptive render's parameters over an image of n_pixels; resolves rp.pixel_end
+int check_adaptive(rt_render_params &rp, const rt_adaptive_params &ap, uint64_t n_pixels, const std::string &who) {
+    if (rp.mode != RT_MODE_BEAUTY) return fail(RT_ERR_INVALID_ARG, who + ": beauty renders only");
+    if (rp.samples < 2) return fail(RT_ERR_INVALID_ARG, who + ": samples (the maximum spp) < 2");
+    if (rp.sample_begin != 0 || rp.sample_end != 0)
+        return fail(RT_ERR_INVALID_ARG, who + ": every pixel starts at sample 0 (sample_begin / sample_end must be 0)");
+    if (rp.flags & RT_FLAG_ACCUMULATE) return fail(RT_ERR_INVALID_ARG, who + ": RT_FLAG_ACCUMULATE is not supported");
+    if (ap.min_samples < 2 || ap.step_samples == 0 || !(ap.abs_floor > 0.0f) || !(ap.rel_error >= 0.0f))
+        return fail(RT_ERR_INVALID_ARG, who + ": needs min_samples >= 2, step_samples >= 1, abs_floor > 0, rel_error >= 0");
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, who + ": illegal pixel range");
+    return RT_OK;
+}
+
+// The adaptive render of rt_gpu_render_adaptive (views == nullptr) and rt_gpu_render_views_adaptive over every device of
+// the handle; rp and ap are validated and rp.pixel_end resolved.
+int render_adaptive_on_devices(rt_gpu_ctx *ctx, const rt_render_params &rp, const rt_adaptive_params &ap, const ViewSet *views) {
+    const uint32_t n_views = views ? static_cast<uint32_t>(views->cams.size()) : 1u;
+    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height * n_views;
+    // every device adapts a contiguous part of the range (a pixel's decisions depend on its own sums only)
+    const int n = static_cast<int>(ctx->devs.size());
+    const uint64_t n_px = rp.pixel_end - rp.pixel_begin;
+    std::vector<AdaptiveRun> runs(n);
+    ctx->have_render = false;  // the sums are being replaced
+    for (int g = 0; g < n; ++g) {
+        runs[g].d = ctx->devs[g].get();
+        const size_t b = rp.pixel_begin + n_px * g / n, e = rp.pixel_begin + n_px * (g + 1) / n;
+        if (int rc = setup_adaptive(ctx, runs[g], rp, b, e, views)) return rc;
+    }
+    uint64_t launches = 0;
+    if (int rc = enqueue_render_adaptive(ctx, runs, rp, ap, views, launches)) return rc;
+    if (n > 1)
+        if (int rc = reduce_to_device0(ctx, static_cast<size_t>(n_pixels), true)) return rc;
+    if (int rc = finish_render(ctx, rp, launches)) return rc;
+    if (std::getenv("RT_TIMING")) {  // contiguous tiles are not load-balanced: the per-device times show by how much
+        for (int g = 0; g < n; ++g) {
+            float ms = 0.0f;
+            cudaEventElapsedTime(&ms, runs[g].d->ev_begin, runs[g].d->ev_end);
+            std::fprintf(stderr, "rt_gpu adaptive: device %d pixels [%zu, %zu) %.2f ms, %llu samples\n", runs[g].d->device, runs[g].pix0,
+                         runs[g].pix0 + runs[g].n_render, ms, static_cast<unsigned long long>(runs[g].d->h_stats[3]));
+        }
+    }
+    ctx->last = rp;
+    ctx->last_views = views ? n_views : 0u;
+    ctx->last_adaptive = ap;
+    ctx->have_render = true;
+    ctx->adaptive = ctx->adaptive_sums = true;
+    return RT_OK;
+}
+
 }  // namespace
 
 int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
@@ -1361,20 +1448,10 @@ int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const r
     if (!ctx || !params || !views) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: null argument");
     if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render_views: no scene uploaded");
     if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: not available for course text scenes");
-    if (views->n_views == 0 || !views->cameras) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: no views / null cameras");
     rt_render_params rp = *params;
+    ViewSet vs;
+    if (int rc = check_views(rp, *views, "rt_gpu_render_views", vs)) return rc;
     const uint64_t per_view = static_cast<uint64_t>(rp.width) * rp.height, V = views->n_views;
-    if (per_view == 0 || per_view > 0x7FFFFFFFull || per_view * V > 0x7FFFFFFFull)
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: illegal image size (the stacked image has n_views * width * height pixels)");
-    if ((views->view_base + V) * per_view > (1ull << 32))
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: (view_base + n_views) * width * height exceeds the 32-bit pixel key");
-    for (uint32_t v = 0; v < views->n_views; ++v) {
-        const rt_camera &c = views->cameras[v];
-        bool finite = std::isfinite(c.fov_x);
-        for (int k = 0; k < 3; ++k)
-            finite = finite && std::isfinite(c.position[k]) && std::isfinite(c.right[k]) && std::isfinite(c.up[k]) && std::isfinite(c.forward[k]);
-        if (!finite) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: camera " + std::to_string(v) + " has a non-finite value");
-    }
     if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: samples == 0");
     if (rp.sample_end == 0) rp.sample_end = rp.samples;
     if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: sample_begin > sample_end");
@@ -1385,9 +1462,6 @@ int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const r
         (!ctx->have_render || ctx->adaptive_sums || ctx->last.width != rp.width || ctx->last.height != rp.height ||
          std::max(ctx->last_views, 1u) != views->n_views))
         return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: RT_FLAG_ACCUMULATE needs a previous render of the same width, height and n_views");
-    ViewSet vs;
-    vs.view_base = views->view_base;
-    for (uint32_t v = 0; v < views->n_views; ++v) vs.cams.push_back(make_camera(views->cameras[v], rp.width, rp.height));
     return render_on_devices(ctx, rp, &vs);
 }
 
@@ -1398,51 +1472,26 @@ int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, cons
     if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: not available for course text scenes");
     if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull)
         return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: illegal image size");
-    if (rp.mode != RT_MODE_BEAUTY) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: beauty renders only");
-    if (rp.samples < 2) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: samples (the maximum spp) < 2");
-    if (rp.sample_begin != 0 || rp.sample_end != 0)
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: every pixel starts at sample 0 (sample_begin / sample_end must be 0)");
-    if (rp.flags & RT_FLAG_ACCUMULATE) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: RT_FLAG_ACCUMULATE is not supported");
-    if (ap->min_samples < 2 || ap->step_samples == 0 || !(ap->abs_floor > 0.0f) || !(ap->rel_error >= 0.0f))
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: needs min_samples >= 2, step_samples >= 1, abs_floor > 0, rel_error >= 0");
-    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height;
-    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
-    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_adaptive: illegal pixel range");
-    // every device adapts a contiguous part of the range (a pixel's decisions depend on its own sums only)
-    const int n = static_cast<int>(ctx->devs.size());
-    const uint64_t n_px = rp.pixel_end - rp.pixel_begin;
-    std::vector<AdaptiveRun> runs(n);
-    ctx->have_render = false;  // the sums are being replaced
-    for (int g = 0; g < n; ++g) {
-        runs[g].d = ctx->devs[g].get();
-        const size_t b = rp.pixel_begin + n_px * g / n, e = rp.pixel_begin + n_px * (g + 1) / n;
-        if (int rc = setup_adaptive(ctx, runs[g], rp, b, e)) return rc;
-    }
-    uint64_t launches = 0;
-    if (int rc = enqueue_render_adaptive(ctx, runs, rp, *ap, launches)) return rc;
-    if (n > 1)
-        if (int rc = reduce_to_device0(ctx, static_cast<size_t>(n_pixels), true)) return rc;
-    if (int rc = finish_render(ctx, rp, launches)) return rc;
-    if (std::getenv("RT_TIMING")) {  // contiguous tiles are not load-balanced: the per-device times show by how much
-        for (int g = 0; g < n; ++g) {
-            float ms = 0.0f;
-            cudaEventElapsedTime(&ms, runs[g].d->ev_begin, runs[g].d->ev_end);
-            std::fprintf(stderr, "rt_gpu adaptive: device %d pixels [%zu, %zu) %.2f ms, %llu samples\n", runs[g].d->device, runs[g].pix0,
-                         runs[g].pix0 + runs[g].n_render, ms, static_cast<unsigned long long>(runs[g].d->h_stats[3]));
-        }
-    }
-    ctx->last = rp;
-    ctx->last_views = 0;
-    ctx->last_adaptive = *ap;
-    ctx->have_render = true;
-    ctx->adaptive = ctx->adaptive_sums = true;
-    return RT_OK;
+    if (int rc = check_adaptive(rp, *ap, static_cast<uint64_t>(rp.width) * rp.height, "rt_gpu_render_adaptive")) return rc;
+    return render_adaptive_on_devices(ctx, rp, *ap, nullptr);
+}
+
+int rt_gpu_render_views_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views, const rt_adaptive_params *ap) {
+    const std::string who = "rt_gpu_render_views_adaptive";
+    if (!ctx || !params || !views || !ap) return fail(RT_ERR_INVALID_ARG, who + ": null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, who + ": no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, who + ": not available for course text scenes");
+    rt_render_params rp = *params;
+    ViewSet vs;
+    if (int rc = check_views(rp, *views, who, vs)) return rc;
+    if (int rc = check_adaptive(rp, *ap, static_cast<uint64_t>(rp.width) * rp.height * views->n_views, who)) return rc;
+    return render_adaptive_on_devices(ctx, rp, *ap, &vs);
 }
 
 int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error) {
     if (!ctx) return fail(RT_ERR_INVALID_ARG, "rt_gpu_readback_adaptive: null handle");
     if (!ctx->have_render || !ctx->adaptive) return fail(RT_ERR_NO_RENDER, "rt_gpu_readback_adaptive: the last render was not adaptive");
-    const size_t n_pix = static_cast<size_t>(ctx->last.width) * ctx->last.height;
+    const size_t n_pix = last_pixels(ctx);  // times the views after rt_gpu_render_views_adaptive
     if (sample_counts) {  // reduced to device 0
         DeviceState &d = *ctx->devs[0];
         CU_CHECK(cudaSetDevice(d.device));

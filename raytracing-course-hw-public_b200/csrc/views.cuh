@@ -5,7 +5,9 @@
 // reads that view's camera.  Its paths carry the Philox pixel key (view_base + v) * W * H + y * W + x, and the host
 // hands k_shade a BatchParams whose pix0 is shifted by the same view_base * W * H, so k_shade's radiance slot
 // (sample - s0) * npix + (pixel - pix0) is the one of the stacked render.  k_extend, k_shade, k_lightpdf_list,
-// k_accumulate, the reduce and the readback kernels work on the stacked index unchanged.
+// k_accumulate, the reduce and the readback kernels work on the stacked index unchanged.  The adaptive form
+// (rt_gpu_render_views_adaptive) is the same with k_generate_active_views in place of k_generate_active; the rounds,
+// the rule kernels and k_accumulate_active of adaptive.cuh work on the stacked index unchanged as well.
 //
 // The split is a pure function, compiled for the host as well (tests).
 #ifndef RT_VIEWS_CUH
@@ -58,6 +60,28 @@ __global__ void __launch_bounds__(256) k_generate_views(const Camera *__restrict
     const uint32_t pixel = bp.tiled ? tiled_pixel(pl, bp.width) : bp.pix0 + pl;
     const ViewPixel vp = split_view_pixel(pixel, bp.width, bp.height);
     emit_camera_ray_at(cams[vp.view], bp, q, slot, slot, pixel + key_offset, vp.x, vp.y, bp.s0 + j);
+}
+
+// Queue 0 of an adaptive multi-view batch (rt_gpu_render_views_adaptive): k_generate_active (adaptive.cuh) over the
+// stacked image.  The list holds stacked pixels; bp is the unshifted stacked batch (pix0 / npix = the whole range,
+// height the height of one view), so the radiance slot j * npix + (pixel - pix0) is the one k_shade derives from the
+// key pixel + key_offset with its pix0 shifted by the same key_offset.
+__global__ void __launch_bounds__(256) k_generate_active_views(const Camera *__restrict__ cams, BatchParams bp, Queues q,
+                                                               const uint32_t *__restrict__ list, const uint32_t *__restrict__ active,
+                                                               uint32_t key_offset) {
+    const uint32_t n_act = *active;
+    const uint32_t n = n_act * bp.k;
+    const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
+    if (slot == 0) {
+        q.count[0] = n;
+        atomicAdd(q.stats + 3, static_cast<unsigned long long>(n));
+    }
+    if (slot >= n) return;
+    const uint32_t j = slot / n_act;
+    const uint32_t li = slot - j * n_act;
+    const uint32_t pixel = list[li];
+    const ViewPixel vp = split_view_pixel(pixel, bp.width, bp.height);
+    emit_camera_ray_at(cams[vp.view], bp, q, slot, j * bp.npix + (pixel - bp.pix0), pixel + key_offset, vp.x, vp.y, bp.s0 + j);
 }
 
 }  // namespace rt

@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu
 SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upload_text_scene", "rt_gpu_render", "rt_gpu_readback",
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
            "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive",
-           "rt_gpu_render_views"]
+           "rt_gpu_render_views", "rt_gpu_render_views_adaptive"]
 
 _lib = None
 
@@ -34,6 +34,8 @@ def lib():
         L.rt_gpu_readback.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_gpu_render_adaptive.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params)]
         L.rt_gpu_render_views.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views)]
+        L.rt_gpu_render_views_adaptive.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views),
+                                                   C.POINTER(rt_adaptive_params)]
         L.rt_gpu_readback_adaptive.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.rt_gpu_accum_device_ptr.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
         L.rt_gpu_readback_rgb8.argtypes = [C.c_void_p, C.c_void_p]
@@ -139,17 +141,31 @@ class RtGpu:
         self._last = (width, height, RT_MODE_BEAUTY)
         self._views = None
 
+    def render_views_adaptive(self, cameras, width, height, max_samples, min_samples, step_samples, rel_error, abs_floor=1e-3,
+                              seed=0, view_base=0, max_paths_in_flight=0, pixel_begin=0, pixel_end=0):
+        """Adaptive multi-view render (rt_gpu_render_views_adaptive): render_adaptive over the stacked image of
+        render_views (pixel_begin / pixel_end index it; pixel p of view v is keyed (view_base + v) * W * H + p).
+        readback(), readback_rgb8() and readback_adaptive() then return [V, H, W, ...]."""
+        cams = (rt_camera * max(len(cameras), 1))(*[c.to_c() for c in cameras])
+        v = rt_views(len(cameras), view_base, cams)
+        p = rt_render_params(width, height, max_samples, 0, 0, RT_MODE_BEAUTY, seed, max_paths_in_flight, 0, pixel_begin,
+                             pixel_end)
+        a = rt_adaptive_params(min_samples, step_samples, rel_error, abs_floor)
+        _check(lib().rt_gpu_render_views_adaptive(self._h, C.byref(p), C.byref(v), C.byref(a)), "rt_gpu_render_views_adaptive")
+        self._last = (width, height, RT_MODE_BEAUTY)
+        self._views = len(cameras)
+
     def readback_adaptive(self):
-        """(sample counts uint32 [H, W], err float32 [H, W]) of the last adaptive render."""
-        w, h, _ = self._last
-        counts = np.empty((h, w), np.uint32)
-        err = np.empty((h, w), np.float32)
+        """(sample counts uint32 [H, W], err float32 [H, W]) of the last adaptive render; [V, H, W] each after
+        render_views_adaptive."""
+        counts = np.empty(self._shape(), np.uint32)
+        err = np.empty(self._shape(), np.float32)
         _check(lib().rt_gpu_readback_adaptive(self._h, counts.ctypes.data_as(C.c_void_p), err.ctypes.data_as(C.c_void_p)),
                "rt_gpu_readback_adaptive")
         return counts, err
 
     def readback(self):
-        """(rgb_mean float32 [H, W, 3], or [V, H, W, 3] after render_views; stats dict) of the last beauty render."""
+        """(rgb_mean float32 [H, W, 3], or [V, H, W, 3] after render_views / render_views_adaptive; stats dict) of the last beauty render."""
         out = np.empty(self._shape(3), np.float32)
         st = rt_stats()
         _check(lib().rt_gpu_readback(self._h, out.ctypes.data_as(C.c_void_p), None, C.byref(st)), "rt_gpu_readback")
