@@ -342,6 +342,44 @@ int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const r
 int rt_gpu_render_views_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views,
                                  const rt_adaptive_params *ap);
 
+/* ---- camera projections -----------------------------------------------------------------------------------------
+ * rt_gpu_render_projected renders the views of rt_views, each through its own projection of its camera (position and
+ * right / up / forward basis; fov_x is used by the pinhole and thin-lens kinds only).  For image point (px, py) in
+ * pixels (centres at + 0.5), with W x H the size of one view:
+ *   RT_PROJ_PINHOLE        the camera ray of rt_gpu_render_views, bit for bit;
+ *   RT_PROJ_THIN_LENS      d = the pinhole direction; focus = position + d * focus_distance / dot(d, forward) (the plane
+ *                          in focus lies focus_distance along forward); the ray starts at a uniform point of the lens disc
+ *                          of aperture_radius spanned by right and up and passes through focus.  aperture_radius == 0 is
+ *                          the pinhole, bit for bit;
+ *   RT_PROJ_ORTHOGRAPHIC   origin position + a * right - b * up with a = (2 px / W - 1) * half_width,
+ *                          b = (2 py / H - 1) * half_height (glTF xmag / ymag), direction forward (normalised);
+ *   RT_PROJ_EQUIRECT       u = (px - 0.5) / W, v = (py - 0.5) / H, phi = (u - 0.5) * 2 pi, theta = (0.5 - v) * pi,
+ *                          d = cos(theta) sin(phi) * right + sin(theta) * up + cos(theta) cos(phi) * forward, normalised:
+ *                          the full sphere, forward at the image centre.  With forward = +x, right = +z, up = +y a view
+ *                          of the environment map's size looks up texel (i, j) at the centre of pixel (i, j).
+ * Lens samples use their own Philox stream (counter word 2 = 0xFFFFFFFE); every other random number of a path is the
+ * one rt_gpu_render_views draws.  RT_MODE_PRIMARY_IDS traces pixel centres through the lens centre.
+ * ap == NULL: the contract of rt_gpu_render_views (image, keys, readbacks, accumulation, multi-device split).
+ * ap != NULL: the contract of rt_gpu_render_views_adaptive.  So all-pinhole projections give exactly those calls.
+ * RT_ERR_INVALID_ARG for everything the corresponding view call refuses, and for projections == NULL, an unknown kind,
+ * a non-finite field, aperture_radius < 0, focus_distance <= 0 with aperture_radius > 0, and half_width or
+ * half_height <= 0 for RT_PROJ_ORTHOGRAPHIC.  Fields a kind does not use are ignored. */
+#define RT_PROJ_PINHOLE 0u
+#define RT_PROJ_THIN_LENS 1u
+#define RT_PROJ_ORTHOGRAPHIC 2u
+#define RT_PROJ_EQUIRECT 3u
+
+typedef struct rt_projection {
+    uint32_t kind;          /* RT_PROJ_* */
+    float aperture_radius;  /* thin lens: radius of the lens disc (world units); 0 = pinhole */
+    float focus_distance;   /* thin lens: distance of the plane in focus along forward; > 0 when aperture_radius > 0 */
+    float half_width;       /* orthographic: half the view's extent along right (glTF xmag); > 0 */
+    float half_height;      /* orthographic: half the view's extent along up (glTF ymag); > 0 */
+} rt_projection;
+
+int rt_gpu_render_projected(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views,
+                            const rt_projection *projections /* n_views */, const rt_adaptive_params *ap /* NULL = fixed */);
+
 /* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene.
  * which = 0: uint32[8] {n_tris, binary node slots, 4-wide nodes, root link, worst-case traversal stack need, depth of
  * the binary tree, 1 if built on the device, levels of the top-down phase}; 1: rt_bvh_node[slots] (the binary tree in the

@@ -64,6 +64,71 @@ class rt_views(C.Structure):
     _fields_ = [("n_views", C.c_uint32), ("view_base", C.c_uint32), ("cameras", C.POINTER(rt_camera))]
 
 
+RT_PROJ_PINHOLE, RT_PROJ_THIN_LENS, RT_PROJ_ORTHOGRAPHIC, RT_PROJ_EQUIRECT = 0, 1, 2, 3
+
+
+class rt_projection(C.Structure):
+    _fields_ = [("kind", C.c_uint32), ("aperture_radius", C.c_float), ("focus_distance", C.c_float), ("half_width", C.c_float),
+                ("half_height", C.c_float)]
+
+
+class Projection:
+    """How a view maps pixels to rays (rt_projection, include/rt_gpu.h): Projection.pinhole(), thin_lens(aperture_radius,
+    focus_distance), orthographic(half_width, half_height) (glTF xmag / ymag) or equirect().  Fields a kind does not use
+    are 0.  Two projections are equal when kind and every value are equal bit for bit."""
+
+    __slots__ = ("kind", "aperture_radius", "focus_distance", "half_width", "half_height")
+    NAMES = {RT_PROJ_PINHOLE: "pinhole", RT_PROJ_THIN_LENS: "thin_lens", RT_PROJ_ORTHOGRAPHIC: "ortho", RT_PROJ_EQUIRECT: "equirect"}
+
+    def __init__(self, kind=RT_PROJ_PINHOLE, aperture_radius=0.0, focus_distance=0.0, half_width=0.0, half_height=0.0):
+        self.kind = int(kind)
+        self.aperture_radius, self.focus_distance = np.float32(aperture_radius), np.float32(focus_distance)
+        self.half_width, self.half_height = np.float32(half_width), np.float32(half_height)
+
+    @classmethod
+    def pinhole(cls):
+        return cls(RT_PROJ_PINHOLE)
+
+    @classmethod
+    def thin_lens(cls, aperture_radius, focus_distance):
+        return cls(RT_PROJ_THIN_LENS, aperture_radius=aperture_radius, focus_distance=focus_distance)
+
+    @classmethod
+    def orthographic(cls, half_width, half_height):
+        return cls(RT_PROJ_ORTHOGRAPHIC, half_width=half_width, half_height=half_height)
+
+    @classmethod
+    def equirect(cls):
+        return cls(RT_PROJ_EQUIRECT)
+
+    @classmethod
+    def parse(cls, text):
+        """The CLI form: 'pinhole', 'thin_lens:<aperture>:<focus>', 'ortho:<half_w>:<half_h>' or 'equirect'."""
+        name, *args = text.split(":")
+        makers = {"pinhole": (cls.pinhole, 0), "thin_lens": (cls.thin_lens, 2), "ortho": (cls.orthographic, 2), "equirect": (cls.equirect, 0)}
+        if name not in makers or len(args) != makers[name][1]:
+            raise ValueError(f"projection {text!r}: expected pinhole, thin_lens:<aperture>:<focus>, ortho:<half_w>:<half_h> or equirect")
+        return makers[name][0](*(float(a) for a in args))
+
+    def to_c(self):
+        return rt_projection(self.kind, float(self.aperture_radius), float(self.focus_distance), float(self.half_width),
+                             float(self.half_height))
+
+    def _bits(self):
+        return (self.kind, np.array([self.aperture_radius, self.focus_distance, self.half_width, self.half_height],
+                                    np.float32).view(np.uint32).tolist())
+
+    def __eq__(self, other):
+        return isinstance(other, Projection) and self._bits() == other._bits()
+
+    __hash__ = None
+
+    def __repr__(self):
+        return (f"Projection({self.NAMES.get(self.kind, self.kind)}, aperture_radius={float(self.aperture_radius)!r}, "
+                f"focus_distance={float(self.focus_distance)!r}, half_width={float(self.half_width)!r}, "
+                f"half_height={float(self.half_height)!r})")
+
+
 class Camera:
     """A camera of a scene (rt_camera): position, the right / up / forward axes and the horizontal field of view fov_x
     in radians, all float32.  Two cameras are equal when every value is equal bit for bit."""
@@ -184,7 +249,8 @@ class SceneData:
         self.scene_bvh = BvhData(np.zeros(0, NODE_DTYPE), np.zeros(0, np.uint32), RT_NO_CHILD)
         self.light_bvh = BvhData(np.zeros(0, NODE_DTYPE), np.zeros(0, np.uint32), RT_NO_CHILD)
         self.cameras = []  # every camera node of the source glTF in traversal order (gltf.load_gltf); the scene's own
-                           # camera is the last of them
+                           # camera is the last perspective one
+        self.projections = []  # the Projection of each entry of `cameras`
 
     def camera(self):
         """The scene's own camera (the one rt_gpu_render uses) as a Camera."""

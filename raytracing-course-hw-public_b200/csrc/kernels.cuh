@@ -123,6 +123,16 @@ __device__ __forceinline__ uint32_t tiled_pixel(uint32_t pl, uint32_t width) {
     return (ty * 4u + (in >> 3)) * width + tx * 8u + (in & 7u);
 }
 
+// The queue-0 record of a camera ray (origin o, direction dir) of Philox key (pixel, sample) at queue position `slot`,
+// its radiance slot `rad_slot` cleared
+__device__ __forceinline__ void emit_ray_record(const BatchParams &bp, const Queues &q, uint32_t slot, uint32_t rad_slot, uint32_t pixel,
+                                                uint32_t sample, f3 o, f3 dir) {
+    q_store<2>(q.o_out + slot, make_float4(o.x, o.y, o.z, __uint_as_float(pixel)));
+    q_store<2>(q.d_out + slot, make_float4(dir.x, dir.y, dir.z, __uint_as_float(sample)));
+    q_store<2>(q.thr_out + slot, make_float4(1.0f, 1.0f, 1.0f, -1.0f));
+    q_store<3>(q.rad + rad_slot, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+}
+
 // The camera ray through pixel (px, py) of `cam` for Philox key (pixel, sample) into queue position `slot`, its radiance
 // slot `rad_slot` cleared.  The multi-view k_generate_views (views.cuh) keys a view's pixel apart from its (px, py).
 __device__ __forceinline__ void emit_camera_ray_at(const Camera &cam, const BatchParams &bp, const Queues &q, uint32_t slot, uint32_t rad_slot,
@@ -135,10 +145,7 @@ __device__ __forceinline__ void emit_camera_ray_at(const Camera &cam, const Batc
         jy = u01(r.y);
     }
     const f3 dir = camera_dir(cam, static_cast<float>(px) + jx, static_cast<float>(py) + jy);
-    q_store<2>(q.o_out + slot, make_float4(cam.pos.x, cam.pos.y, cam.pos.z, __uint_as_float(pixel)));
-    q_store<2>(q.d_out + slot, make_float4(dir.x, dir.y, dir.z, __uint_as_float(sample)));
-    q_store<2>(q.thr_out + slot, make_float4(1.0f, 1.0f, 1.0f, -1.0f));
-    q_store<3>(q.rad + rad_slot, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
+    emit_ray_record(bp, q, slot, rad_slot, pixel, sample, cam.pos, dir);
 }
 
 // The camera ray of row-major (pixel, sample).  k_generate and the adaptive k_generate_active (adaptive.cuh) both go

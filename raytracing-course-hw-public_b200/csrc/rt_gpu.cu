@@ -34,6 +34,7 @@
 #include "gpu_build.cuh"
 #include "adaptive.cuh"
 #include "views.cuh"
+#include "projection.cuh"
 #include "rt_gpu.h"
 
 namespace {
@@ -206,6 +207,7 @@ struct DeviceState {
     DevBuf<int32_t> prim_ids;
     DevBuf<uint8_t> rgb8;
     DevBuf<rt::Camera> cams;  // the cameras of the last multi-view render (rt_gpu_render_views), one per view
+    DevBuf<rt::Projection> projs;  // their projections when it was rt_gpu_render_projected
     int extend_blocks = 0, shade_blocks = 0, light_blocks = 0;
     rt::LightBox light_box{};  // box of all light triangles (k_shade tests the rays it queues against it)
     // profiling
@@ -540,11 +542,24 @@ rt_camera scene_camera(const DScene &s) {
     return c;
 }
 
-// The cameras of a multi-view render (rt_gpu_render_views), one per view, and the Philox key of its first view
+// The cameras of a multi-view render (rt_gpu_render_views), one per view, and the Philox key of its first view.
+// rt_gpu_render_projected adds one projection per view (projection.cuh); without them queue 0 is k_generate_views.
+static_assert(sizeof(rt::Projection) == sizeof(rt_projection) && rt::kProjPinhole == RT_PROJ_PINHOLE && rt::kProjThinLens == RT_PROJ_THIN_LENS &&
+                  rt::kProjOrthographic == RT_PROJ_ORTHOGRAPHIC && rt::kProjEquirect == RT_PROJ_EQUIRECT,
+              "rt::Projection mirrors rt_projection");
 struct ViewSet {
     std::vector<rt::Camera> cams;
+    std::vector<rt::Projection> projs;
     uint32_t view_base = 0;
 };
+
+// Uploads the cameras of `views` (and their projections) to device d on its stream
+int upload_views(DeviceState &d, const ViewSet &views) {
+    if (int rc = d.cams.upload(views.cams, d.stream)) return rc;
+    if (!views.projs.empty())
+        if (int rc = d.projs.upload(views.projs, d.stream)) return rc;
+    return RT_OK;
+}
 
 void mark(rt_gpu_ctx *ctx, DeviceState &d, int kind) {
     if (!ctx->profiling) return;
@@ -752,7 +767,7 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
     if (int rc = d.counters.alloc(n_counters)) return rc;
     const rt::Queues q_gen = queues_of(d, qdepth, -1);
     if (views)
-        if (int rc = d.cams.upload(views->cams, d.stream)) return rc;
+        if (int rc = upload_views(d, *views)) return rc;
     // per-kernel profiling needs the kernels one after the other on one stream
     const bool split_allowed = !ids_mode && !ctx->profiling && !std::getenv("RT_NO_SPLIT");
 
@@ -777,7 +792,9 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
             bp.tiled = !ids_mode && pix0 == 0 && npix == n_pix && W % 8 == 0 && (H * n_views) % 4 == 0 && !std::getenv("RT_NO_TILES");
             const uint32_t n = bp.npix * bp.k;
             CU_CHECK(cudaMemsetAsync(d.counters.p, 0, n_counters * sizeof(uint32_t), d.stream));
-            if (views)
+            if (views && !views->projs.empty())
+                rt::k_generate_proj<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, d.projs.p, bp, q_gen, key_offset);
+            else if (views)
                 rt::k_generate_views<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, bp, q_gen, key_offset);
             else
                 rt::k_generate<<<(n + 255) / 256, 256, 0, d.stream>>>(cam, bp, q_gen);
@@ -848,7 +865,7 @@ int setup_adaptive(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_params &rp
         if (int rc = d.awords.alloc(2 * static_cast<size_t>(run.n_words))) return rc;
     }
     if (views)
-        if (int rc = d.cams.upload(views->cams, d.stream)) return rc;
+        if (int rc = upload_views(d, *views)) return rc;
     d.apix0 = pix0;
     d.apix1 = pix1;
     CU_CHECK(cudaMemsetAsync(d.stats.p, 0, 4 * sizeof(unsigned long long), d.stream));
@@ -901,7 +918,9 @@ int enqueue_adaptive_round(rt_gpu_ctx *ctx, AdaptiveRun &run, const rt_render_pa
         bp.k = std::min(run.k_max, k - j0);
         const uint32_t n = npix * bp.k;  // the grid of k_generate_active; the queue holds n_active * k paths
         CU_CHECK(cudaMemsetAsync(d.counters.p, 0, n_counters_of(qdepth) * sizeof(uint32_t), d.stream));
-        if (views)
+        if (views && !views->projs.empty())
+            rt::k_generate_active_proj<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, d.projs.p, bp, q_gen, list, active, run.key_offset);
+        else if (views)
             rt::k_generate_active_views<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, bp, q_gen, list, active, run.key_offset);
         else
             rt::k_generate_active<<<(n + 255) / 256, 256, 0, d.stream>>>(run.cam, bp, q_gen, list, active);
@@ -1372,6 +1391,34 @@ int check_views(const rt_render_params &rp, const rt_views &views, const std::st
     return RT_OK;
 }
 
+// The checks of the projections of rt_gpu_render_projected (one per view of vs, already checked by check_views).
+// Fills vs.projs.  Fields a kind does not use are not looked at.
+int check_projections(const rt_projection *projections, const std::string &who, ViewSet &vs) {
+    vs.projs.clear();
+    for (size_t v = 0; v < vs.cams.size(); ++v) {
+        const rt_projection &p = projections[v];
+        const std::string at = who + ": projection " + std::to_string(v);
+        rt::Projection q{p.kind, 0.0f, 0.0f, 0.0f, 0.0f};
+        if (p.kind == RT_PROJ_THIN_LENS) {
+            if (!std::isfinite(p.aperture_radius) || !std::isfinite(p.focus_distance)) return fail(RT_ERR_INVALID_ARG, at + " has a non-finite value");
+            if (p.aperture_radius < 0.0f) return fail(RT_ERR_INVALID_ARG, at + ": aperture_radius < 0");
+            if (p.aperture_radius > 0.0f && !(p.focus_distance > 0.0f))
+                return fail(RT_ERR_INVALID_ARG, at + ": focus_distance <= 0 with a non-zero aperture");
+            q.aperture_radius = p.aperture_radius;
+            q.focus_distance = p.focus_distance;
+        } else if (p.kind == RT_PROJ_ORTHOGRAPHIC) {
+            if (!std::isfinite(p.half_width) || !std::isfinite(p.half_height)) return fail(RT_ERR_INVALID_ARG, at + " has a non-finite value");
+            if (!(p.half_width > 0.0f) || !(p.half_height > 0.0f)) return fail(RT_ERR_INVALID_ARG, at + ": half_width / half_height <= 0");
+            q.half_width = p.half_width;
+            q.half_height = p.half_height;
+        } else if (p.kind != RT_PROJ_PINHOLE && p.kind != RT_PROJ_EQUIRECT) {
+            return fail(RT_ERR_INVALID_ARG, at + ": unknown kind " + std::to_string(p.kind));
+        }
+        vs.projs.push_back(q);
+    }
+    return RT_OK;
+}
+
 // The checks of an adaptive render's parameters over an image of n_pixels; resolves rp.pixel_end
 int check_adaptive(rt_render_params &rp, const rt_adaptive_params &ap, uint64_t n_pixels, const std::string &who) {
     if (rp.mode != RT_MODE_BEAUTY) return fail(RT_ERR_INVALID_ARG, who + ": beauty renders only");
@@ -1422,6 +1469,45 @@ int render_adaptive_on_devices(rt_gpu_ctx *ctx, const rt_render_params &rp, cons
     return RT_OK;
 }
 
+// rt_gpu_render_views (projections == nullptr) and the fixed form of rt_gpu_render_projected after their null checks
+int render_views_checked(rt_gpu_ctx *ctx, const rt_render_params &params, const rt_views &views, const rt_projection *projections,
+                         const std::string &who) {
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, who + ": no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, who + ": not available for course text scenes");
+    rt_render_params rp = params;
+    ViewSet vs;
+    if (int rc = check_views(rp, views, who, vs)) return rc;
+    if (projections)
+        if (int rc = check_projections(projections, who, vs)) return rc;
+    const uint64_t per_view = static_cast<uint64_t>(rp.width) * rp.height, V = views.n_views;
+    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, who + ": samples == 0");
+    if (rp.sample_end == 0) rp.sample_end = rp.samples;
+    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, who + ": sample_begin > sample_end");
+    const uint64_t n_pixels = per_view * V;
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, who + ": illegal pixel range");
+    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY &&
+        (!ctx->have_render || ctx->adaptive_sums || ctx->last.width != rp.width || ctx->last.height != rp.height ||
+         std::max(ctx->last_views, 1u) != views.n_views))
+        return fail(RT_ERR_INVALID_ARG, who + ": RT_FLAG_ACCUMULATE needs a previous render of the same width, height and n_views");
+    return render_on_devices(ctx, rp, &vs);
+}
+
+// rt_gpu_render_views_adaptive (projections == nullptr) and the adaptive form of rt_gpu_render_projected after their
+// null checks
+int render_views_adaptive_checked(rt_gpu_ctx *ctx, const rt_render_params &params, const rt_views &views, const rt_projection *projections,
+                                  const rt_adaptive_params &ap, const std::string &who) {
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, who + ": no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, who + ": not available for course text scenes");
+    rt_render_params rp = params;
+    ViewSet vs;
+    if (int rc = check_views(rp, views, who, vs)) return rc;
+    if (projections)
+        if (int rc = check_projections(projections, who, vs)) return rc;
+    if (int rc = check_adaptive(rp, ap, static_cast<uint64_t>(rp.width) * rp.height * views.n_views, who)) return rc;
+    return render_adaptive_on_devices(ctx, rp, ap, &vs);
+}
+
 }  // namespace
 
 int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
@@ -1446,23 +1532,7 @@ int rt_gpu_render(rt_gpu_ctx *ctx, const rt_render_params *params) {
 
 int rt_gpu_render_views(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views) {
     if (!ctx || !params || !views) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: null argument");
-    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_render_views: no scene uploaded");
-    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: not available for course text scenes");
-    rt_render_params rp = *params;
-    ViewSet vs;
-    if (int rc = check_views(rp, *views, "rt_gpu_render_views", vs)) return rc;
-    const uint64_t per_view = static_cast<uint64_t>(rp.width) * rp.height, V = views->n_views;
-    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: samples == 0");
-    if (rp.sample_end == 0) rp.sample_end = rp.samples;
-    if (rp.sample_begin > rp.sample_end) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: sample_begin > sample_end");
-    const uint64_t n_pixels = per_view * V;
-    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
-    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: illegal pixel range");
-    if ((rp.flags & RT_FLAG_ACCUMULATE) && rp.mode == RT_MODE_BEAUTY &&
-        (!ctx->have_render || ctx->adaptive_sums || ctx->last.width != rp.width || ctx->last.height != rp.height ||
-         std::max(ctx->last_views, 1u) != views->n_views))
-        return fail(RT_ERR_INVALID_ARG, "rt_gpu_render_views: RT_FLAG_ACCUMULATE needs a previous render of the same width, height and n_views");
-    return render_on_devices(ctx, rp, &vs);
+    return render_views_checked(ctx, *params, *views, nullptr, "rt_gpu_render_views");
 }
 
 int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_adaptive_params *ap) {
@@ -1479,13 +1549,15 @@ int rt_gpu_render_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, cons
 int rt_gpu_render_views_adaptive(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views, const rt_adaptive_params *ap) {
     const std::string who = "rt_gpu_render_views_adaptive";
     if (!ctx || !params || !views || !ap) return fail(RT_ERR_INVALID_ARG, who + ": null argument");
-    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, who + ": no scene uploaded");
-    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, who + ": not available for course text scenes");
-    rt_render_params rp = *params;
-    ViewSet vs;
-    if (int rc = check_views(rp, *views, who, vs)) return rc;
-    if (int rc = check_adaptive(rp, *ap, static_cast<uint64_t>(rp.width) * rp.height * views->n_views, who)) return rc;
-    return render_adaptive_on_devices(ctx, rp, *ap, &vs);
+    return render_views_adaptive_checked(ctx, *params, *views, nullptr, *ap, who);
+}
+
+int rt_gpu_render_projected(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views, const rt_projection *projections,
+                            const rt_adaptive_params *ap) {
+    const std::string who = "rt_gpu_render_projected";
+    if (!ctx || !params || !views || !projections) return fail(RT_ERR_INVALID_ARG, who + ": null argument");
+    if (!ap) return render_views_checked(ctx, *params, *views, projections, who);
+    return render_views_adaptive_checked(ctx, *params, *views, projections, *ap, who);
 }
 
 int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error) {

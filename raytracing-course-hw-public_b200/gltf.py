@@ -22,7 +22,7 @@ import os
 import numpy as np
 
 from . import host
-from ._abi import MATERIAL_DTYPE, TEXTURE_DTYPE, Camera, SceneData
+from ._abi import MATERIAL_DTYPE, TEXTURE_DTYPE, Camera, Projection, SceneData
 
 F = np.float32
 _libm = ctypes.CDLL(ctypes.util.find_library("m") or "libm.so.6")
@@ -177,7 +177,8 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
         return buffers[int(view["buffer"])][off:off + count * dt.itemsize].view(dt).astype(np.int64)
 
     cam = {}
-    cameras = []  # every camera node, in traversal order; the reference keeps only the last (cam)
+    cameras = []  # every camera node, in traversal order; the reference keeps only the last perspective one (cam)
+    projections = []  # the projection of each entry of `cameras`
     pos_chunks, nrm_chunks, uv_chunks, tan_chunks, mat_chunks = [], [], [], [], []
     materials = []
     mat_index = {}
@@ -229,9 +230,7 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
         normal_transform = _normal_matrix(transform)
 
         if "camera" in node:
-            persp = doc["cameras"][int(node["camera"])]["perspective"]
-            fov_y = F(persp["yfov"])
-            ar = F(persp["aspectRatio"]) if "aspectRatio" in persp else F(aspect_ratio)
+            cdef = doc["cameras"][int(node["camera"])]
 
             def col_dir(v):  # norm(transform * vec4(v, 0)).xyz with vec4 length
                 r = np.array([F(F(F(F(transform[i, 0] * v[0]) + F(transform[i, 1] * v[1])) + F(transform[i, 2] * v[2]))
@@ -239,12 +238,24 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
                 ln = np.sqrt(F(F(F(r[0] * r[0]) + F(r[1] * r[1])) + F(r[2] * r[2])) + F(r[3] * r[3]))
                 return (r / ln)[:3]
 
+        if "camera" in node and "perspective" not in cdef and "orthographic" in cdef:
+            # an orthographic node joins `cameras` only: the scene camera (the reference's, which reads perspective
+            # cameras alone) stays the last perspective node; fov_x is unused by the projection
+            ortho = cdef["orthographic"]
+            cameras.append(Camera(transform[:3, 3].copy(), col_dir(np.array([1, 0, 0], F)), col_dir(np.array([0, 1, 0], F)),
+                                  col_dir(np.array([0, 0, -1], F)), F(0)))
+            projections.append(Projection.orthographic(F(ortho["xmag"]), F(ortho["ymag"])))
+        elif "camera" in node:
+            persp = cdef["perspective"]
+            fov_y = F(persp["yfov"])
+            ar = F(persp["aspectRatio"]) if "aspectRatio" in persp else F(aspect_ratio)
             cam["position"] = transform[:3, 3].copy()
             cam["forward"] = col_dir(np.array([0, 0, -1], F))
             cam["up"] = col_dir(np.array([0, 1, 0], F))
             cam["right"] = col_dir(np.array([1, 0, 0], F))
             cam["fov_x"] = F(atanf(F(tanf(F(fov_y / F(2))) * ar)) * F(2))
             cameras.append(Camera(cam["position"], cam["right"], cam["up"], cam["forward"], cam["fov_x"]))
+            projections.append(Projection.pinhole())
 
         if "mesh" in node:
             for prim in doc["meshes"][int(node["mesh"])]["primitives"]:
@@ -298,6 +309,7 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
 
     s = SceneData()
     s.cameras = cameras
+    s.projections = projections
     if cam:
         s.camera_position, s.camera_right = cam["position"], cam["right"]
         s.camera_up, s.camera_forward, s.fov_x = cam["up"], cam["forward"], cam["fov_x"]

@@ -6,8 +6,8 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_camera, rt_render_params,
-                   rt_scene_desc, rt_stats, rt_views)
+from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_camera, rt_projection,
+                   rt_render_params, rt_scene_desc, rt_stats, rt_views)
 
 # RT_GPU_LIB selects another build of the same C ABI (kernel A/B experiments, tools/build_variants.sh)
 LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu.so")
@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu
 SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upload_text_scene", "rt_gpu_render", "rt_gpu_readback",
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
            "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive",
-           "rt_gpu_render_views", "rt_gpu_render_views_adaptive"]
+           "rt_gpu_render_views", "rt_gpu_render_views_adaptive", "rt_gpu_render_projected"]
 
 _lib = None
 
@@ -36,6 +36,8 @@ def lib():
         L.rt_gpu_render_views.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views)]
         L.rt_gpu_render_views_adaptive.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views),
                                                    C.POINTER(rt_adaptive_params)]
+        L.rt_gpu_render_projected.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views), C.POINTER(rt_projection),
+                                              C.POINTER(rt_adaptive_params)]
         L.rt_gpu_readback_adaptive.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.rt_gpu_accum_device_ptr.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
         L.rt_gpu_readback_rgb8.argtypes = [C.c_void_p, C.c_void_p]
@@ -155,6 +157,24 @@ class RtGpu:
         self._last = (width, height, RT_MODE_BEAUTY)
         self._views = len(cameras)
 
+    def render_projected(self, cameras, projections, width, height, samples, seed=0, view_base=0, sample_begin=0, sample_end=0,
+                         mode=RT_MODE_BEAUTY, max_paths_in_flight=0, accumulate=False, pixel_begin=0, pixel_end=0, adaptive=None):
+        """Projected multi-view render (rt_gpu_render_projected): render_views with projections[v] (a Projection) applied
+        to cameras[v].  adaptive=None renders a fixed spp with render_views' contract; adaptive=(min_samples,
+        step_samples, rel_error[, abs_floor]) renders with render_views_adaptive's contract, `samples` being the maximum
+        spp.  readback(), readback_rgb8() and, when adaptive, readback_adaptive() then return [V, H, W, ...]."""
+        if len(projections) != len(cameras):
+            raise ValueError(f"render_projected: {len(cameras)} cameras but {len(projections)} projections")
+        cams = (rt_camera * max(len(cameras), 1))(*[c.to_c() for c in cameras])
+        projs = (rt_projection * max(len(projections), 1))(*[pj.to_c() for pj in projections])
+        v = rt_views(len(cameras), view_base, cams)
+        p = rt_render_params(width, height, samples, sample_begin, sample_end, mode, seed, max_paths_in_flight,
+                             RT_FLAG_ACCUMULATE if accumulate else 0, pixel_begin, pixel_end)
+        a = None if adaptive is None else C.byref(rt_adaptive_params(*adaptive) if len(adaptive) == 4 else rt_adaptive_params(*adaptive, 1e-3))
+        _check(lib().rt_gpu_render_projected(self._h, C.byref(p), C.byref(v), projs, a), "rt_gpu_render_projected")
+        self._last = (width, height, mode)
+        self._views = len(cameras)
+
     def readback_adaptive(self):
         """(sample counts uint32 [H, W], err float32 [H, W]) of the last adaptive render; [V, H, W] each after
         render_views_adaptive."""
@@ -187,10 +207,13 @@ class RtGpu:
         _check(lib().rt_gpu_readback_rgb8(self._h, out.ctypes.data_as(C.c_void_p)), "rt_gpu_readback_rgb8")
         return out
 
-    def primary_ids(self, width, height, cameras=None, view_base=0):
-        """Primary-hit ids [H, W] of the scene's camera, or [V, H, W] of `cameras` (render_views)."""
+    def primary_ids(self, width, height, cameras=None, view_base=0, projections=None):
+        """Primary-hit ids [H, W] of the scene's camera, or [V, H, W] of `cameras` (render_views; render_projected with
+        `projections`)."""
         if cameras is None:
             self.render(width, height, 1, mode=RT_MODE_PRIMARY_IDS)
+        elif projections is not None:
+            self.render_projected(cameras, projections, width, height, 1, view_base=view_base, mode=RT_MODE_PRIMARY_IDS)
         else:
             self.render_views(cameras, width, height, 1, view_base=view_base, mode=RT_MODE_PRIMARY_IDS)
         ids = np.empty(self._shape(), np.int32)

@@ -23,6 +23,8 @@
 //             reference's compile-time USE_ENV_MAP / ENV_MAP_PATH, src/config.h:35-37)
 //   RT_ADAPTIVE  relative-error target of an adaptive render (rt_gpu_render_adaptive, glTF scenes): <samples> becomes
 //             the maximum spp, min_samples = step_samples = max(2, ceil(samples / 16)); the samples traced on stderr
+//   RT_PROJECTION  projection of the scene camera (rt_gpu_render_projected, glTF scenes): thin_lens:<aperture>:<focus>,
+//             ortho:<half_w>:<half_h>, equirect or pinhole; combines with RT_ADAPTIVE
 #define STB_IMAGE_IMPLEMENTATION
 
 #include <algorithm>
@@ -34,6 +36,7 @@
 #include <iostream>
 #include <memory>
 #include <stdexcept>
+#include <string>
 #include <vector>
 
 #include "config.h"
@@ -65,8 +68,35 @@ unsigned env_uint(const char *name, unsigned fallback) {
     return v && *v ? static_cast<unsigned>(std::strtoul(v, nullptr, 10)) : fallback;
 }
 
-// render what was uploaded and feed the float means to the reference's Image::set_pixel (image.h:40)
-void render_into(rt_gpu_ctx *gpu, unsigned width, unsigned height, unsigned samples, Image &img) {
+// RT_PROJECTION's value -> p; false when it is malformed
+bool parse_projection(const std::string &v, rt_projection &p) {
+    p = rt_projection{};
+    const size_t c1 = v.find(':'), c2 = c1 == std::string::npos ? c1 : v.find(':', c1 + 1);
+    const std::string name = v.substr(0, c1);
+    if (name == "pinhole" || name == "equirect") {
+        p.kind = name == "pinhole" ? RT_PROJ_PINHOLE : RT_PROJ_EQUIRECT;
+        return c1 == std::string::npos;
+    }
+    if ((name != "thin_lens" && name != "ortho") || c2 == std::string::npos || v.find(':', c2 + 1) != std::string::npos) return false;
+    char *end1 = nullptr, *end2 = nullptr;
+    const std::string a = v.substr(c1 + 1, c2 - c1 - 1), b = v.substr(c2 + 1);
+    const float x = std::strtof(a.c_str(), &end1), y = std::strtof(b.c_str(), &end2);
+    if (a.empty() || b.empty() || *end1 || *end2) return false;
+    if (name == "thin_lens") {
+        p.kind = RT_PROJ_THIN_LENS;
+        p.aperture_radius = x;
+        p.focus_distance = y;
+    } else {
+        p.kind = RT_PROJ_ORTHOGRAPHIC;
+        p.half_width = x;
+        p.half_height = y;
+    }
+    return true;
+}
+
+// render what was uploaded and feed the float means to the reference's Image::set_pixel (image.h:40).  camera: the
+// scene camera that RT_PROJECTION applies to (nullptr: text scene, where it is refused).
+void render_into(rt_gpu_ctx *gpu, unsigned width, unsigned height, unsigned samples, Image &img, const rt_camera *camera) {
     rt_render_params params{};
     params.width = width;
     params.height = height;
@@ -77,11 +107,20 @@ void render_into(rt_gpu_ctx *gpu, unsigned width, unsigned height, unsigned samp
     // library's 512 Mi (68 GB) cost 1.7 % of the render and save ~0.15 s of cudaMalloc / cudaFree (RT_PATHS overrides).
     params.max_paths_in_flight = env_uint("RT_PATHS", 128u << 20);
     const char *adaptive = std::getenv("RT_ADAPTIVE");
-    if (adaptive && *adaptive) {
-        rt_adaptive_params ap{};
-        ap.min_samples = ap.step_samples = std::max(2u, (samples + 15) / 16);
-        ap.rel_error = std::strtof(adaptive, nullptr);
-        ap.abs_floor = 1e-3f;
+    rt_adaptive_params ap{};
+    ap.min_samples = ap.step_samples = std::max(2u, (samples + 15) / 16);
+    ap.rel_error = adaptive && *adaptive ? std::strtof(adaptive, nullptr) : 0.0f;
+    ap.abs_floor = 1e-3f;
+    const char *projection = std::getenv("RT_PROJECTION");
+    if (projection && *projection) {
+        rt_projection proj;
+        if (!camera) throw std::runtime_error("RT_PROJECTION applies to glTF scenes only");
+        if (!parse_projection(projection, proj))
+            throw std::runtime_error(std::string("RT_PROJECTION=") + projection +
+                                     ": expected thin_lens:<aperture>:<focus>, ortho:<half_w>:<half_h>, equirect or pinhole");
+        const rt_views views{1, 0, camera};
+        check(rt_gpu_render_projected(gpu, &params, &views, &proj, adaptive && *adaptive ? &ap : nullptr), "rt_gpu_render_projected");
+    } else if (adaptive && *adaptive) {
         check(rt_gpu_render_adaptive(gpu, &params, &ap), "rt_gpu_render_adaptive");
     } else {
         check(rt_gpu_render(gpu, &params), "rt_gpu_render");
@@ -121,7 +160,7 @@ int run_text_scene(const char *path, unsigned width, unsigned height, unsigned s
         rt_gpu_ctx *gpu = nullptr;
         check(rt_gpu_create(&gpu, static_cast<int>(env_uint("RT_GPUS", 1)), 0), "rt_gpu_create");
         check(rt_gpu_upload_text_scene(gpu, ts), "rt_gpu_upload_text_scene");
-        render_into(gpu, width, height, samples, img);
+        render_into(gpu, width, height, samples, img, nullptr);
         rt_gpu_destroy(gpu);
     }
     rt_text_scene_free(ts);
@@ -177,7 +216,7 @@ int main(int argc, char **argv) try {
         clock.lap("rt_gpu_create (CUDA init)");
         check(rt_gpu_upload_scene(gpu, &flat.desc), "rt_gpu_upload_scene");
         clock.lap("rt_gpu_upload_scene");
-        render_into(gpu, width, height, samples, img);
+        render_into(gpu, width, height, samples, img, &flat.desc.camera);
         clock.lap("render + readback + set_pixel");
         rt_gpu_destroy(gpu);
         clock.lap("rt_gpu_destroy");
