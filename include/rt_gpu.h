@@ -380,7 +380,44 @@ typedef struct rt_projection {
 int rt_gpu_render_projected(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views,
                             const rt_projection *projections /* n_views */, const rt_adaptive_params *ap /* NULL = fixed */);
 
-/* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene.
+/* ---- animated geometry ------------------------------------------------------------------------------------------
+ * rt_gpu_update_geometry moves the triangles of the uploaded scene in place: positions, normals, tangents and the light
+ * BVH are replaced, with the meaning they have in rt_scene_desc; triangles, uv, materials, textures, camera, sky, flags
+ * and ray depth stay as uploaded.  The scene BVH keeps its topology (binary tree, triangle order, and which binary nodes
+ * form each 4-wide node with which children): every box is refit to the new positions and re-quantised.  So:
+ *   - the link words of rt_gpu_debug_get_bvh selector 3 and the counts of selector 0 do not change, nor does the
+ *     traversal-stack need (an update never fails on RT_EXT_STACK_CAP);
+ *   - upload(A); update(B); update(A) leaves the device scene byte-identical to upload(A), and update(A) right after
+ *     upload(A) changes nothing;
+ *   - afterwards selectors 1..4 describe the refit tree: binary boxes are the exact union of what lies below them,
+ *     quantised boxes contain every vertex below them and the device triangles hold the new positions.
+ * A tree refit far from the positions it was built for traces slower (its boxes overlap more); a re-upload builds a
+ * new tree.  The light side becomes what rt_gpu_upload_scene makes of light_bvh and the new positions: light nodes,
+ * light triangles, the sampling list, the light normals and areas, and the light box.
+ * The last render's sums, counts, ids and stats are left alone, and so are the accumulation rules: RT_FLAG_ACCUMULATE
+ * on the next render adds samples of the new geometry to the old sums (motion blur by sub-frame accumulation).
+ * RT_ERR_NO_SCENE before any upload.  RT_ERR_INVALID_ARG, with the scene untouched, for a null argument, a text scene,
+ * n_tris != the uploaded n_tris, a null tri_pos or tri_normals with n_tris > 0, a light BVH with another n_objects or
+ * with ids or links out of range, and a scene whose tree was not built on the device (uploaded with
+ * RT_SCENE_KEEP_HOST_BVH, RT_KEEP_HOST_BVH or RT_HOST_BUILD set, or by the 8-wide library: those trees live on the
+ * host; re-upload instead).  RT_ERR_BAD_SCENE for a non-finite vertex or a node that cannot be quantised: these are
+ * found on the device after the arrays were overwritten, so the handle then holds no scene and renders return
+ * RT_ERR_NO_SCENE until the next upload.  Every device of a handle is updated; the call returns after the device
+ * work is complete. */
+typedef struct rt_geometry_update {
+    uint32_t n_tris;            /* must equal the uploaded scene's n_tris */
+    uint32_t _pad;
+    const float *tri_pos;       /* n_tris*9, scene.objects order; required when n_tris > 0 */
+    const float *tri_normals;   /* n_tris*9; required when n_tris > 0 */
+    const float *tri_tangents;  /* n_tris*9 or NULL => (1,0,0), as in rt_scene_desc */
+    rt_bvh_desc light_bvh;      /* the light BVH over the NEW positions (what rt_scene_desc.light_bvh would be); same
+                                   n_objects as uploaded; empty when the scene has no emitters */
+} rt_geometry_update;
+
+int rt_gpu_update_geometry(rt_gpu_ctx *ctx, const rt_geometry_update *u);
+
+/* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene (with the
+ * boxes of any rt_gpu_update_geometry since).
  * which = 0: uint32[8] {n_tris, binary node slots, 4-wide nodes, root link, worst-case traversal stack need, depth of
  * the binary tree, 1 if built on the device, levels of the top-down phase}; 1: rt_bvh_node[slots] (the binary tree in the
  * slot layout left = i + 1, right = i + 2 * n_left; unused slots are undefined); 2: uint32[n_tris] scene.objects id at

@@ -175,6 +175,11 @@ class rt_scene_desc(C.Structure):
     ]
 
 
+class rt_geometry_update(C.Structure):
+    _fields_ = [("n_tris", C.c_uint32), ("_pad", C.c_uint32), ("tri_pos", C.c_void_p), ("tri_normals", C.c_void_p),
+                ("tri_tangents", C.c_void_p), ("light_bvh", rt_bvh_desc)]
+
+
 class rt_render_params(C.Structure):
     _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("samples", C.c_uint32), ("sample_begin", C.c_uint32),
                 ("sample_end", C.c_uint32), ("mode", C.c_uint32), ("seed", C.c_uint64),
@@ -271,6 +276,19 @@ class SceneData:
         self.materials = np.ascontiguousarray(self.materials, MATERIAL_DTYPE)
         self.textures = np.ascontiguousarray(self.textures, TEXTURE_DTYPE)
         self.texels = np.ascontiguousarray(self.texels, np.uint8)
+
+    def geometry_update(self):
+        """ctypes rt_geometry_update aliasing this object's positions, normals, tangents and light BVH (keep `self`
+        alive while it is used)."""
+        self._normalise()
+        u = rt_geometry_update()
+        u.n_tris = self.n_tris
+        u.tri_pos = _ptr(self.tri_pos)
+        u.tri_normals = _ptr(self.tri_normals)
+        u.tri_tangents = _ptr(self.tri_tangents)
+        u.light_bvh = self.light_bvh.desc()
+        u._owner = self
+        return u
 
     def without_scene_bvh(self):
         """Shallow copy that passes no scene BVH (rt_gpu.h: scene_bvh.n_nodes == 0 -> the library builds it)."""

@@ -54,6 +54,53 @@ def run_views(scene, cameras, width, height, samples, seed=0, n_gpus=1, projecti
         return rt.readback()
 
 
+def parse_frames(text):
+    """RT_FRAMES=<count>:<fps> -> (count >= 1, fps > 0)"""
+    try:
+        count, fps = text.split(":")
+        count, fps = int(count), float(fps)
+    except ValueError:
+        count, fps = 0, 0.0
+    if count < 1 or not (0 < fps < float("inf")):
+        raise ValueError(f"RT_FRAMES={text}: expected <count>:<fps> with count >= 1 and fps > 0")
+    return count, fps
+
+
+def run_frames(path, width, height, samples, count, fps, out, animation=0, seed=0, n_gpus=1, rel_error=None, projection=None,
+               env_map=None):
+    """Frames f = 0 .. count - 1 of a glTF animation, frame f at t0 + f / fps: frame 0 is uploaded, every later frame
+    moves the uploaded geometry (update_geometry; only the light BVH is built on the host).  Each frame renders its
+    camera through `projection` (pinhole by default) with seed + f, at `samples` spp or adaptively with rel_error, to
+    <stem>_<f><ext>.  The file's buffers and textures are read once."""
+    import time as clock
+
+    from . import gltf, gpu, host
+
+    src = gltf.GltfFile(path)
+    t0, _ = gltf.animation_range(src, animation)
+    paths = int(os.environ.get("RT_PATHS", 128 << 20))
+    proj = projection if projection is not None else Projection.pinhole()
+    step = adaptive_steps(samples)
+    with gpu.RtGpu(n_gpus, 0) as rt:
+        for f, frame_path in enumerate(view_paths(out, count)):
+            t = t0 + f / fps
+            c0 = clock.perf_counter()
+            scene = gltf.load_gltf(src, width / height, build_bvh=f == 0, env_map=env_map, time=t, animation=animation)
+            c1 = clock.perf_counter()
+            if f == 0:
+                rt.upload_scene(scene)
+            else:
+                rt.update_geometry(gltf.build_light_bvh(scene))
+            c2 = clock.perf_counter()
+            rt.render_projected([scene.camera()], [proj], width, height, samples, seed=seed + f, max_paths_in_flight=paths,
+                                adaptive=None if rel_error is None else (step, step, rel_error))
+            mean, stats = rt.readback()
+            host.write_ppm(frame_path, host.tonemap_rgb8(mean[0]))
+            print(f"rt_gpu frame {f} (t = {t:.6g} s): load {(c1 - c0) * 1e3:.1f} ms, {'upload' if f == 0 else 'update'} "
+                  f"{(c2 - c1) * 1e3:.1f} ms, render {stats['render_ms']:.1f} ms", file=sys.stderr)
+    return 0
+
+
 def view_paths(out, n):
     """<stem>_<i><ext> for the n views of RT_CAMERAS=all"""
     stem, ext = os.path.splitext(out)
@@ -69,11 +116,13 @@ def main(argv=None):
 
     try:
         width, height, samples = int(argv[2]), int(argv[3]), int(argv[4])
+        # RT_FRAMES=<count>:<fps> (RT_ANIMATION=<index>, default 0): frames of the glTF's animation, see run_frames
+        frames = os.environ.get("RT_FRAMES")
         if textscene.is_text_scene(argv[1]):
             # course text scenes (parity unpinned): width / height / samples of 0 take DIMENSIONS / SAMPLES of the file
             scene = textscene.load_text_scene(argv[1])
             width, height, samples = width or scene.width, height or scene.height, samples or scene.samples
-        else:
+        elif frames is None:
             scene = gltf.load_gltf(argv[1], width / height, env_map=os.environ.get("RT_ENV_MAP") or None)
         # RT_ADAPTIVE=<rel_error>: `samples` is the maximum spp; every pixel stops once its relative error is reached
         adaptive = os.environ.get("RT_ADAPTIVE")
@@ -92,8 +141,23 @@ def main(argv=None):
                 return 1
         else:
             projection = None
-        # RT_CAMERAS=all: every camera node of the glTF in one multi-view render, view i to <stem>_<i><ext>
         cameras = os.environ.get("RT_CAMERAS")
+        if frames is not None:
+            if cameras is not None or textscene.is_text_scene(argv[1]):
+                print("RT_FRAMES renders one camera of an animated glTF scene: it cannot be combined with RT_CAMERAS or a "
+                      "text scene", file=sys.stderr)
+                return 1
+            try:
+                count, fps = parse_frames(frames)
+                animation = int(os.environ.get("RT_ANIMATION", "0"))
+                gltf.animation_range(argv[1], animation)
+            except ValueError as e:  # also gltf.AnimationError: no animations, or no such animation
+                print(f"RT_FRAMES: {e}", file=sys.stderr)
+                return 1
+            return run_frames(argv[1], width, height, samples, count, fps, argv[5], animation=animation,
+                              seed=int(os.environ.get("RT_SEED", "0")), n_gpus=int(os.environ.get("RT_GPUS", "1")),
+                              rel_error=rel_error, projection=projection, env_map=os.environ.get("RT_ENV_MAP") or None)
+        # RT_CAMERAS=all: every camera node of the glTF in one multi-view render, view i to <stem>_<i><ext>
         if cameras is not None:
             if cameras != "all":
                 print(f"RT_CAMERAS={cameras}: the only value is 'all'", file=sys.stderr)

@@ -884,6 +884,137 @@ __global__ void __launch_bounds__(128) kb_emit(Arrays A, uint32_t n_slots) {
     A.qnodes4[flags_before(A, s)] = q;
 }
 
+// ---- refit (rt_gpu_update_geometry) ------------------------------------------------------------------------------------
+// The tree keeps its topology: the binary slots, the triangle order idx[parity], the leaf ends `last` and the 4-wide
+// grouping.  Only boxes change.  State recorded at the first update after an upload, from the pristine tree:
+//   kr_levels_init / kr_levels   the used binary slots, level by level from the root (unused slots hold undefined data)
+//   kr_wide_slots                for each 4-wide node, the binary slot behind each child (open_wide picks children by
+//                                box area, so collapsing the refit boxes again could regroup)
+// Every update then runs kr_refit once per binary level from the deepest up, kr_requant over the 4-wide nodes, and kb_tris.
+// Boxes reduce with fminf / fmaxf, as kb_setup, kb_split and kb_small do, so refitting to the uploaded positions
+// reproduces the uploaded tree bit for bit.
+constexpr uint32_t kMaxLevels = RT_STACK_SIZE + 2;
+
+struct Refit {
+    uint32_t *order;   // [n_slots] used binary slots, level by level
+    uint32_t *lstart;  // [kMaxLevels] first entry of each level in `order`
+    uint32_t *lcount;  // [kMaxLevels] entries of each level
+    int32_t *wslot;    // [4 * n_wide] binary slot behind child i of 4-wide node w; -1: absent child
+};
+
+__global__ void kr_levels_init(Refit R) {
+    R.lstart[0] = 0;
+    R.lcount[0] = 1;
+    R.order[0] = 0;
+}
+
+// level l lists its inner nodes' children as level l + 1 (appended right behind level l)
+__global__ void __launch_bounds__(256) kr_levels(Arrays A, Refit R, uint32_t l) {
+    const uint32_t begin = R.lstart[l], cnt = R.lcount[l], next = begin + cnt;
+    if (blockIdx.x == 0 && threadIdx.x == 0) R.lstart[l + 1] = next;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < cnt; k += gridDim.x * blockDim.x) {
+        const rt_bvh_node &nd = A.nodes[R.order[begin + k]];
+        if (nd.left_child == RT_NO_CHILD) continue;
+        const uint32_t at = next + atomicAdd(&R.lcount[l + 1], 2u);
+        R.order[at] = nd.left_child;
+        R.order[at + 1] = nd.right_child;
+    }
+}
+
+// open_wide, keeping the binary slot of every child; the links it implies are checked against kb_emit's (error bit 1)
+__global__ void __launch_bounds__(128) kr_wide_slots(Arrays A, Refit R, uint32_t n_slots) {
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n_slots || !A.mark[s]) return;
+    const rt_bvh_node *nodes = A.nodes;
+    uint32_t slot[4] = {nodes[s].left_child, nodes[s].right_child, 0, 0};
+    int n = 2;
+    auto inner = [&](uint32_t i) { return nodes[i].left_child != RT_NO_CHILD || nodes[i].right_child != RT_NO_CHILD; };
+    while (n < 4) {
+        int best = -1;
+        float best_area = -1.0f;
+        for (int i = 0; i < n; ++i)
+            if (inner(slot[i])) {
+                const float a = child_area(child_of(nodes, slot[i]));
+                if (a > best_area) {
+                    best_area = a;
+                    best = i;
+                }
+            }
+        if (best < 0) break;
+        const uint32_t b = slot[best];
+        slot[best] = nodes[b].left_child;
+        slot[n++] = nodes[b].right_child;
+    }
+    const uint32_t w = flags_before(A, s);
+    const QNode4 &q = A.qnodes4[w];
+    bool same = true;
+    for (int i = 0; i < 4; ++i) {
+        int32_t link = ~static_cast<int32_t>(A.n);
+        if (i < n) link = inner(slot[i]) ? static_cast<int32_t>(flags_before(A, slot[i])) : ~static_cast<int32_t>(nodes[slot[i]].obj_begin);
+        same = same && link == q.link[i];
+        R.wslot[4 * w + i] = i < n ? static_cast<int32_t>(slot[i]) : -1;
+    }
+    if (!same) atomicOr(&A.c->error, 2u);
+}
+
+// the binary nodes of one level: a leaf becomes the union of its triangles' boxes (kb_setup's), an inner node the union
+// of its children's.  Non-finite vertices set error bit 0, as in kb_setup.
+__global__ void __launch_bounds__(256) kr_refit(Arrays A, Refit R, uint32_t begin, uint32_t cnt, int parity) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= cnt) return;
+    rt_bvh_node &nd = A.nodes[R.order[begin + k]];
+    float lo[3] = {HUGE_VALF, HUGE_VALF, HUGE_VALF}, hi[3] = {-HUGE_VALF, -HUGE_VALF, -HUGE_VALF};
+    if (nd.left_child == RT_NO_CHILD) {
+        bool finite = true;
+        for (uint32_t p = nd.obj_begin; p < nd.obj_end; ++p) {
+            const float *v = A.tri_pos + static_cast<size_t>(A.idx[parity][p]) * 9;
+            for (int d = 0; d < 3; ++d) {
+                const float a = v[d], b = v[3 + d], c = v[6 + d];
+                lo[d] = fminf(lo[d], fminf(a, fminf(b, c)));
+                hi[d] = fmaxf(hi[d], fmaxf(a, fmaxf(b, c)));
+                finite = finite && rt::detail::finite_f(a) && rt::detail::finite_f(b) && rt::detail::finite_f(c);
+            }
+        }
+        if (!finite) atomicOr(&A.c->error, 1u);
+    } else {
+        const rt_bvh_node &l = A.nodes[nd.left_child], &r = A.nodes[nd.right_child];
+        for (int d = 0; d < 3; ++d) {
+            lo[d] = fminf(l.bmin[d], r.bmin[d]);
+            hi[d] = fmaxf(l.bmax[d], r.bmax[d]);
+        }
+    }
+    for (int d = 0; d < 3; ++d) {
+        nd.bmin[d] = lo[d];
+        nd.bmax[d] = hi[d];
+    }
+}
+
+// kb_emit's quantisation of every 4-wide node from the refit binary boxes of its recorded children; links are kept
+__global__ void __launch_bounds__(128) kr_requant(Arrays A, Refit R, uint32_t n_wide) {
+    const uint32_t w = blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= n_wide) return;
+    QNode4 q;
+    memset(&q, 0, sizeof q);
+    int n = 0;
+    for (int i = 0; i < 4; ++i) {
+        q.link[i] = A.qnodes4[w].link[i];
+        n += R.wslot[4 * w + i] >= 0 ? 1 : 0;
+    }
+    for (int a = 0; a < 3; ++a) {
+        float lo[4], hi[4];
+        uint8_t ql[4] = {255, 255, 255, 255}, qh[4] = {0, 0, 0, 0};  // absent child: inverted box
+        for (int i = 0; i < n; ++i) {
+            const rt_bvh_node &c = A.nodes[R.wslot[4 * w + i]];
+            lo[i] = c.bmin[a];
+            hi[i] = c.bmax[a];
+        }
+        if (!rt::detail::quantize_axis_n(lo, hi, n, q.org[a], ql, qh)) atomicOr(&A.c->error, 1u);
+        q.lo[a] = static_cast<uint32_t>(ql[0]) | static_cast<uint32_t>(ql[1]) << 8 | static_cast<uint32_t>(ql[2]) << 16 | static_cast<uint32_t>(ql[3]) << 24;
+        q.hi[a] = static_cast<uint32_t>(qh[0]) | static_cast<uint32_t>(qh[1]) << 8 | static_cast<uint32_t>(qh[2]) << 16 | static_cast<uint32_t>(qh[3]) << 24;
+    }
+    A.qnodes4[w] = q;
+}
+
 }  // namespace rtb
 
 #endif  // RT_GPU_BUILD_CUH

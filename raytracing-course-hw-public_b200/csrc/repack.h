@@ -798,6 +798,35 @@ inline int pack_bvh(const rt_scene_desc &sc, const rt_bvh_desc &src, PackedBvh &
     return rc;
 }
 
+// The light side of a scene: out.light (the light BVH; the traversal of the all-hit light pdf uses a rebuilt tree when
+// `rebuild`), out.light_sample (the sampling list, in the host light BVH's object order) and out.light_extra (DLight
+// normals and areas).  Reads sc.tri_pos and sc.light_bvh only, so that rt_gpu_update_geometry can run it on new positions.
+inline int pack_lights(const rt_scene_desc &sc, PackedScene &out, bool rebuild, int formats) {
+    PackedBvh host_order;
+    if (int rc = pack_bvh(sc, sc.light_bvh, host_order, formats == RT_PACK_Q8 ? 0 : formats)) return rc;
+    out.light_sample = host_order.tris;
+    if (formats == RT_PACK_Q8 && !(rebuild && sc.light_bvh.n_objects > 0 && sc.light_bvh.root != RT_NO_CHILD)) {
+        if (int rc = pack_bvh(sc, sc.light_bvh, out.light, formats)) return rc;
+    } else if (rebuild && sc.light_bvh.n_objects > 0 && sc.light_bvh.root != RT_NO_CHILD) {
+        BuiltBvh built;
+        build_sah_bvh(sc.tri_pos, sc.light_bvh.objects, sc.light_bvh.n_objects, built);
+        if (int rc = pack_bvh(sc, built.desc(), out.light, formats, true)) return rc;
+    } else {
+        out.light = host_order;
+    }
+    out.light_extra.resize(sc.light_bvh.n_objects);
+    for (uint32_t k = 0; k < sc.light_bvh.n_objects; ++k) {
+        const DTri &t = out.light.tris[k];
+        // crs(v, u), triangle::normal / square (geometry.h:477-483)
+        const float cx = t.e1y * t.e2z - t.e1z * t.e2y;
+        const float cy = t.e1z * t.e2x - t.e1x * t.e2z;
+        const float cz = t.e1x * t.e2y - t.e1y * t.e2x;
+        const float l = std::sqrt(cx * cx + cy * cy + cz * cz);
+        out.light_extra[k] = {cx / l, cy / l, cz / l, l / 2};
+    }
+    return RT_OK;
+}
+
 // `rebuild_scene_bvh`: build the scene BVH with the library's SAH builder (sah_build.h) over the triangles of
 // sc.scene_bvh instead of adopting the host's tree; the light BVH is always adopted as passed.
 // A host that passes NO scene BVH (scene_bvh.n_nodes == 0; rt_gpu.h) leaves the build to the library: the tree is built
@@ -821,21 +850,7 @@ inline int pack_scene(const rt_scene_desc &sc, PackedScene &out, bool rebuild_sc
     } else if (int rc = pack_bvh(sc, sc.scene_bvh, out.scene, formats)) {
         return rc;
     }
-    // light BVH: the traversal (all-hit light pdf) uses a rebuilt tree as well; the sampling list keeps the host's order
-    {
-        PackedBvh host_order;
-        if (int rc = pack_bvh(sc, sc.light_bvh, host_order, formats == RT_PACK_Q8 ? 0 : formats)) return rc;
-        out.light_sample = host_order.tris;
-        if (formats == RT_PACK_Q8 && !(rebuild_scene_bvh && sc.light_bvh.n_objects > 0 && sc.light_bvh.root != RT_NO_CHILD)) {
-            if (int rc = pack_bvh(sc, sc.light_bvh, out.light, formats)) return rc;
-        } else if (rebuild_scene_bvh && sc.light_bvh.n_objects > 0 && sc.light_bvh.root != RT_NO_CHILD) {
-            BuiltBvh built;
-            build_sah_bvh(sc.tri_pos, sc.light_bvh.objects, sc.light_bvh.n_objects, built);
-            if (int rc = pack_bvh(sc, built.desc(), out.light, formats, true)) return rc;
-        } else {
-            out.light = host_order;
-        }
-    }
+    if (int rc = pack_lights(sc, out, rebuild_scene_bvh, formats)) return rc;
 
     lap = PackLap();
     const uint32_t n = with_scene ? static_cast<uint32_t>(out.scene.order.size()) : 0u;  // device triangle order = packed BVH order
@@ -870,16 +885,6 @@ inline int pack_scene(const rt_scene_desc &sc, PackedScene &out, bool rebuild_sc
         }
     });
     lap.lap(5);
-    out.light_extra.resize(sc.light_bvh.n_objects);
-    for (uint32_t k = 0; k < sc.light_bvh.n_objects; ++k) {
-        const DTri &t = out.light.tris[k];
-        // crs(v, u), triangle::normal / square (geometry.h:477-483)
-        const float cx = t.e1y * t.e2z - t.e1z * t.e2y;
-        const float cy = t.e1z * t.e2x - t.e1x * t.e2z;
-        const float cz = t.e1x * t.e2y - t.e1y * t.e2x;
-        const float l = std::sqrt(cx * cx + cy * cy + cz * cz);
-        out.light_extra[k] = {cx / l, cy / l, cz / l, l / 2};
-    }
 
     out.materials.resize(sc.n_materials);
     for (uint32_t i = 0; i < sc.n_materials; ++i) {

@@ -147,6 +147,11 @@ struct DeviceState {
     rtb::Arrays built{};                  // device pointers of the last device build (diagnostics)
     uint32_t built_info[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // n_tris, n_slots, n_wide, root4, stack_need, max_depth, 1 = device build, levels
     int built_parity = 0;
+    // refit of that tree (rt_gpu_update_geometry): recorded at the first update after an upload
+    DevBuf<uint8_t> refit_scratch;
+    rtb::Refit refit{};
+    bool refit_ready = false;
+    std::vector<uint32_t> refit_lstart, refit_lcount;  // the binary levels of refit.order
     // course text scene (rt_gpu_upload_text_scene)
     DevBuf<rt_text_prim> tprims;
     DevBuf<rt_text_light> tlights;
@@ -347,6 +352,7 @@ int device_build_scene(DeviceState &d, const rt_scene_desc &sc, double *t_h2d_ms
         t_last = now;
     };
     lap("h2d+alloc");
+    d.refit_ready = false;
     std::memset(d.built_info, 0, sizeof d.built_info);
     d.built = A;
     d.built_parity = 0;
@@ -430,22 +436,14 @@ int device_build_scene(DeviceState &d, const rt_scene_desc &sc, double *t_h2d_ms
     return RT_OK;
 }
 
-int upload_to_device(DeviceState &d, const rt_scene_desc &sc, const rt::PackedScene &p, bool device_built) {
-    CU_CHECK(cudaSetDevice(d.device));
+// The light side of a packed scene on device d (light nodes, light triangles, the sampling list, DLight records, the
+// light box) and the DScene fields that refer to it.  Shared by rt_gpu_upload_scene and rt_gpu_update_geometry.
+int upload_lights(DeviceState &d, const rt::PackedScene &p, uint32_t n_lights) {
 #if RT_EXT_WIDE8  // only the node format the traversal kernel was built for goes to the device
-    if (int rc = d.qnodes8.upload(p.scene.qnodes8, d.stream)) return rc;
     if (int rc = d.lqnodes8.upload(p.light.qnodes8, d.stream)) return rc;
 #else
-    if (!device_built)
-        if (int rc = d.qnodes4.upload(p.scene.qnodes4, d.stream)) return rc;
     if (int rc = d.lqnodes4.upload(p.light.qnodes4, d.stream)) return rc;
 #endif
-    if (!device_built) {
-        if (int rc = d.tris.upload(p.scene.tris, d.stream)) return rc;
-        if (int rc = d.attrs.upload(p.attrs, d.stream)) return rc;
-        if (int rc = d.tangents.upload(p.tangents, d.stream)) return rc;
-        std::memset(d.built_info, 0, sizeof d.built_info);
-    }
     {   // box of all light triangles, widened by 1e-4 of its size and of the coordinates' magnitude: a ray that misses
         // it has no light-pdf term (k_lightpdf); the last entry of light.tris is the null triangle
         float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
@@ -468,37 +466,172 @@ int upload_to_device(DeviceState &d, const rt_scene_desc &sc, const rt::PackedSc
     if (int rc = d.ltris.upload(p.light.tris, d.stream)) return rc;
     if (int rc = d.lsample.upload(p.light_sample, d.stream)) return rc;
     if (int rc = d.light_extra.upload(p.light_extra, d.stream)) return rc;
+    d.scene.light.root4 = p.light.root4;
+    d.scene.light.n_nodes8 = static_cast<uint32_t>(p.light.qnodes8.size());
+    d.scene.light.root = p.light.root;
+    d.scene.light.n_tris = static_cast<uint32_t>(p.light.tris.size());
+    d.scene.n_lights = n_lights;
+    d.scene.light.qnodes4 = d.lqnodes4.p;
+    d.scene.light.qnodes8 = d.lqnodes8.p;
+    d.scene.light.nodes = nullptr;
+    d.scene.light.qnodes = nullptr;
+    d.scene.light.tris = d.ltris.p;
+    d.scene.light_sample = d.lsample.p;
+    d.scene.light_extra = d.light_extra.p;
+    return RT_OK;
+}
+
+// The node halves k_extend reads: [scene lo | light lo | scene hi | light hi], 32 bytes per node and half.  Its layout
+// depends on both node counts, so an update of the light BVH makes it again.
+int split_nodes(DeviceState &d, size_t n_scene, size_t n_light) {
+#if !RT_EXT_WIDE8
+    const size_t n_all = std::max<size_t>(n_scene + n_light, 1);
+    if (int rc = d.q4split.alloc(n_all * 4)) return rc;
+    char *lo = reinterpret_cast<char *>(d.q4split.p), *hi = lo + n_all * 32;
+    if (n_scene) rt::k_split_nodes<<<static_cast<uint32_t>((n_scene * 4 + 255) / 256), 256, 0, d.stream>>>(d.qnodes4.p, static_cast<uint32_t>(n_scene), lo, hi);
+    if (n_light) rt::k_split_nodes<<<static_cast<uint32_t>((n_light * 4 + 255) / 256), 256, 0, d.stream>>>(d.lqnodes4.p, static_cast<uint32_t>(n_light), lo + n_scene * 32, hi + n_scene * 32);
+    CU_CHECK(cudaGetLastError());
+    d.scene.scene.q4lo = lo;
+    d.scene.light.q4lo = lo + n_scene * 32;
+    d.scene.scene.q4_hi_off = d.scene.light.q4_hi_off = static_cast<uint32_t>(n_all * 32);
+#else
+    (void)d, (void)n_scene, (void)n_light;
+#endif
+    return RT_OK;
+}
+
+// rt_gpu_update_geometry on one device: the new positions, normals and tangents go into the build's input copies, the
+// binary boxes are refit from the leaves up, the 4-wide nodes re-quantised and DTri / DAttr (/ DTangent) rewritten.  The
+// topology stays the upload's (gpu_build.cuh, "refit").  `phases`: RT_TIMING's serialised phase times.
+int device_refit_scene(DeviceState &d, const rt_geometry_update &u, std::string &phases) {
+    using namespace rtb;
+    CU_CHECK(cudaSetDevice(d.device));
+    const uint32_t n = d.built_info[0], n_slots = d.built_info[1], n_wide = d.built_info[2], depth = d.built_info[5];
+    const int parity = d.built_parity;
+    cudaStream_t st = d.stream;
+    Arrays A = d.built;
+    Counters &hc = *d.h_counters;
+    auto fetch_counters = [&]() -> int {
+        CU_CHECK(cudaMemcpyAsync(&hc, A.c, sizeof(Counters), cudaMemcpyDeviceToHost, st));
+        CU_CHECK(cudaStreamSynchronize(st));
+        return RT_OK;
+    };
+    const bool timing = std::getenv("RT_TIMING") != nullptr;
+    auto t_last = std::chrono::steady_clock::now();
+    auto lap = [&](const char *name) {
+        if (!timing) return;
+        cudaStreamSynchronize(st);
+        const auto now = std::chrono::steady_clock::now();
+        char buf[64];
+        std::snprintf(buf, sizeof buf, " %s %.3f", name, std::chrono::duration<double, std::milli>(now - t_last).count());
+        phases += buf;
+        t_last = now;
+    };
+    if (n == 0) return RT_OK;  // only the null triangle
+    if (!d.refit_ready) {  // from the pristine tree, before any box changes
+        size_t off = 0;
+        auto carve = [&](size_t bytes) {
+            const size_t at = off;
+            off += (bytes + 255) / 256 * 256;
+            return at;
+        };
+        const size_t o_order = carve(static_cast<size_t>(n_slots) * 4), o_lstart = carve(kMaxLevels * 4), o_lcount = carve(kMaxLevels * 4);
+        const size_t o_wslot = carve(std::max<size_t>(n_wide, 1) * 16);
+        if (int rc = d.refit_scratch.alloc(off)) return rc;
+        uint8_t *base = d.refit_scratch.p;
+        Refit &R = d.refit;
+        R.order = reinterpret_cast<uint32_t *>(base + o_order);
+        R.lstart = reinterpret_cast<uint32_t *>(base + o_lstart);
+        R.lcount = reinterpret_cast<uint32_t *>(base + o_lcount);
+        R.wslot = reinterpret_cast<int32_t *>(base + o_wslot);
+        CU_CHECK(cudaMemsetAsync(R.lcount, 0, kMaxLevels * 4, st));
+        kr_levels_init<<<1, 1, 0, st>>>(R);
+        const uint32_t g = std::min<uint32_t>((n + 255) / 256, 1024);
+        for (uint32_t l = 0; l < depth; ++l) kr_levels<<<g, 256, 0, st>>>(A, R, l);
+        if (n_wide) kr_wide_slots<<<(n_slots + 127) / 128, 128, 0, st>>>(A, R, n_slots);
+        CU_CHECK(cudaGetLastError());
+        d.refit_lstart.resize(depth + 1);
+        d.refit_lcount.resize(depth + 1);
+        CU_CHECK(cudaMemcpyAsync(d.refit_lstart.data(), R.lstart, (depth + 1) * 4, cudaMemcpyDeviceToHost, st));
+        CU_CHECK(cudaMemcpyAsync(d.refit_lcount.data(), R.lcount, (depth + 1) * 4, cudaMemcpyDeviceToHost, st));
+        if (int rc = fetch_counters()) return rc;
+        if (hc.error) return fail(RT_ERR_CUDA, "rt_gpu_update_geometry: the recorded 4-wide grouping does not reproduce the uploaded links");
+        d.refit_ready = true;
+        lap("record");
+    }
+    CU_CHECK(cudaMemcpyAsync(d.in_pos.p, u.tri_pos, static_cast<size_t>(n) * 36, cudaMemcpyHostToDevice, st));
+    CU_CHECK(cudaMemcpyAsync(d.in_nrm.p, u.tri_normals, static_cast<size_t>(n) * 36, cudaMemcpyHostToDevice, st));
+    if (u.tri_tangents) {
+        if (int rc = d.in_tan.alloc(static_cast<size_t>(n) * 9)) return rc;
+        CU_CHECK(cudaMemcpyAsync(d.in_tan.p, u.tri_tangents, static_cast<size_t>(n) * 36, cudaMemcpyHostToDevice, st));
+    }
+    A.tri_tangents = u.tri_tangents ? d.in_tan.p : nullptr;
+    lap("h2d");
+    CU_CHECK(cudaMemsetAsync(&A.c->error, 0, 2 * sizeof(uint32_t), st));  // error, any_tangent
+    if (A.tri_tangents) kb_tangent_flag<<<(n + 255) / 256, 256, 0, st>>>(A);
+    for (uint32_t l = depth + 1; l-- > 0;)  // every level up to `depth` holds nodes
+        kr_refit<<<(d.refit_lcount[l] + 255) / 256, 256, 0, st>>>(A, d.refit, d.refit_lstart[l], d.refit_lcount[l], parity);
+    lap("refit");
+    if (n_wide) kr_requant<<<(n_wide + 127) / 128, 128, 0, st>>>(A, d.refit, n_wide);
+    CU_CHECK(cudaGetLastError());
+    if (int rc = fetch_counters()) return rc;
+    lap("quantise");
+    if (hc.error) return fail(RT_ERR_BAD_SCENE, "rt_gpu_update_geometry: non-finite triangle or a node that cannot be quantised; the scene is gone");
+    const bool with_tangents = A.tri_tangents && hc.any_tangent;
+    A.tangents = nullptr;
+    if (with_tangents) {
+        if (int rc = d.tangents.alloc(n)) return rc;
+        A.tangents = d.tangents.p;
+    }
+    kb_tris<<<(n + 1 + 255) / 256, 256, 0, st>>>(A, parity, with_tangents ? 1 : 0);
+    CU_CHECK(cudaGetLastError());
+    d.built = A;
+    d.scene.tangents = A.tangents;
+    lap("tris");
+    return RT_OK;
+}
+
+// Structural check of a host BVH before anything is dereferenced through it; null when it is well formed
+const char *bvh_problem(const rt_bvh_desc &b, uint32_t n_tris) {
+    if (b.root != RT_NO_CHILD && b.root >= b.n_nodes) return "BVH root out of range";
+    for (uint32_t i = 0; i < b.n_objects; ++i)
+        if (b.objects[i] >= n_tris) return "BVH object id out of range";
+    for (uint32_t i = 0; i < b.n_nodes; ++i) {
+        const rt_bvh_node &nd = b.nodes[i];
+        if ((nd.left_child != RT_NO_CHILD && nd.left_child >= b.n_nodes) || (nd.right_child != RT_NO_CHILD && nd.right_child >= b.n_nodes) ||
+            nd.obj_begin > nd.obj_end || nd.obj_end > b.n_objects)
+            return "BVH node links out of range";
+    }
+    return nullptr;
+}
+
+int upload_to_device(DeviceState &d, const rt_scene_desc &sc, const rt::PackedScene &p, bool device_built) {
+    CU_CHECK(cudaSetDevice(d.device));
+#if RT_EXT_WIDE8  // only the node format the traversal kernel was built for goes to the device
+    if (int rc = d.qnodes8.upload(p.scene.qnodes8, d.stream)) return rc;
+#else
+    if (!device_built)
+        if (int rc = d.qnodes4.upload(p.scene.qnodes4, d.stream)) return rc;
+#endif
+    if (!device_built) {
+        if (int rc = d.tris.upload(p.scene.tris, d.stream)) return rc;
+        if (int rc = d.attrs.upload(p.attrs, d.stream)) return rc;
+        if (int rc = d.tangents.upload(p.tangents, d.stream)) return rc;
+        std::memset(d.built_info, 0, sizeof d.built_info);
+    }
     if (int rc = d.materials.upload(p.materials, d.stream)) return rc;
     if (int rc = d.textures.upload(p.textures, d.stream)) return rc;
     if (int rc = d.texels.upload(p.texels, d.stream)) return rc;
     std::vector<float> lut(p.gamma_lut, p.gamma_lut + 256);
     if (int rc = d.lut.upload(lut, d.stream)) return rc;
     rt::fill_scene_constants(sc, p, d.scene);
+    if (int rc = upload_lights(d, p, sc.light_bvh.n_objects)) return rc;
     d.scene.scene.nodes = nullptr;  // the device traverses the quantised copies only
     d.scene.scene.qnodes = nullptr;  // the 2-wide form exists on the host only (tests)
     d.scene.scene.qnodes4 = d.qnodes4.p;
-    d.scene.light.qnodes4 = d.lqnodes4.p;
     d.scene.scene.qnodes8 = d.qnodes8.p;
-    d.scene.light.qnodes8 = d.lqnodes8.p;
-#if !RT_EXT_WIDE8
-    {   // the node halves k_extend reads: [scene lo | light lo | scene hi | light hi], 32 bytes per node and half
-        const size_t n_scene = device_built ? d.built_info[2] : p.scene.qnodes4.size(), n_light = p.light.qnodes4.size();
-        const size_t n_all = std::max<size_t>(n_scene + n_light, 1);
-        if (int rc = d.q4split.alloc(n_all * 4)) return rc;
-        char *lo = reinterpret_cast<char *>(d.q4split.p), *hi = lo + n_all * 32;
-        if (n_scene) rt::k_split_nodes<<<static_cast<uint32_t>((n_scene * 4 + 255) / 256), 256, 0, d.stream>>>(d.qnodes4.p, static_cast<uint32_t>(n_scene), lo, hi);
-        if (n_light) rt::k_split_nodes<<<static_cast<uint32_t>((n_light * 4 + 255) / 256), 256, 0, d.stream>>>(d.lqnodes4.p, static_cast<uint32_t>(n_light), lo + n_scene * 32, hi + n_scene * 32);
-        CU_CHECK(cudaGetLastError());
-        d.scene.scene.q4lo = lo;
-        d.scene.light.q4lo = lo + n_scene * 32;
-        d.scene.scene.q4_hi_off = d.scene.light.q4_hi_off = static_cast<uint32_t>(n_all * 32);
-    }
-#endif
+    if (int rc = split_nodes(d, device_built ? d.built_info[2] : p.scene.qnodes4.size(), p.light.qnodes4.size())) return rc;
     d.scene.scene.tris = d.tris.p;
-    d.scene.light.nodes = nullptr;
-    d.scene.light.qnodes = nullptr;
-    d.scene.light.tris = d.ltris.p;
-    d.scene.light_sample = d.lsample.p;
     d.scene.attrs = d.attrs.p;
     d.scene.tangents = p.tangents.empty() ? nullptr : d.tangents.p;
     if (device_built) {
@@ -506,7 +639,6 @@ int upload_to_device(DeviceState &d, const rt_scene_desc &sc, const rt::PackedSc
         d.scene.scene.n_tris = d.built_info[0] + 1;
         d.scene.tangents = d.built.tangents;
     }
-    d.scene.light_extra = d.light_extra.p;
     d.scene.materials = d.materials.p;
     d.scene.textures = d.textures.p;
     d.scene.texels = d.texels.p;
@@ -1102,7 +1234,7 @@ void rt_gpu_destroy(rt_gpu_ctx *ctx) {
         if (d.h_counters) cudaFreeHost(d.h_counters);
         if (d.h_active) cudaFreeHost(d.h_active);
         d.alist.release(); d.awords.release(); d.acounts.release(); d.actr.release(); d.aerr.release();
-        d.in_pos.release(); d.in_nrm.release(); d.in_uv.release(); d.in_tan.release(); d.in_mat.release(); d.build_scratch.release();
+        d.in_pos.release(); d.in_nrm.release(); d.in_uv.release(); d.in_tan.release(); d.in_mat.release(); d.build_scratch.release(); d.refit_scratch.release();
         d.counters.release(); d.stats.release();
         d.prim_ids.release(); d.rgb8.release(); d.cams.release();
         for (cudaEvent_t e : d.event_pool) cudaEventDestroy(e);
@@ -1132,18 +1264,8 @@ int rt_gpu_upload_scene(rt_gpu_ctx *ctx, const rt_scene_desc *scene) {
             return fail(RT_ERR_BAD_SCENE, "rt_gpu_upload_scene: null BVH array");
     for (uint32_t i = 0; i < scene->n_tris; ++i)
         if (scene->tri_material[i] >= scene->n_materials) return fail(RT_ERR_BAD_SCENE, "material id out of range");
-    for (const rt_bvh_desc *b : {&scene->scene_bvh, &scene->light_bvh}) {
-        if (b->root != RT_NO_CHILD && b->root >= b->n_nodes) return fail(RT_ERR_BAD_SCENE, "BVH root out of range");
-        for (uint32_t i = 0; i < b->n_objects; ++i)
-            if (b->objects[i] >= scene->n_tris) return fail(RT_ERR_BAD_SCENE, "BVH object id out of range");
-        for (uint32_t i = 0; i < b->n_nodes; ++i) {
-            const rt_bvh_node &nd = b->nodes[i];
-            if ((nd.left_child != RT_NO_CHILD && nd.left_child >= b->n_nodes) ||
-                (nd.right_child != RT_NO_CHILD && nd.right_child >= b->n_nodes) || nd.obj_begin > nd.obj_end ||
-                nd.obj_end > b->n_objects)
-                return fail(RT_ERR_BAD_SCENE, "BVH node links out of range");
-        }
-    }
+    for (const rt_bvh_desc *b : {&scene->scene_bvh, &scene->light_bvh})
+        if (const char *why = bvh_problem(*b, scene->n_tris)) return fail(RT_ERR_BAD_SCENE, why);
     for (uint32_t i = 0; i < scene->n_materials; ++i) {
         const rt_material &m = scene->materials[i];
         for (int32_t t : {m.color_tex, m.emissive_tex, m.metallic_roughness_tex, m.normal_tex})
@@ -1197,6 +1319,55 @@ int rt_gpu_upload_scene(rt_gpu_ctx *ctx, const rt_scene_desc *scene) {
     ctx->have_render = false;
     ctx->adaptive = ctx->adaptive_sums = false;
     ctx->text_scene = false;
+    return RT_OK;
+}
+
+int rt_gpu_update_geometry(rt_gpu_ctx *ctx, const rt_geometry_update *u) {
+    if (!ctx || !u) return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_gpu_update_geometry: no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: a text scene has no triangle geometry to update");
+    const DeviceState &d0 = *ctx->devs[0];
+    if (d0.built_info[6] != 1)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: the scene BVH was not built on the device (RT_SCENE_KEEP_HOST_BVH, "
+                                        "RT_KEEP_HOST_BVH, RT_HOST_BUILD or the 8-wide library): re-upload the scene instead");
+    if (u->n_tris != d0.built_info[0]) return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: n_tris differs from the uploaded scene's");
+    if (u->n_tris > 0 && (!u->tri_pos || !u->tri_normals))
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: null tri_pos / tri_normals with n_tris > 0");
+    const rt_bvh_desc &lb = u->light_bvh;
+    if ((lb.n_nodes > 0 && !lb.nodes) || (lb.n_objects > 0 && !lb.objects)) return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: null BVH array");
+    if (lb.n_objects != d0.scene.n_lights)
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: the light BVH has another number of objects than the uploaded one");
+    if (const char *why = bvh_problem(lb, u->n_tris)) return fail(RT_ERR_INVALID_ARG, std::string("rt_gpu_update_geometry: ") + why);
+    // the light side, as rt_gpu_upload_scene packs it for a device-built scene (rt::pack_scene with !keep)
+    rt_scene_desc sc{};
+    sc.abi_version = RT_GPU_ABI_VERSION;
+    sc.n_tris = u->n_tris;
+    sc.tri_pos = u->tri_pos;
+    sc.light_bvh = lb;
+    rt::PackedScene &packed = ctx->packed;
+    if (rt::pack_lights(sc, packed, true, rt::RT_PACK_Q4))
+        return fail(RT_ERR_INVALID_ARG, "rt_gpu_update_geometry: the light BVH cannot be re-packed (inner node with objects, depth > 64, "
+                                        "or a traversal that needs more than RT_EXT_STACK_CAP stack entries)");
+    // from here on the device arrays change: a failure leaves no scene
+    for (auto &dp : ctx->devs) {
+        DeviceState &d = *dp;
+        std::string phases;
+        const auto t0 = std::chrono::steady_clock::now();
+        int rc = device_refit_scene(d, *u, phases);
+        if (rc == RT_OK) rc = upload_lights(d, packed, lb.n_objects);
+        if (rc == RT_OK) rc = split_nodes(d, d.built_info[2], packed.light.qnodes4.size());
+        if (rc == RT_OK) {
+            const cudaError_t e = cudaStreamSynchronize(d.stream);
+            if (e != cudaSuccess) rc = fail(RT_ERR_CUDA, std::string("rt_gpu_update_geometry: ") + cudaGetErrorString(e));
+        }
+        if (rc != RT_OK) {
+            ctx->have_scene = false;
+            return rc;
+        }
+        if (std::getenv("RT_TIMING"))
+            std::fprintf(stderr, "rt_gpu_update_geometry: device %d %.3f ms (phases, serialised:%s)\n", d.device,
+                         std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(), phases.c_str());
+    }
     return RT_OK;
 }
 

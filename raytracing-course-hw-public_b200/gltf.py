@@ -135,15 +135,11 @@ LIGHT_TRIANGLE_INTENSITY = 10.0
 LIGHT_TRIANGLE_RELATIVE_POS = ((10.0, 0.0, -0.1), (0.0, 10.0, -0.1), (0.0, -10.0, -0.1))
 
 
-def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triangle=None):
-    """parse_gltf_scene(path, ar) + RaytracerStaticContext (both BVH builds) -> SceneData.
+class AnimationError(ValueError):
+    """An animation the loader cannot sample (see load_gltf's `time`)."""
 
-    `aspect_ratio` is width/height as the CLI passes it (src/main.cpp:27).  `env_map`: image file used as the
-    equirectangular environment map `Scene::bg` (what main.cpp:29-31 loads when USE_ENV_MAP is compiled in; None =
-    HEAD's constant white sky)."""
-    with open(path) as f:
-        doc = json.load(f)
-    base = os.path.dirname(os.path.abspath(path))
+
+def _read_buffers(doc, base):
     buffers = []
     for b in doc.get("buffers", []):
         raw = np.zeros(int(b["byteLength"]), np.uint8)
@@ -151,9 +147,139 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
             data = np.frombuffer(f.read(int(b["byteLength"])), np.uint8)
         raw[:data.size] = data
         buffers.append(raw)
+    return buffers
 
-    tex_images = [_load_texture(os.path.join(base, doc["images"][int(t["source"])]["uri"]))
-                  for t in doc.get("textures", [])]
+
+_COMPS = {"SCALAR": 1, "VEC2": 2, "VEC3": 3, "VEC4": 4}
+
+
+def _float_accessor(doc, buffers, idx):
+    """A float accessor as the glTF specification lays it out (bufferView and accessor byteOffset, byteStride):
+    [count, components] float32.  Animation data only; vertex attributes keep the reference's reading."""
+    acc = doc["accessors"][idx]
+    if int(acc["componentType"]) != 5126:
+        raise AnimationError(f"accessor {idx}: animation data must be float (componentType 5126)")
+    view = doc["bufferViews"][int(acc["bufferView"])]
+    comps, count = _COMPS[acc["type"]], int(acc["count"])
+    stride = int(view.get("byteStride", 4 * comps))
+    off = int(view.get("byteOffset", 0)) + int(acc.get("byteOffset", 0))
+    buf = buffers[int(view["buffer"])]
+    out = np.empty((count, comps), F)
+    for k in range(count):
+        out[k] = buf[off + k * stride:off + k * stride + 4 * comps].view(F)
+    return out
+
+
+def _animation(doc, animation):
+    anims = doc.get("animations") or []
+    if not anims:
+        raise AnimationError("the file has no animations")
+    if not 0 <= animation < len(anims):
+        raise AnimationError(f"animation {animation} out of range: the file has {len(anims)}")
+    return anims[animation]
+
+
+class GltfFile:
+    """A glTF file read once: its JSON, buffers and texture images (images are decoded on first use and kept), so that
+    many frames of an animation can be flattened from one read (load_gltf and animation_range take one for a path)."""
+
+    def __init__(self, path):
+        self.path = path
+        with open(path) as f:
+            self.doc = json.load(f)
+        self.base = os.path.dirname(os.path.abspath(path))
+        self.buffers = _read_buffers(self.doc, self.base)
+        self._images = {}
+
+    def image(self, path):
+        if path not in self._images:
+            self._images[path] = _load_texture(path)
+        return self._images[path]
+
+    def textures(self):
+        return [self.image(os.path.join(self.base, self.doc["images"][int(t["source"])]["uri"])) for t in self.doc.get("textures", [])]
+
+
+def _opened(path):
+    return path if isinstance(path, GltfFile) else GltfFile(path)
+
+
+def animation_range(path, animation=0):
+    """[t0, t1]: the first and the last key time of animation `animation` of a glTF file (a path or a GltfFile), in
+    seconds.  Raises AnimationError when the file has no such animation."""
+    src = _opened(path)
+    anim = _animation(src.doc, animation)
+    times = [_float_accessor(src.doc, src.buffers, int(s["input"])).reshape(-1) for s in anim["samplers"]]
+    return float(min(t.min() for t in times)), float(max(t.max() for t in times))
+
+
+def _slerp(q0, q1, u):
+    """Shortest-arc spherical interpolation of unit quaternions (x, y, z, w) in float64, normalised."""
+    d = float(np.dot(q0, q1))
+    if d < 0:
+        q1, d = -q1, -d
+    if d > 1.0 - 1e-9:
+        q = q0 + u * (q1 - q0)
+    else:
+        th = np.arccos(min(d, 1.0))
+        q = (np.sin((1 - u) * th) * q0 + np.sin(u * th) * q1) / np.sin(th)
+    return q / np.linalg.norm(q)
+
+
+def sample_channel(times, values, interpolation, path, t):
+    """The value of one animation sampler at time t (float32): times clamp at both ends, a key's own time returns the
+    stored key value itself, and between keys LINEAR interpolates (slerp for rotations) and STEP holds the earlier key."""
+    times = np.asarray(times, F).reshape(-1)
+    if interpolation not in ("LINEAR", "STEP"):
+        raise AnimationError(f"{interpolation} interpolation is not supported")
+    t = float(t)
+    if t <= float(times[0]):
+        return values[0].copy()
+    if t >= float(times[-1]):
+        return values[-1].copy()
+    k = int(np.searchsorted(times.astype(np.float64), t, side="right")) - 1  # times[k] <= t < times[k + 1]
+    if float(times[k]) == t or interpolation == "STEP":
+        return values[k].copy()
+    u = (t - float(times[k])) / (float(times[k + 1]) - float(times[k]))
+    a, b = values[k].astype(np.float64), values[k + 1].astype(np.float64)
+    return (_slerp(a, b, u) if path == "rotation" else a + u * (b - a)).astype(F)
+
+
+def _animated_trs(doc, buffers, animation, time):
+    """{node: {"translation" | "rotation" | "scale": float32 value}} of animation `animation` at `time`."""
+    anim = _animation(doc, animation)
+    if doc.get("skins") or any("skin" in n for n in doc.get("nodes", [])):
+        raise AnimationError("skinned meshes are not supported")
+    out = {}
+    for ch in anim["channels"]:
+        path, node = ch["target"]["path"], ch["target"].get("node")
+        smp = anim["samplers"][int(ch["sampler"])]
+        interpolation = smp.get("interpolation", "LINEAR")
+        if path == "weights":
+            raise AnimationError("morph-target weights are not supported")
+        if interpolation == "CUBICSPLINE":
+            raise AnimationError("CUBICSPLINE interpolation is not supported")
+        if node is None or path not in ("translation", "rotation", "scale"):
+            continue
+        times = _float_accessor(doc, buffers, int(smp["input"]))
+        values = _float_accessor(doc, buffers, int(smp["output"]))
+        out.setdefault(int(node), {})[path] = sample_channel(times, values, interpolation, path, time)
+    return out
+
+
+def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triangle=None, time=None, animation=0):
+    """parse_gltf_scene(path, ar) + RaytracerStaticContext (both BVH builds) -> SceneData.
+
+    `aspect_ratio` is width/height as the CLI passes it (src/main.cpp:27).  `env_map`: image file used as the
+    equirectangular environment map `Scene::bg` (what main.cpp:29-31 loads when USE_ENV_MAP is compiled in; None =
+    HEAD's constant white sky).  `path` may be a GltfFile (read once, flattened many times).  `time` (seconds): the scene at that time of animation `animation`; its translation,
+    rotation and scale channels replace the targeted nodes' TRS before the node transform is composed (LINEAR and
+    STEP samplers; CUBICSPLINE, morph-target weights and skins raise AnimationError).  time=None ignores animations."""
+    src = _opened(path)
+    doc, buffers = src.doc, src.buffers
+    animated = {} if time is None else _animated_trs(doc, buffers, animation, time)
+
+    tex_images = src.textures()
 
     def accessor_raw(idx, dtype, comps):
         """interpret_accessor, scene.h:118-133: bufferView byteOffset only, tightly packed."""
@@ -221,6 +347,8 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
 
     def handle_node(node_idx, parent):
         node = doc["nodes"][node_idx]
+        if node_idx in animated:
+            node = {**node, **animated[node_idx]}
         rotation = node.get("rotation", [0, 0, 0, 1])
         translation = np.array(node.get("translation", [0, 0, 0]), F)
         scale = np.array(node.get("scale", [1, 1, 1]), F)
@@ -354,7 +482,7 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
         s.tri_material = cat(s.tri_material, np.array([mat_index[key]], np.uint32))
     s.materials = np.array(materials, MATERIAL_DTYPE) if materials else np.zeros(0, MATERIAL_DTYPE)
     if env_map is not None:
-        env = _load_texture(env_map)
+        env = src.image(env_map)
         if env.shape[0] * env.shape[1] > 1 or not (env[0, 0, :3] == 255).all():  # 1x1 white = HEAD's constant sky
             tex_images = tex_images + [env]
             s.env_texture = len(tex_images)
@@ -374,6 +502,11 @@ def load_gltf(path, aspect_ratio, build_bvh=True, env_map=None, add_light_triang
 def build_bvhs(s):
     """RaytracerStaticContext, raytracer.h:440-447: BVH over all objects + BVH over emission != 0."""
     s.scene_bvh = host.build_bvh(s.tri_pos)
+    return build_light_bvh(s)
+
+
+def build_light_bvh(s):
+    """The BVH over emission != 0 alone (raytracer.h:444-447): what an update of moved geometry passes."""
     if s.n_tris:
         em = s.materials["emission"][s.tri_material]
         s.light_bvh = host.build_bvh(s.tri_pos, select=(em != 0).any(axis=1))

@@ -6,8 +6,8 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_camera, rt_projection,
-                   rt_render_params, rt_scene_desc, rt_stats, rt_views)
+from ._abi import (RT_FLAG_ACCUMULATE, RT_MODE_BEAUTY, RT_MODE_PRIMARY_IDS, rt_adaptive_params, rt_camera, rt_geometry_update,
+                   rt_projection, rt_render_params, rt_scene_desc, rt_stats, rt_views)
 
 # RT_GPU_LIB selects another build of the same C ABI (kernel A/B experiments, tools/build_variants.sh)
 LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu.so")
@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu
 SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upload_text_scene", "rt_gpu_render", "rt_gpu_readback",
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
            "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive",
-           "rt_gpu_render_views", "rt_gpu_render_views_adaptive", "rt_gpu_render_projected"]
+           "rt_gpu_render_views", "rt_gpu_render_views_adaptive", "rt_gpu_render_projected", "rt_gpu_update_geometry"]
 
 _lib = None
 
@@ -30,6 +30,7 @@ def lib():
         L.rt_gpu_destroy.restype = None
         L.rt_gpu_upload_scene.argtypes = [C.c_void_p, C.POINTER(rt_scene_desc)]
         L.rt_gpu_upload_text_scene.argtypes = [C.c_void_p, C.c_void_p]
+        L.rt_gpu_update_geometry.argtypes = [C.c_void_p, C.POINTER(rt_geometry_update)]
         L.rt_gpu_render.argtypes = [C.c_void_p, C.POINTER(rt_render_params)]
         L.rt_gpu_readback.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_gpu_render_adaptive.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params)]
@@ -95,6 +96,13 @@ class RtGpu:
         d = scene.desc()
         _check(lib().rt_gpu_upload_scene(self._h, C.byref(d)), "rt_gpu_upload_scene")
         self._scene = scene
+
+    def update_geometry(self, scene):
+        """Move the uploaded scene's triangles (rt_gpu_update_geometry): `scene` is a SceneData of the same triangles at
+        new positions; its positions, normals, tangents and light_bvh are passed (build the light BVH over the new
+        positions with host.build_bvh(tri_pos, select=emissive)).  The library refits its own scene BVH."""
+        u = scene.geometry_update()
+        _check(lib().rt_gpu_update_geometry(self._h, C.byref(u)), "rt_gpu_update_geometry")
 
     def upload_text_scene(self, scene):
         """Course text scene (textscene.TextScene); render / readback / primary_ids then work on it."""

@@ -47,6 +47,7 @@ class GltfBuilder:
         self.scene_nodes = []
         self.files = {}
         self.extensions_used = set()
+        self.animations = []
 
     def _view(self, data: bytes):
         while len(self.blob) % 4:
@@ -111,6 +112,25 @@ class GltfBuilder:
         self.cameras.append({"type": "perspective", "perspective": persp})
         return self.node(camera=len(self.cameras) - 1, **node_kw)
 
+    def animation(self, channels, name=None):
+        """One glTF animation from channels (node, path, key times, key values, interpolation); path is "translation",
+        "rotation", "scale" or "weights".  Returns its index."""
+        samplers, chans = [], []
+        comps = {"translation": 3, "rotation": 4, "scale": 3, "weights": 1}
+        for node, path, times, values, interp in channels:
+            t = np.asarray(times, np.float32).reshape(-1)
+            inp = self.accessor(t, FLOAT, "SCALAR")
+            self.accessors[inp]["min"], self.accessors[inp]["max"] = [float(t.min())], [float(t.max())]
+            v = np.asarray(values, np.float32).reshape(-1, comps[path])
+            out = self.accessor(v if comps[path] > 1 else v.reshape(-1), FLOAT, {1: "SCALAR", 3: "VEC3", 4: "VEC4"}[comps[path]])
+            samplers.append({"input": inp, "output": out, "interpolation": interp})
+            chans.append({"sampler": len(samplers) - 1, "target": {"node": node, "path": path}})
+        anim = {"samplers": samplers, "channels": chans}
+        if name is not None:
+            anim["name"] = name
+        self.animations.append(anim)
+        return len(self.animations) - 1
+
     def write(self, out_dir):
         os.makedirs(out_dir, exist_ok=True)
         binname = self.name + ".bin"
@@ -131,6 +151,8 @@ class GltfBuilder:
         }
         if self.extensions_used:
             doc["extensionsUsed"] = sorted(self.extensions_used)
+        if self.animations:
+            doc["animations"] = self.animations
         with open(os.path.join(out_dir, binname), "wb") as f:
             f.write(bytes(self.blob))
         for fn, data in self.files.items():
