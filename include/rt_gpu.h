@@ -425,6 +425,15 @@ int rt_gpu_update_geometry(rt_gpu_ctx *ctx, const rt_geometry_update *u);
  * dst == NULL only reports the size in *bytes.  Selectors 1..4 are empty when the host built the tree. */
 int rt_gpu_debug_get_bvh(rt_gpu_ctx *ctx, int which, void *dst, size_t *bytes);
 
+/* Diagnostic (tests): the light pdf (bvh_mix_dist::pdf, the 1 / n_lights factor included) of n caller rays, as the next
+ * k_shade reads it from the queue for a pending ray: rays is n x 6 floats (origin, then direction as the renderer stores
+ * it), pdf receives n floats.  The default library appends the rays to a pending queue with k_shade's own append (box of
+ * all lights: 0 on a miss, else listed) and runs k_lightpdf_list; the 8-wide library runs k_extend8 over them as a
+ * bounce > 0.  Device 0 only; buffers are allocated per call and freed before it returns, which is after the device work.
+ * RT_ERR_NO_SCENE before any upload; RT_ERR_INVALID_ARG for a null pointer (rays / pdf with n > 0) or a text scene.  A
+ * scene without emitters gives zeros and launches nothing. */
+int rt_gpu_debug_light_pdf(rt_gpu_ctx *ctx, uint64_t n, const float *rays, float *pdf);
+
 /* Per-kernel timing (serialises launches with events; off by default). */
 int rt_gpu_set_profiling(rt_gpu_ctx *ctx, int enable);
 

@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(kExtendThreads, RT_EXT8_MINB)
                         q8_group_hits(f2u(ga.a), f2u(ga.b), f2u(ga.c), f2u(ga.d), f2u(ga.e), f2u(ga.f), g, px, py, pz, one, eps, best_t) |
                         q8_group_hits(f2u(gb.a), f2u(gb.b), f2u(gb.c), f2u(gb.d), f2u(gb.e), f2u(gb.f), g, px, py, pz, one, eps, best_t) << 4;
                     const uint32_t imask = f2u(h.d);
-                    const uint32_t inner = hs & imask, leafm = hs & ~imask;
+                    const uint32_t inner = hs & imask, leafm = hs & ~imask & leaf8_slots(f2u(h.g));  // no empty slot (leaf8_slots)
                     gx = inner ? f2u(h.e) : 0u;
                     gy = inner ? (oct_permute(inner, octinv) << 24) | imask : 0u;
                     if (leafm) {

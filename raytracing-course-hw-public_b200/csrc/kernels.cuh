@@ -663,6 +663,46 @@ __device__ __forceinline__ bool light_box_test(const LightBox &box, f3 o, f3 d, 
     return t0 <= t1;
 }
 
+// k_shade's warp-aggregated append to queue `next` (RT_LIGHT_KERNEL == 2): the lanes of `mask` (the warp's __ballot of
+// the entries it keeps) get consecutive slots of the out queue, returned per lane.  A pending ray (`pend`) that misses
+// the box of all lights has light pdf 0, stored at its slot of lpdf_out; the others are listed for k_lightpdf_list.
+// Both atomics are issued before either result is waited for.  k_lightpdf_debug appends through here as well.
+__device__ __forceinline__ uint32_t append_to_queue(const Queues &q, uint32_t *out_counter, uint32_t next, const LightBox &light_box,
+                                                    uint32_t mask, bool pend, f3 o, f3 d, float eps) {
+    const uint32_t FULL = 0xFFFFFFFFu;
+    const uint32_t lane = lane_id();
+    uint32_t dst = 0;
+    const bool pass = pend && light_box_test(light_box, o, d, eps);
+    const uint32_t mp = __ballot_sync(FULL, pass);
+    uint32_t lp = 0;
+    if (lane == 0) {
+        if (mask) dst = atomicAdd(out_counter, static_cast<uint32_t>(__popc(mask)));
+        if (mp) lp = atomicAdd(q.light_count + next * kCounterStride, static_cast<uint32_t>(__popc(mp)));
+    }
+    dst = __shfl_sync(FULL, dst, 0) + static_cast<uint32_t>(__popc(mask & ((1u << lane) - 1u)));
+    lp = __shfl_sync(FULL, lp, 0) + static_cast<uint32_t>(__popc(mp & ((1u << lane) - 1u)));
+    if (pend && !pass) q_store<0>(q.lpdf_out + dst, 0.0f);
+    if (pass) q.light_list[lp] = dst;
+    return dst;
+}
+
+// rt_gpu_debug_light_pdf: n caller rays (o4 / d4, the pending bit set) appended as pending rays to queue 1 exactly as
+// k_shade appends them; slot_of[i] = the queue slot of ray i.  Whole warps: the grid covers n rounded up to 32.
+__global__ void __launch_bounds__(128) k_lightpdf_debug(const float4 *__restrict__ o4, const float4 *__restrict__ d4, uint32_t n, Queues q,
+                                                       LightBox light_box, float eps, uint32_t *__restrict__ slot_of) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool alive = i < n;
+    const float4 a = alive ? o4[i] : make_float4(0, 0, 0, 0), b = alive ? d4[i] : make_float4(0, 0, 1, 0);
+    const f3 o = mk3(a.x, a.y, a.z), d = mk3(b.x, b.y, b.z);
+    const uint32_t mask = __ballot_sync(0xFFFFFFFFu, alive);
+    const uint32_t dst = append_to_queue(q, q.count + kCounterStride, 1, light_box, mask, alive, o, d, eps);
+    if (alive) {
+        q.o_out[dst] = a;
+        q.d_out[dst] = b;
+        slot_of[i] = dst;
+    }
+}
+
 // k_shade, bounce b.  For every entry of queue b:
 //   1. if the path is pending (its previous bounce sampled a direction and the scene has lights): resolve that
 //      bounce with the light pdf k_extend summed along this very ray — p = p_partial + (1 - VNDF_factor)/2 * lpdf,
@@ -794,20 +834,7 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade(
         const uint32_t mask = __ballot_sync(FULL, alive);
         uint32_t dst = 0;
 #if RT_LIGHT_KERNEL == 2
-        // a pending ray that misses the box of all lights has light pdf 0; the others are listed for k_lightpdf_list
-        // (both atomics are issued before either result is waited for)
-        const bool pend = alive && pending >= 0.0f;
-        const bool pass = pend && light_box_test(light_box, o, d, s.eps);
-        const uint32_t mp = __ballot_sync(FULL, pass);
-        uint32_t lp = 0;
-        if (lane == 0) {
-            if (mask) dst = atomicAdd(out_counter, static_cast<uint32_t>(__popc(mask)));
-            if (mp) lp = atomicAdd(q.light_count + (bounce + 1) * kCounterStride, static_cast<uint32_t>(__popc(mp)));
-        }
-        dst = __shfl_sync(FULL, dst, 0) + static_cast<uint32_t>(__popc(mask & ((1u << lane) - 1u)));
-        lp = __shfl_sync(FULL, lp, 0) + static_cast<uint32_t>(__popc(mp & ((1u << lane) - 1u)));
-        if (pend && !pass) q_store<0>(q.lpdf_out + dst, 0.0f);
-        if (pass) q.light_list[lp] = dst;
+        dst = append_to_queue(q, out_counter, bounce + 1, light_box, mask, alive && pending >= 0.0f, o, d, s.eps);
 #else
         if (lane == 0 && mask) dst = atomicAdd(out_counter, static_cast<uint32_t>(__popc(mask)));
         dst = __shfl_sync(FULL, dst, 0) + static_cast<uint32_t>(__popc(mask & ((1u << lane) - 1u)));

@@ -537,6 +537,16 @@ RT_HD uint32_t leaf8_offset(uint32_t counts, uint32_t s) {
     const uint32_t below = counts & ((1u << (2u * s)) - 1u);
     return popc32(below & 0x5555u) + 2u * popc32(below & 0xAAAAu);
 }
+// bit s set where slot s is a leaf child (count != 0).  An empty slot's inverted box is not always a miss: an axis-parallel
+// ray has 1/d = +-inf on the other two axes, their slab planes become NaN and drop out of fminf / fmaxf, and in a node
+// that is flat along the ray the remaining axis' planes 0 and 255 can coincide.  Its leaf8_offset is the next slot's
+// first triangle, so a hit empty slot visits triangles twice: harmless for a closest hit, a doubled light-pdf term.
+RT_HD uint32_t leaf8_slots(uint32_t counts) {
+    uint32_t m = (counts | (counts >> 1)) & 0x5555u;
+    m = (m | (m >> 1)) & 0x3333u;
+    m = (m | (m >> 2)) & 0x0F0Fu;
+    return (m | (m >> 4)) & 0xFFu;
+}
 
 // closest_hit() over the 8-wide nodes: the sequential statement of k_extend's 8-wide mode (group stack without
 // distances: an entry is culled when its own children are tested against the current best).  `steps` counts node steps.
@@ -569,7 +579,7 @@ RT_HD Hit closest_hit_q8(const DBvh &bvh, f3 o, f3 d, float min_dst, uint32_t *s
             const uint32_t hs = q8_group_hits(f2u(a.a), f2u(a.b), f2u(a.c), f2u(a.d), f2u(a.e), f2u(a.f), g, px, py, pz, qnode_one(), min_dst, best.t) |
                                 q8_group_hits(f2u(b.a), f2u(b.b), f2u(b.c), f2u(b.d), f2u(b.e), f2u(b.f), g, px, py, pz, qnode_one(), min_dst, best.t) << 4;
             const uint32_t imask = f2u(h.d), counts = f2u(h.g);
-            uint32_t leaf = hs & ~imask;
+            uint32_t leaf = hs & ~imask & leaf8_slots(counts);
             while (leaf) {  // highest slot first, like the kernel's leaf phase
                 const uint32_t s = bfind32(leaf);
                 leaf &= ~(1u << s);
@@ -697,7 +707,7 @@ RT_HD float light_pdf_q8(const DScene &s, f3 x, f3 dir) {
             const uint32_t hs = q8_group_hits(f2u(a.a), f2u(a.b), f2u(a.c), f2u(a.d), f2u(a.e), f2u(a.f), g, px, py, pz, qnode_one(), s.eps, INFINITY) |
                                 q8_group_hits(f2u(b.a), f2u(b.b), f2u(b.c), f2u(b.d), f2u(b.e), f2u(b.f), g, px, py, pz, qnode_one(), s.eps, INFINITY) << 4;
             const uint32_t imask = f2u(h.d), counts = f2u(h.g);
-            uint32_t leaf = hs & ~imask;
+            uint32_t leaf = hs & ~imask & leaf8_slots(counts);
             while (leaf) {
                 const uint32_t sl = bfind32(leaf);
                 leaf &= ~(1u << sl);
@@ -708,8 +718,7 @@ RT_HD float light_pdf_q8(const DScene &s, f3 x, f3 dir) {
                     float t, bb, cc;
                     if (tri_test(mk3(t0.x, t0.y, t0.z), mk3(t1.x, t1.y, t1.z), mk3(t2.x, t2.y, t2.z), x, dir, s.eps, t, bb, cc)) {
                         const f4 le = ld4(s.light_extra + k);
-                        const f3 y = x + dir * t;
-                        const f3 xy = y - x;
+                        const f3 xy = dir * t;  // y - x, as light_pdf forms it
                         const float d2 = len2(xy);
                         const f3 w = xy * (1.0f / sqrtf(d2));
                         sum += d2 / (fabsf(dot(w, mk3(le.x, le.y, le.z))) * le.w);
@@ -766,9 +775,9 @@ RT_HD float light_pdf(const DScene &s, f3 x, f3 dir) {
                 if (tri_test(mk3(t0.x, t0.y, t0.z), mk3(t1.x, t1.y, t1.z), mk3(t2.x, t2.y, t2.z), x, dir, s.eps, t, b,
                              c)) {
                     const f4 le = ld4(s.light_extra + k);
-                    // y = x + dir*t; |x - y|^2 and norm(y - x) as the reference forms them
-                    const f3 y = x + dir * t;
-                    const f3 xy = y - x;
+                    // y - x = dir * t, as the kernels form it (light_pdf_term).  The reference's (x + dir * t) - x loses
+                    // the low bits of t * dir to the magnitude of x: 4 % of a term at |x| = 3e4 and t = 0.1.
+                    const f3 xy = dir * t;
                     const float d2 = len2(xy);
                     const f3 w = xy * (1.0f / sqrtf(d2));
                     sum += d2 / (fabsf(dot(w, mk3(le.x, le.y, le.z))) * le.w);

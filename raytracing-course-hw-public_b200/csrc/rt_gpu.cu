@@ -1880,6 +1880,89 @@ int rt_gpu_debug_get_bvh(rt_gpu_ctx *ctx, int which, void *dst, size_t *bytes) {
     return RT_OK;
 }
 
+int rt_gpu_debug_light_pdf(rt_gpu_ctx *ctx, uint64_t n, const float *rays, float *pdf) {
+    const std::string who = "rt_gpu_debug_light_pdf";
+    if (!ctx || (n && (!rays || !pdf))) return fail(RT_ERR_INVALID_ARG, who + ": null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, who + ": no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, who + ": not available for course text scenes");
+    if (n > 0x7FFFFFFFu) return fail(RT_ERR_INVALID_ARG, who + ": more than 2^31 - 1 rays");
+    std::fill(pdf, pdf + n, 0.0f);
+    DeviceState &d = *ctx->devs[0];
+    if (n == 0 || d.scene.n_lights == 0) return RT_OK;
+    CU_CHECK(cudaSetDevice(d.device));
+    const uint32_t m = static_cast<uint32_t>(n);
+    // the rays as pending queue records: (origin, 0), (direction, pending bit)
+    std::vector<float4> o4(m), d4(m);
+    for (uint32_t i = 0; i < m; ++i) {
+        const float *r = rays + 6 * static_cast<size_t>(i);
+        o4[i] = make_float4(r[0], r[1], r[2], 0.0f);
+        d4[i] = make_float4(r[3], r[4], r[5], -0.0f);  // w bits 0x80000000: pending, sample 0
+    }
+    struct Scratch {  // per-call buffers, freed on every return
+        DevBuf<float4> o, d, o2, d2, hit;
+        DevBuf<float> lpdf;
+        DevBuf<uint32_t> list, slot, cnt;
+        ~Scratch() {
+            o.release(); d.release(); o2.release(); d2.release(); hit.release();
+            lpdf.release(); list.release(); slot.release(); cnt.release();
+        }
+    } sb;
+    if (int rc = sb.o.upload(o4, d.stream)) return rc;
+    if (int rc = sb.d.upload(d4, d.stream)) return rc;
+    if (int rc = sb.lpdf.alloc(m)) return rc;
+    const size_t n_cnt = 8 * static_cast<size_t>(rt::kCounterStride);  // count, fetch, light_count: [2] each, own lines
+    if (int rc = sb.cnt.alloc(n_cnt)) return rc;
+    CU_CHECK(cudaMemsetAsync(sb.cnt.p, 0, n_cnt * sizeof(uint32_t), d.stream));
+    const float inv_n_lights = 1.0f / static_cast<float>(d.scene.n_lights);
+    rt::Queues q{};
+    q.count = sb.cnt.p;
+    q.fetch_ext = sb.cnt.p + 2 * rt::kCounterStride;
+    q.fetch_shade = sb.cnt.p + 4 * rt::kCounterStride;
+    q.light_count = sb.cnt.p + 6 * rt::kCounterStride;
+    q.lpdf = q.lpdf_out = sb.lpdf.p;
+    std::vector<float> out(m);
+#if RT_EXT_WIDE8
+    // k_extend8 over a queue 1 of pending rays: its light mode stores the pdf, its scene mode a hit nobody reads
+    if (int rc = sb.hit.alloc(m)) return rc;
+    CU_CHECK(cudaMemcpyAsync(sb.cnt.p + rt::kCounterStride, &m, sizeof(uint32_t), cudaMemcpyHostToDevice, d.stream));
+    q.o_in = sb.o.p;
+    q.d_in = sb.d.p;
+    q.hit = sb.hit.p;
+    rt::k_extend8<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q, 1,
+                                                                         0x3F800000u);
+    CU_CHECK(cudaGetLastError());
+    CU_CHECK(cudaMemcpyAsync(out.data(), sb.lpdf.p, m * sizeof(float), cudaMemcpyDeviceToHost, d.stream));
+    CU_CHECK(cudaStreamSynchronize(d.stream));
+    for (uint32_t i = 0; i < m; ++i) pdf[i] = out[i];
+#else
+    // k_shade's append (light-box test, lpdf = 0 on a miss, the list otherwise), then k_lightpdf_list as a render runs it
+    if (int rc = sb.o2.alloc(m)) return rc;
+    if (int rc = sb.d2.alloc(m)) return rc;
+    if (int rc = sb.list.alloc(m)) return rc;
+    if (int rc = sb.slot.alloc(m)) return rc;
+    q.o_out = sb.o2.p;
+    q.d_out = sb.d2.p;
+    q.light_list = sb.list.p;
+    rt::k_lightpdf_debug<<<(m + 127) / 128, 128, 0, d.stream>>>(sb.o.p, sb.d.p, m, q, d.light_box, d.scene.eps, sb.slot.p);
+    CU_CHECK(cudaGetLastError());
+    rt::Queues ql = q;  // queue 1 is now the input of the light kernel
+    ql.o_in = sb.o2.p;
+    ql.d_in = sb.d2.p;
+    rt::k_lightpdf_list<<<d.light_blocks, rt::kLightThreads, 0, d.stream>>>(d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, ql, 1,
+                                                                            0x3F800000u);
+    CU_CHECK(cudaGetLastError());
+    std::vector<uint32_t> slot(m);
+    CU_CHECK(cudaMemcpyAsync(out.data(), sb.lpdf.p, m * sizeof(float), cudaMemcpyDeviceToHost, d.stream));
+    CU_CHECK(cudaMemcpyAsync(slot.data(), sb.slot.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, d.stream));
+    CU_CHECK(cudaStreamSynchronize(d.stream));
+    for (uint32_t i = 0; i < m; ++i) {
+        if (slot[i] >= m) return fail(RT_ERR_CUDA, who + ": queue slot out of range");
+        pdf[i] = out[slot[i]];
+    }
+#endif
+    return RT_OK;
+}
+
 int rt_gpu_set_profiling(rt_gpu_ctx *ctx, int enable) {
     if (!ctx) return fail(RT_ERR_INVALID_ARG, "rt_gpu_set_profiling: null handle");
     ctx->profiling = enable != 0;

@@ -16,7 +16,8 @@ LIB_PATH = os.environ.get("RT_GPU_LIB") or os.path.join(_abi.PKG_DIR, "librt_gpu
 SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upload_text_scene", "rt_gpu_render", "rt_gpu_readback",
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
            "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive",
-           "rt_gpu_render_views", "rt_gpu_render_views_adaptive", "rt_gpu_render_projected", "rt_gpu_update_geometry"]
+           "rt_gpu_render_views", "rt_gpu_render_views_adaptive", "rt_gpu_render_projected", "rt_gpu_update_geometry",
+           "rt_gpu_debug_light_pdf"]
 
 _lib = None
 
@@ -45,6 +46,7 @@ def lib():
         L.rt_gpu_set_profiling.argtypes = [C.c_void_p, C.c_int]
         L.rt_gpu_debug_get_bvh.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_size_t)]
         L.rt_gpu_fp32_peak.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
+        L.rt_gpu_debug_light_pdf.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
         L.rt_gpu_last_error.restype = C.c_char_p
         _lib = L
     return _lib
@@ -235,6 +237,15 @@ class RtGpu:
         out = np.zeros(n.value // np.dtype(dtype).itemsize, dtype)
         if n.value:
             _check(lib().rt_gpu_debug_get_bvh(self._h, which, out.ctypes.data_as(C.c_void_p), C.byref(n)), "rt_gpu_debug_get_bvh")
+        return out
+
+    def debug_light_pdf(self, rays):
+        """Diagnostic: the light pdf the next k_shade would read for each of `rays` (n x 6 float32: origin, direction) as a
+        pending ray (rt_gpu_debug_light_pdf); float32 [n]."""
+        rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 6)
+        out = np.zeros(len(rays), np.float32)
+        _check(lib().rt_gpu_debug_light_pdf(self._h, len(rays), rays.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p)),
+               "rt_gpu_debug_light_pdf")
         return out
 
     def fp32_peak_tflops(self):

@@ -508,6 +508,114 @@ int hc_brute_hits(const float *tri, uint64_t n_tris, const float *rays, uint64_t
     return 0;
 }
 
+// ---- independent light-pdf reference ------------------------------------------------------------------------------------
+// bvh_mix_dist::pdf of each ray by brute force over every light triangle, in double precision, sharing no code with
+// pt_core.cuh.  Each (ray, light) pair is classified by hc_brute_hits' rule (clear hit / borderline / clear miss, local
+// tolerance w).  A hit pair contributes term = t^2 |d|^2 / (cos * A), A = area2 / 2 of the float32 vertices, with the
+// per-term relative tolerance
+//   tau = c_tol * 2^-23 * (1 / cos + |e1| |e2| / |n| + 1) + 2 w / t:
+// 1 / cos for the float32 cosine, |e1| |e2| / |n| for the cancellation in the cross product that gives the light's normal
+// and area (the kernels' DLight record suffers it as well: slivers), 1 for the rest of the term's arithmetic, and 2 w / t
+// for t^2 when t itself is only known to w.  Per ray, with m = n_clear + n_border terms:
+//   lo = sum_clear term max(0, 1 - tau) (1 - (m + 4) 2^-23) / n_lights
+//   hi = sum_{clear + border} term (1 + tau) (1 + (m + 4) 2^-23) / n_lights      (+inf when a borderline term is not finite)
+// (m + 4) 2^-23 bounds the float32 summation of m terms, the 1 / n_lights factor and the final rounding.  A float32
+// evaluation of the same sum must lie in [lo, hi]; a ray without clear and borderline pairs must give exactly 0.
+int hc_brute_light_pdf(const float *tri, uint64_t n_lights, const float *rays, uint64_t n_rays, double eps, double c_tol, double *lo,
+                       double *hi, int32_t *n_clear, int32_t *n_border) {
+    struct T {
+        double v[3][3], e1[3], e2[3], n[3], area2, alt[3], sliver;
+    };
+    std::vector<T> tr(n_lights);
+    auto len = [](const double *a) { return std::sqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]); };
+    for (uint64_t k = 0; k < n_lights; ++k) {
+        T &t = tr[k];
+        for (int i = 0; i < 3; ++i)
+            for (int a = 0; a < 3; ++a) t.v[i][a] = tri[9 * k + 3 * i + a];
+        double e12[3];
+        for (int a = 0; a < 3; ++a) t.e1[a] = t.v[1][a] - t.v[0][a], t.e2[a] = t.v[2][a] - t.v[0][a], e12[a] = t.v[2][a] - t.v[1][a];
+        t.n[0] = t.e1[1] * t.e2[2] - t.e1[2] * t.e2[1];
+        t.n[1] = t.e1[2] * t.e2[0] - t.e1[0] * t.e2[2];
+        t.n[2] = t.e1[0] * t.e2[1] - t.e1[1] * t.e2[0];
+        t.area2 = len(t.n);
+        const double l[3] = {len(e12), len(t.e2), len(t.e1)};
+        for (int i = 0; i < 3; ++i) t.alt[i] = l[i] > 0 ? t.area2 / l[i] : 0.0;
+        t.sliver = t.area2 > 0 ? l[1] * l[2] / t.area2 : INFINITY;
+    }
+    const double u = std::ldexp(1.0, -23);
+    const double inv_n = n_lights ? 1.0 / (double)n_lights : 0.0;
+    auto work = [&](uint64_t r0, uint64_t r1) {
+        for (uint64_t r = r0; r < r1; ++r) {
+            const double o[3] = {rays[6 * r], rays[6 * r + 1], rays[6 * r + 2]}, d[3] = {rays[6 * r + 3], rays[6 * r + 4], rays[6 * r + 5]};
+            const double dl = len(d);
+            double s_lo = 0, s_hi = 0;
+            int32_t nc = 0, nb = 0;
+            for (uint64_t k = 0; k < n_lights; ++k) {
+                const T &t = tr[k];
+                const double det = -(d[0] * t.n[0] + d[1] * t.n[1] + d[2] * t.n[2]);
+                if (det == 0.0 || t.area2 == 0.0) continue;  // clear miss
+                const double y[3] = {o[0] - t.v[0][0], o[1] - t.v[0][1], o[2] - t.v[0][2]};
+                const double rr[3] = {d[1] * y[2] - d[2] * y[1], d[2] * y[0] - d[0] * y[2], d[0] * y[1] - d[1] * y[0]};
+                const double beta = -(t.e2[0] * rr[0] + t.e2[1] * rr[1] + t.e2[2] * rr[2]) / det;
+                const double gamma = (t.e1[0] * rr[0] + t.e1[1] * rr[1] + t.e1[2] * rr[2]) / det;
+                const double tt = (y[0] * t.n[0] + y[1] * t.n[1] + y[2] * t.n[2]) / det;
+                double m = 0;
+                for (int i = 0; i < 3; ++i)
+                    for (int a = 0; a < 3; ++a) m = std::max(m, std::fabs(t.v[i][a] - o[a]));
+                const double cosg = std::fabs(det) / (dl * t.area2);
+                const double w = c_tol * u * (m + std::fabs(tt)) / cosg;
+                const double dist = std::min({(1.0 - beta - gamma) * t.alt[0], beta * t.alt[1], gamma * t.alt[2]});
+                if (dist < -w || tt < eps - w) continue;  // clear miss
+                const double term = tt * tt * dl * dl / (cosg * t.area2 / 2);
+                const double tau = c_tol * u * (1 / cosg + t.sliver + 1) + 2 * w / std::fabs(tt);
+                if (dist > w && tt > eps + w && cosg > 1e-4) {
+                    ++nc;
+                    s_lo += term * std::max(0.0, 1 - tau);
+                    s_hi += term * (1 + tau);
+                } else {
+                    ++nb;
+                    s_hi += std::isfinite(term) && std::isfinite(tau) ? term * (1 + tau) : INFINITY;
+                }
+            }
+            const double mm = (double)(nc + nb) + 4;
+            lo[r] = s_lo * (1 - mm * u) * inv_n;
+            hi[r] = s_hi * (1 + mm * u) * inv_n;
+            n_clear[r] = nc;
+            n_border[r] = nb;
+        }
+    };
+    const unsigned n_threads = std::max(1u, std::min(64u, std::thread::hardware_concurrency()));
+    std::vector<std::thread> pool;
+    const uint64_t chunk = (n_rays + n_threads - 1) / n_threads;
+    for (unsigned i = 0; i < n_threads; ++i) {
+        const uint64_t a = std::min<uint64_t>(n_rays, i * chunk), b = std::min<uint64_t>(n_rays, a + chunk);
+        if (a < b) pool.emplace_back(work, a, b);
+    }
+    for (auto &th : pool) th.join();
+    return 0;
+}
+
+// The light pdf (bvh_mix_dist::pdf, 1 / n_lights included) of arbitrary rays (n x 6 floats: origin, direction) through the
+// host compilation of the device math, the scene packed as hc_render packs it: pdf_exact = light_pdf over the exact
+// binary light nodes, pdf_q8 = light_pdf_q8 over the 8-wide quantised light nodes.  A scene without lights gives 0.
+int hc_light_pdf(const rt_scene_desc *sc, uint64_t n, const float *rays, float *pdf_exact, float *pdf_q8) {
+    const bool keep = g_wide8;
+    for (int pass = 0; pass < 2; ++pass) {
+        HostScene hs;
+        g_wide8 = pass == 1;
+        const int rc = build(sc, hs);
+        g_wide8 = keep;
+        if (rc) return rc;
+        if ((pass == 1) != (hs.d.light.n_nodes8 != 0) && hs.d.n_lights) return -100;  // not the node format asked for
+        float *out = pass ? pdf_q8 : pdf_exact;
+        for (uint64_t i = 0; i < n; ++i) {
+            const f3 o = mk3(rays[6 * i], rays[6 * i + 1], rays[6 * i + 2]), d = mk3(rays[6 * i + 3], rays[6 * i + 4], rays[6 * i + 5]);
+            out[i] = hs.d.n_lights ? light_pdf(hs.d, o, d) : 0.0f;
+        }
+    }
+    return 0;
+}
+
 // Wall time of the re-pack phases (ms): out[0] SAH build, out[1] pack_bvh of the scene tree (triangles, nodes, both
 // quantisations, collapse), out[2] whole pack_scene with rebuild, out[3] the upload path's pack_scene (4-wide only),
 // out[4..7] its phases.
