@@ -416,6 +416,46 @@ typedef struct rt_geometry_update {
 
 int rt_gpu_update_geometry(rt_gpu_ctx *ctx, const rt_geometry_update *u);
 
+/* ---- AOV render -------------------------------------------------------------------------------------------------
+ * rt_gpu_render_aov returns per-pixel feature buffers ("arbitrary output variables": the guides of a denoiser and the
+ * layers of compositing) from the camera samples of the beauty render.  The image, views, projections, keys and pixel
+ * range are those of rt_gpu_render (views == NULL: the scene camera, one image), rt_gpu_render_views (projections ==
+ * NULL) or rt_gpu_render_projected: n = n_views * width * height pixels, view-major (n = width * height without views).
+ * Sample s of pixel p is the camera ray those calls trace for the same params, views, projections and seed, bit for
+ * bit; the samples are [0, samples).  RT_MODE_PRIMARY_IDS traces the rays of that mode instead: pixel centres through
+ * the lens centre, sample 0, the whole image.
+ * Visible surface of a sample: the beauty path's alpha pass-throughs are walked with its own coins (at bounce b the hit
+ * is visible when u01(philox(key, b, 0).x) <= its alpha; otherwise the walk goes on from the hit along the same
+ * direction), for at most ray_depth hits.  Its values, or all zero when a sample misses or passes through ray_depth
+ * hits:
+ *   coverage  1;
+ *   albedo    the base colour times the colour texture;
+ *   normal    the world-space shading normal (normal map included), flipped towards the ray;
+ *   emission  the emissive factor times the emissive texture;
+ *   depth     the distance along the camera ray from its origin (the sum of the walked segments).
+ * Each pixel's per-sample values are NaN-scrubbed and summed in float32 in the order of the beauty render's sums, and
+ * rt_gpu_readback_aov divides by samples (1 for RT_MODE_PRIMARY_IDS): a value is the mean over ALL samples, misses
+ * counting 0.  So coverage is the fraction of samples with a visible surface, "mean over covered samples" is a value
+ * divided by coverage, and the mean normal is not re-normalised.  Pixels outside [pixel_begin, pixel_end) read 0.
+ * With ray_depth = 1 and a black constant sky, emission equals the beauty render's rgb_mean of the same call and
+ * batches, bit for bit.  View v of a call equals a one-view call with view_base = v.
+ * The beauty render's sums, adaptive counts and errors, primary ids, stats and accumulation rules are left alone, so a
+ * beauty render followed by rt_gpu_render_aov with the same arguments gives an image and its matching buffers.  Paths
+ * in flight per batch follow max_paths_in_flight (the default is sized from free memory); a path takes 48 bytes
+ * beyond the beauty render's.  A multi-device handle renders on device 0 only, with the one-device result.
+ * RT_ERR_NO_SCENE before an upload.  RT_ERR_INVALID_ARG for a null ctx or params, a text scene, a mode other than
+ * RT_MODE_BEAUTY / RT_MODE_PRIMARY_IDS, samples == 0 (beauty), sample_begin or sample_end != 0, RT_FLAG_ACCUMULATE,
+ * projections without views, an illegal image size or pixel range, and whatever rt_gpu_render_views /
+ * rt_gpu_render_projected refuse for the views and projections. */
+int rt_gpu_render_aov(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views /* NULL: the scene camera */,
+                      const rt_projection *projections /* NULL: pinhole; non-NULL requires views */);
+
+/* The last AOV render's means: albedo, normal and emission n * 3 floats, depth and coverage n floats (any pointer may
+ * be NULL); stats holds that render's own samples, extension rays, kernel launches and render_ms.  RT_ERR_NO_RENDER
+ * before any AOV render on the handle. */
+int rt_gpu_readback_aov(rt_gpu_ctx *ctx, float *albedo, float *normal, float *emission, float *depth, float *coverage,
+                        rt_stats *stats);
+
 /* Diagnostic (tests): the scene BVH the library built on the device during the last rt_gpu_upload_scene (with the
  * boxes of any rt_gpu_update_geometry since).
  * which = 0: uint32[8] {n_tris, binary node slots, 4-wide nodes, root link, worst-case traversal stack need, depth of

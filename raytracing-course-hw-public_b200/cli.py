@@ -12,10 +12,36 @@ def adaptive_steps(samples):
     return max(2, -(-samples // 16))
 
 
-def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1, rel_error=None, projection=None):
+AOV_NAMES = ("albedo", "normal", "emission", "depth", "coverage")
+
+
+def parse_aov(text):
+    """RT_AOV=<samples> -> samples of the AOV render (unset, empty or 0: off)"""
+    if text is None or text == "":
+        return 0
+    if not text.isdigit():
+        raise ValueError(f"RT_AOV={text}: expected the AOV render's samples per pixel, an integer >= 0")
+    return int(text)
+
+
+def aov_paths(out, prefix=""):
+    """{name: <stem><prefix>_<name>.pfm} of the AOV buffers written next to the image `out`"""
+    stem, _ = os.path.splitext(out)
+    return {k: f"{stem}{prefix}_{k}.pfm" for k in AOV_NAMES}
+
+
+def write_aovs(aovs, out, prefix=""):
+    from . import pfm
+
+    for k, path in aov_paths(out, prefix).items():
+        pfm.write_pfm(path, aovs[k])
+
+
+def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1, rel_error=None, projection=None, aov=0):
     """Mirror of run_raytracer(scene, image) (src/raytracer.h:629): float means [H, W, 3] + stats.  With rel_error,
     `samples` is the maximum spp of an adaptive render (rt_gpu_render_adaptive).  With projection (a Projection), the
-    scene camera is rendered through it (rt_gpu_render_projected)."""
+    scene camera is rendered through it (rt_gpu_render_projected).  With aov > 0 the AOV render (rt_gpu_render_aov) of
+    `aov` spp follows on the same camera, projection and seed, and its readback_aov dict is returned third."""
     from . import gpu, textscene
 
     with gpu.RtGpu(n_gpus, 0) as rt:
@@ -30,28 +56,42 @@ def run_raytracer(scene, width, height, samples, seed=0, n_gpus=1, rel_error=Non
             rt.render_projected([scene.camera()], [projection], width, height, samples, seed=seed, max_paths_in_flight=paths,
                                 adaptive=None if rel_error is None else (step, step, rel_error))
             mean, stats = rt.readback()
-            return mean[0], stats
+            if not aov:
+                return mean[0], stats
+            rt.render_aov(width, height, aov, seed=seed, cameras=[scene.camera()], projections=[projection], max_paths_in_flight=paths)
+            return mean[0], stats, {k: v[0] for k, v in rt.readback_aov().items()}
         if rel_error is None:
             rt.render(width, height, samples, seed=seed, max_paths_in_flight=paths)
         else:
             step = adaptive_steps(samples)
             rt.render_adaptive(width, height, samples, step, step, rel_error, seed=seed, max_paths_in_flight=paths)
-        return rt.readback()
+        if not aov:
+            return rt.readback()
+        mean, stats = rt.readback()
+        rt.render_aov(width, height, aov, seed=seed, max_paths_in_flight=paths)
+        return mean, stats, rt.readback_aov()
 
 
-def run_views(scene, cameras, width, height, samples, seed=0, n_gpus=1, projections=None):
+def run_views(scene, cameras, width, height, samples, seed=0, n_gpus=1, projections=None, aov=0):
     """Every camera of `cameras` in one rt_gpu_render_views call, or in one rt_gpu_render_projected call when a
-    projection of `projections` is not a pinhole: float means [V, H, W, 3] + stats."""
+    projection of `projections` is not a pinhole: float means [V, H, W, 3] + stats.  With aov > 0 the AOV render of
+    `aov` spp over the same views follows, and its readback_aov dict ([V, H, W, ...]) is returned third."""
     from . import gpu
 
     paths = int(os.environ.get("RT_PATHS", 128 << 20))
     with gpu.RtGpu(n_gpus, 0) as rt:
         rt.upload_scene(scene)
-        if projections and any(p != Projection.pinhole() for p in projections):
+        projected = bool(projections) and any(p != Projection.pinhole() for p in projections)
+        if projected:
             rt.render_projected(cameras, projections, width, height, samples, seed=seed, max_paths_in_flight=paths)
         else:
             rt.render_views(cameras, width, height, samples, seed=seed, max_paths_in_flight=paths)
-        return rt.readback()
+        if not aov:
+            return rt.readback()
+        mean, stats = rt.readback()
+        rt.render_aov(width, height, aov, seed=seed, cameras=cameras, projections=projections if projected else None,
+                      max_paths_in_flight=paths)
+        return mean, stats, rt.readback_aov()
 
 
 def parse_frames(text):
@@ -141,6 +181,17 @@ def main(argv=None):
                 return 1
         else:
             projection = None
+        # RT_AOV=<samples>: after the beauty render, the AOV render (rt_gpu_render_aov) of the same camera(s), projection
+        # and seed at <samples> spp, written to <stem>_albedo.pfm, _normal, _emission, _depth and _coverage
+        try:
+            aov = parse_aov(os.environ.get("RT_AOV"))
+        except ValueError as e:
+            print(e, file=sys.stderr)
+            return 1
+        if aov and (frames is not None or textscene.is_text_scene(argv[1])):
+            print("RT_AOV renders the AOV buffers of one glTF render: it cannot be combined with RT_FRAMES or a text scene",
+                  file=sys.stderr)
+            return 1
         cameras = os.environ.get("RT_CAMERAS")
         if frames is not None:
             if cameras is not None or textscene.is_text_scene(argv[1]):
@@ -168,16 +219,23 @@ def main(argv=None):
                 return 1
             cams = scene.cameras or [scene.camera()]  # no camera node: the scene's default camera
             projs = [projection] * len(cams) if projection is not None else scene.projections or [Projection.pinhole()]
-            means, stats = run_views(scene, cams, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
-                                     n_gpus=int(os.environ.get("RT_GPUS", "1")), projections=projs)
+            res = run_views(scene, cams, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
+                            n_gpus=int(os.environ.get("RT_GPUS", "1")), projections=projs, aov=aov)
+            means, stats = res[0], res[1]
             for path, mean in zip(view_paths(argv[5], len(cams)), means):
                 host.write_ppm(path, host.tonemap_rgb8(mean))
+            if aov:
+                for i in range(len(cams)):
+                    write_aovs({k: v[i] for k, v in res[2].items()}, argv[5], f"_{i}")
             ms = max(stats["render_ms"], 1e-9)
             print(f"rt_gpu: {len(cams)} views, {ms:.1f} ms, {stats['samples'] / ms * 1e-3:.1f} Msamples/s", file=sys.stderr)
             return 0
-        mean, stats = run_raytracer(scene, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
-                                    n_gpus=int(os.environ.get("RT_GPUS", "1")), rel_error=rel_error, projection=projection)
+        res = run_raytracer(scene, width, height, samples, seed=int(os.environ.get("RT_SEED", "0")),
+                            n_gpus=int(os.environ.get("RT_GPUS", "1")), rel_error=rel_error, projection=projection, aov=aov)
+        mean, stats = res[0], res[1]
         host.write_ppm(argv[5], host.tonemap_rgb8(mean))
+        if aov:
+            write_aovs(res[2], argv[5])
         ms = max(stats["render_ms"], 1e-9)
         print(f"rt_gpu: {ms:.1f} ms, {stats['samples'] / ms * 1e-3:.1f} Msamples/s", file=sys.stderr)
         if rel_error is not None:

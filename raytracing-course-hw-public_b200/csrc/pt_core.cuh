@@ -799,11 +799,13 @@ RT_HD float light_pdf(const DScene &s, f3 x, f3 dir) {
 // neighbours, per-texel gamma BEFORE interpolation (LUT == powf(k/255, 2.2f)), alpha untouched;
 // 1-texel textures are returned raw (geometry.h:548-550).
 // One out-of-line copy on the device (k_shade calls it for up to four maps per hit): 5 % less k_shade time than the
-// four inlined copies (code size / instruction cache), measured on the B200.
+// four inlined copies (code size / instruction cache), measured on the B200.  COPY selects one of several out-of-line
+// copies: ptxas fits a shared callee's register convention to all of its callers, so a kernel that gets a copy of its
+// own (the AOV render's k_aov_step: COPY 1) leaves k_shade's code exactly as it was.
 #if defined(__CUDACC__) && !defined(RT_TEX_INLINE)
-__host__ __device__ __noinline__
+template <int COPY = 0> __host__ __device__ __noinline__
 #else
-RT_HD
+template <int COPY = 0> RT_HD
 #endif
 f4 tex_sample(const DScene &s, const float *lut, int32_t tex, float u, float v, bool gamma) {
     const f4 ti = ld4(s.textures + tex);
@@ -865,7 +867,7 @@ struct Surface {
     float metallic, roughness, ior;
 };
 
-RT_HD Surface make_surface(const DScene &s, const float *lut, const Hit &h, f3 dir) {
+template <int TEX_COPY = 0> RT_HD Surface make_surface(const DScene &s, const float *lut, const Hit &h, f3 dir) {
     Surface sf;
     const char *tp = reinterpret_cast<const char *>(s.scene.tris + h.tri);
     const f4 t1 = ld4(tp + 16), t2 = ld4(tp + 32);
@@ -896,7 +898,7 @@ RT_HD Surface make_surface(const DScene &s, const float *lut, const Hit &h, f3 d
             tangent = normalize(mk3(g0.x, g0.y, g0.z) * w0 + mk3(g0.w, g1.x, g1.y) * h.b + mk3(g1.z, g1.w, g2.x) * h.c);
         }
         const f3 bitangent = cross(smooth, tangent);  // not normalised, bvh.h:102
-        const f4 n01 = tex_sample(s, lut, normal_tex, tu, tv, false);
+        const f4 n01 = tex_sample<TEX_COPY>(s, lut, normal_tex, tu, tv, false);
         const f3 nl = normalize(mk3(n01.x * 2.0f - 1.0f, n01.y * 2.0f - 1.0f, n01.z * 2.0f - 1.0f));
         ns = normalize(nl.x * tangent + nl.y * bitangent + nl.z * smooth);
     } else if (s.tangents) {
@@ -908,20 +910,20 @@ RT_HD Surface make_surface(const DScene &s, const float *lut, const Hit &h, f3 d
 
     f4 col = f4{m0.x, m0.y, m0.z, m0.w};
     if (color_tex >= 0) {
-        const f4 c = tex_sample(s, lut, color_tex, tu, tv, true);
+        const f4 c = tex_sample<TEX_COPY>(s, lut, color_tex, tu, tv, true);
         col = f4{col.x * c.x, col.y * c.y, col.z * c.z, col.w * c.w};
     }
     sf.color = mk3(col.x, col.y, col.z);
     sf.alpha = col.w;
     sf.emission = mk3(m1.x, m1.y, m1.z);
     if (emissive_tex >= 0) {
-        const f4 e = tex_sample(s, lut, emissive_tex, tu, tv, true);
+        const f4 e = tex_sample<TEX_COPY>(s, lut, emissive_tex, tu, tv, true);
         sf.emission = sf.emission * mk3(e.x, e.y, e.z);
     }
     sf.roughness = m1.w;
     sf.metallic = m2.x;
     if (mr_tex >= 0) {
-        const f4 mr = tex_sample(s, lut, mr_tex, tu, tv, false);
+        const f4 mr = tex_sample<TEX_COPY>(s, lut, mr_tex, tu, tv, false);
         sf.metallic *= mr.z;   // metallic = B, roughness = G (geometry.h:623-626)
         sf.roughness *= mr.y;
     }

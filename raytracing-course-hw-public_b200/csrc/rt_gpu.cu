@@ -35,6 +35,7 @@
 #include "adaptive.cuh"
 #include "views.cuh"
 #include "projection.cuh"
+#include "aov.cuh"
 #include "rt_gpu.h"
 
 namespace {
@@ -113,6 +114,7 @@ template <class T> struct DevBuf {
 };
 
 constexpr size_t kBytesPerPath = 8 * sizeof(float4) + 3 * sizeof(float);  // q_o, q_d, q_thr (x2 parities) + hit + rad + lpdf (x2) + light list
+constexpr size_t kAovBytesPerPath = 3 * sizeof(float4);                       // an AOV render's slots (aov.cuh), beyond the queues
 
 enum KernelKind { K_GENERATE = 0, K_EXTEND = 1, K_SHADE = 2, K_ACCUMULATE = 3, K_IDS = 4, K_LIGHTPDF = 5, K_COUNT = 8 };
 
@@ -213,6 +215,11 @@ struct DeviceState {
     DevBuf<uint8_t> rgb8;
     DevBuf<rt::Camera> cams;  // the cameras of the last multi-view render (rt_gpu_render_views), one per view
     DevBuf<rt::Projection> projs;  // their projections when it was rt_gpu_render_projected
+    // AOV render (rt_gpu_render_aov, aov.cuh): three float4 slots per path of a batch (aov_cap paths), three float4
+    // sums per pixel of the last AOV render, and the means of its readback
+    DevBuf<float4> aov_slots, aov_sums;
+    size_t aov_cap = 0;
+    DevBuf<float> aov_means;
     int extend_blocks = 0, shade_blocks = 0, light_blocks = 0;
     rt::LightBox light_box{};  // box of all light triangles (k_shade tests the rays it queues against it)
     // profiling
@@ -245,6 +252,12 @@ struct rt_gpu_ctx {
     rt_stats stats{};
     uint32_t ray_depth = 0;
     rt::PackedScene packed;  // staging of the last upload, kept so that the next one re-uses its (already touched) memory
+    // the last AOV render (rt_gpu_render_aov): its resolved parameters, views (0 = the scene camera), the sample count
+    // its readback divides by, and its own stats; rt_gpu_readback_aov returns RT_ERR_NO_RENDER before the first
+    bool have_aov = false;
+    rt_render_params aov_last{};
+    uint32_t aov_views = 0, aov_samples = 0;
+    rt_stats aov_stats{};
 };
 
 namespace {
@@ -749,20 +762,25 @@ int enqueue_text_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt
 // 256 Mi paths -> 771 / 819 / 845 / 881 / 896 / 910 Msamples/s on config 4 (B200, measured; a later build: 128 / 256 /
 // 512 / 640 Mi -> 1149 / 1163 / 1169 / 1169).  The default is 512 Mi paths (140 B of queue state each = 75 GB of the
 // 180 GB), capped at half of the free memory.
-size_t batch_cap(const DeviceState &d, uint32_t max_paths_in_flight, size_t want_total) {
+// bytes_per_path: what one path of the batch needs; held_paths / held_bytes: the paths the handle's buffers already hold
+// and their bytes (given back to the free memory when they grow)
+size_t batch_cap_of(uint32_t max_paths_in_flight, size_t want_total, size_t bytes_per_path, size_t held_paths, size_t held_bytes) {
     size_t max_paths = max_paths_in_flight;
     if (max_paths == 0) {
         max_paths = static_cast<size_t>(512) << 20;
         // the memory query is a slow, jittery driver call (tens of ms with 50 GB allocated): only when the queues
         // would have to grow beyond what this handle already holds
-        if (std::min(max_paths, want_total) > d.queue_cap) {
+        if (std::min(max_paths, want_total) > held_paths) {
             size_t free_b = 0, total_b = 0;
             if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess)
-                max_paths = std::min(max_paths, std::max(d.queue_cap, (free_b + d.queue_cap * kBytesPerPath) / 2 / kBytesPerPath));
+                max_paths = std::min(max_paths, std::max(held_paths, (free_b + held_bytes) / 2 / bytes_per_path));
         }
     }
     max_paths = std::max<size_t>(max_paths, 1024);
     return std::min(max_paths, want_total);
+}
+size_t batch_cap(const DeviceState &d, uint32_t max_paths_in_flight, size_t want_total) {
+    return batch_cap_of(max_paths_in_flight, want_total, kBytesPerPath, d.queue_cap, d.queue_cap * kBytesPerPath);
 }
 
 size_t n_counters_of(uint32_t qdepth) { return (6 * static_cast<size_t>(qdepth) + 2) * rt::kCounterStride; }  // one 256-byte line each
@@ -945,6 +963,90 @@ int enqueue_render(rt_gpu_ctx *ctx, DeviceState &d, int dev_index, const rt_rend
             rt::k_accumulate<<<(bp.npix + 255) / 256, 256, 0, d.stream>>>(bp, d.rad, d.accum.p);
             mark(ctx, d, K_ACCUMULATE);
             launches += 2;
+        }
+    }
+    CU_CHECK(cudaGetLastError());
+    CU_CHECK(cudaEventRecord(d.ev_end, d.stream));
+    return RT_OK;
+}
+
+// Enqueue the AOV render (aov.cuh) of samples [0, samples) on device d: enqueue_render's batches and queue 0, then per
+// bounce k_extend and k_aov_step, then k_aov_accumulate into d.aov_sums.  RT_MODE_PRIMARY_IDS: the pixel-centre rays of
+// that mode (sample 0, the whole image).  Touches none of the beauty render's sums, counts, ids or stats.
+int enqueue_render_aov(DeviceState &d, const rt_render_params &rp, const ViewSet *views, uint64_t &launches) {
+    CU_CHECK(cudaSetDevice(d.device));
+    const uint32_t W = rp.width, H = rp.height, depth = d.scene.ray_depth;
+    const uint32_t n_views = views ? static_cast<uint32_t>(views->cams.size()) : 1u;
+    const size_t n_pix = static_cast<size_t>(W) * H * n_views;
+    const rt::Camera cam = make_camera(scene_camera(d.scene), W, H);
+    const uint32_t key_offset = views ? static_cast<uint32_t>(static_cast<uint64_t>(views->view_base) * W * H) : 0u;
+    const bool centre = rp.mode == RT_MODE_PRIMARY_IDS;
+    if (int rc = d.aov_sums.alloc(3 * n_pix)) return rc;
+    if (int rc = d.stats.alloc(4)) return rc;
+    CU_CHECK(cudaMemsetAsync(d.stats.p, 0, 4 * sizeof(unsigned long long), d.stream));
+    CU_CHECK(cudaMemsetAsync(d.aov_sums.p, 0, 3 * n_pix * sizeof(float4), d.stream));
+    const rt::AovPlanes sums{d.aov_sums.p, d.aov_sums.p + n_pix, d.aov_sums.p + 2 * n_pix};
+    CU_CHECK(cudaEventRecord(d.ev_begin, d.stream));
+    const uint32_t s_end = centre ? 1u : rp.samples;
+    const size_t px_begin = centre ? 0 : rp.pixel_begin, px_end = centre ? n_pix : rp.pixel_end;
+    const size_t n_render = px_end - px_begin;
+    if (depth == 0 || n_render == 0) {  // no hit is walked: every value is 0
+        CU_CHECK(cudaEventRecord(d.ev_end, d.stream));
+        return RT_OK;
+    }
+    const size_t cap = batch_cap_of(rp.max_paths_in_flight, n_render * static_cast<size_t>(s_end), kBytesPerPath + kAovBytesPerPath,
+                                    std::min(d.queue_cap, d.aov_cap), d.queue_cap * kBytesPerPath + d.aov_cap * kAovBytesPerPath);
+    if (int rc = d.alloc_queues(cap)) return rc;
+    if (cap > d.aov_cap) {
+        d.aov_cap = 0;
+        if (int rc = d.aov_slots.alloc(3 * cap)) return rc;
+        d.aov_cap = cap;
+    }
+    const rt::AovPlanes slots{d.aov_slots.p, d.aov_slots.p + d.aov_cap, d.aov_slots.p + 2 * d.aov_cap};
+    const uint32_t qdepth = std::max(depth, 1u);
+    const size_t n_counters = n_counters_of(qdepth);
+    if (int rc = d.counters.alloc(n_counters)) return rc;
+    const rt::Queues q_gen = queues_of(d, qdepth, -1);
+    if (views)
+        if (int rc = upload_views(d, *views)) return rc;
+    const float inv_n_lights = d.scene.n_lights ? 1.0f / static_cast<float>(d.scene.n_lights) : 0.0f;
+    rt::BatchParams bp;
+    bp.width = W;
+    bp.height = H;
+    bp.k0 = static_cast<uint32_t>(rp.seed);
+    bp.k1 = static_cast<uint32_t>(rp.seed >> 32);
+    bp.centre = centre ? 1u : 0u;
+    // enqueue_render's batches: all pixels x k samples when the image fits, else pixel chunks x 1 sample
+    const size_t pix_chunk = std::max<size_t>(1, std::min(n_render, cap));
+    for (size_t pix0 = px_begin; pix0 < px_end; pix0 += pix_chunk) {
+        const uint32_t npix = static_cast<uint32_t>(std::min(pix_chunk, px_end - pix0));
+        const uint32_t k_max = static_cast<uint32_t>(std::max<size_t>(1, cap / npix));
+        for (uint32_t s0 = 0; s0 < s_end; s0 += k_max) {
+            bp.pix0 = static_cast<uint32_t>(pix0);
+            bp.npix = npix;
+            bp.s0 = s0;
+            bp.k = std::min(k_max, s_end - s0);
+            bp.tiled = !centre && pix0 == 0 && npix == n_pix && W % 8 == 0 && (H * n_views) % 4 == 0 && !std::getenv("RT_NO_TILES");
+            const uint32_t n = bp.npix * bp.k;
+            CU_CHECK(cudaMemsetAsync(d.counters.p, 0, n_counters * sizeof(uint32_t), d.stream));
+            if (views && !views->projs.empty())
+                rt::k_generate_proj<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, d.projs.p, bp, q_gen, key_offset);
+            else if (views)
+                rt::k_generate_views<<<(n + 255) / 256, 256, 0, d.stream>>>(d.cams.p, bp, q_gen, key_offset);
+            else
+                rt::k_generate<<<(n + 255) / 256, 256, 0, d.stream>>>(cam, bp, q_gen);
+            rt::BatchParams bp_key = bp;  // the slot of a path: (sample - s0) * npix + (key - pix0), as k_shade's
+            bp_key.pix0 += key_offset;
+            // the queues shrink with every bounce; their sizes live on the device, so every bounce is launched
+            const uint32_t step_blocks = static_cast<uint32_t>(std::min<size_t>((n + rt::kAovThreads - 1) / rt::kAovThreads,
+                                                                                static_cast<size_t>(d.sm_count) * 16));
+            for (uint32_t b = 0; b < depth; ++b) {
+                const rt::Queues q = queues_of(d, qdepth, static_cast<int>(b));
+                RT_K_EXTEND<<<d.extend_blocks, rt::kExtendThreads, 0, d.stream>>>(d.scene.scene, d.scene.light, d.scene.light_extra, inv_n_lights, d.scene.eps, q, b, 0x3F800000u);
+                rt::k_aov_step<<<step_blocks, rt::kAovThreads, 0, d.stream>>>(d.scene, d.lut.p, bp_key, q, b, slots);
+            }
+            rt::k_aov_accumulate<<<(bp.npix + 255) / 256, 256, 0, d.stream>>>(bp, slots, sums);
+            launches += 2 + 2 * static_cast<uint64_t>(depth);
         }
     }
     CU_CHECK(cudaGetLastError());
@@ -1237,6 +1339,7 @@ void rt_gpu_destroy(rt_gpu_ctx *ctx) {
         d.in_pos.release(); d.in_nrm.release(); d.in_uv.release(); d.in_tan.release(); d.in_mat.release(); d.build_scratch.release(); d.refit_scratch.release();
         d.counters.release(); d.stats.release();
         d.prim_ids.release(); d.rgb8.release(); d.cams.release();
+        d.aov_slots.release(); d.aov_sums.release(); d.aov_means.release();
         for (cudaEvent_t e : d.event_pool) cudaEventDestroy(e);
         for (cudaEvent_t e : {d.ev_begin, d.ev_end, d.ev_red0, d.ev_red1, d.ev_a, d.ev_b, d.ev_light, d.ev_round[0], d.ev_round[1]})
             if (e) cudaEventDestroy(e);
@@ -1729,6 +1832,79 @@ int rt_gpu_render_projected(rt_gpu_ctx *ctx, const rt_render_params *params, con
     if (!ctx || !params || !views || !projections) return fail(RT_ERR_INVALID_ARG, who + ": null argument");
     if (!ap) return render_views_checked(ctx, *params, *views, projections, who);
     return render_views_adaptive_checked(ctx, *params, *views, projections, *ap, who);
+}
+
+int rt_gpu_render_aov(rt_gpu_ctx *ctx, const rt_render_params *params, const rt_views *views, const rt_projection *projections) {
+    const std::string who = "rt_gpu_render_aov";
+    if (!ctx || !params) return fail(RT_ERR_INVALID_ARG, who + ": null argument");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, who + ": no scene uploaded");
+    if (ctx->text_scene) return fail(RT_ERR_INVALID_ARG, who + ": not available for course text scenes");
+    if (projections && !views) return fail(RT_ERR_INVALID_ARG, who + ": projections need views");
+    rt_render_params rp = *params;
+    if (rp.mode != RT_MODE_BEAUTY && rp.mode != RT_MODE_PRIMARY_IDS) return fail(RT_ERR_INVALID_ARG, who + ": unknown mode");
+    if (rp.sample_begin != 0 || rp.sample_end != 0)
+        return fail(RT_ERR_INVALID_ARG, who + ": the samples are [0, samples) (sample_begin / sample_end must be 0)");
+    if (rp.flags & RT_FLAG_ACCUMULATE) return fail(RT_ERR_INVALID_ARG, who + ": RT_FLAG_ACCUMULATE is not supported");
+    ViewSet vs;
+    if (views) {
+        if (int rc = check_views(rp, *views, who, vs)) return rc;
+        if (projections)
+            if (int rc = check_projections(projections, who, vs)) return rc;
+    } else if (rp.width == 0 || rp.height == 0 || static_cast<uint64_t>(rp.width) * rp.height > 0x7FFFFFFFull) {
+        return fail(RT_ERR_INVALID_ARG, who + ": illegal image size");
+    }
+    if (rp.mode == RT_MODE_BEAUTY && rp.samples == 0) return fail(RT_ERR_INVALID_ARG, who + ": samples == 0");
+    const uint64_t n_pixels = static_cast<uint64_t>(rp.width) * rp.height * (views ? views->n_views : 1u);
+    if (rp.pixel_end == 0) rp.pixel_end = static_cast<uint32_t>(n_pixels);
+    if (rp.pixel_begin > rp.pixel_end || rp.pixel_end > n_pixels) return fail(RT_ERR_INVALID_ARG, who + ": illegal pixel range");
+    // device 0 only, as RT_MODE_PRIMARY_IDS: the sums are its own
+    ctx->have_aov = false;
+    DeviceState &d = *ctx->devs[0];
+    uint64_t launches = 0;
+    if (int rc = enqueue_render_aov(d, rp, views ? &vs : nullptr, launches)) return rc;
+    CU_CHECK(cudaMemcpyAsync(d.h_stats, d.stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, d.stream));
+    CU_CHECK(cudaStreamSynchronize(d.stream));
+    rt_stats st;
+    std::memset(&st, 0, sizeof st);
+    float ms = 0.0f;
+    CU_CHECK(cudaEventElapsedTime(&ms, d.ev_begin, d.ev_end));
+    st.render_ms = ms;
+    st.extension_rays = d.h_stats[0];
+    st.samples = d.h_stats[3];
+    st.kernel_launches = launches;
+    ctx->aov_stats = st;
+    ctx->aov_last = rp;
+    ctx->aov_views = views ? views->n_views : 0u;
+    ctx->aov_samples = rp.mode == RT_MODE_PRIMARY_IDS ? 1u : rp.samples;
+    ctx->have_aov = true;
+    return RT_OK;
+}
+
+int rt_gpu_readback_aov(rt_gpu_ctx *ctx, float *albedo, float *normal, float *emission, float *depth, float *coverage, rt_stats *stats) {
+    const std::string who = "rt_gpu_readback_aov";
+    if (!ctx) return fail(RT_ERR_INVALID_ARG, who + ": null handle");
+    if (!ctx->have_aov) return fail(RT_ERR_NO_RENDER, who + ": no AOV render on this handle");
+    DeviceState &d = *ctx->devs[0];
+    CU_CHECK(cudaSetDevice(d.device));
+    const size_t n = static_cast<size_t>(ctx->aov_last.width) * ctx->aov_last.height * std::max(ctx->aov_views, 1u);
+    if (albedo || normal || emission || depth || coverage) {
+        if (int rc = d.aov_means.alloc(11 * n)) return rc;
+        const rt::AovPlanes sums{d.aov_sums.p, d.aov_sums.p + n, d.aov_sums.p + 2 * n};
+        const uint32_t n32 = static_cast<uint32_t>(n);
+        rt::k_aov_means<<<(n32 + 255) / 256, 256, 0, d.stream>>>(sums, static_cast<float>(ctx->aov_samples), n32, d.aov_means.p);
+        CU_CHECK(cudaGetLastError());
+        const float *m = d.aov_means.p;
+        const struct {
+            float *dst;
+            const float *src;
+            size_t count;
+        } parts[5] = {{albedo, m, 3 * n}, {normal, m + 3 * n, 3 * n}, {emission, m + 6 * n, 3 * n}, {depth, m + 9 * n, n}, {coverage, m + 10 * n, n}};
+        for (const auto &part : parts)
+            if (part.dst) CU_CHECK(cudaMemcpyAsync(part.dst, part.src, part.count * sizeof(float), cudaMemcpyDeviceToHost, d.stream));
+        CU_CHECK(cudaStreamSynchronize(d.stream));
+    }
+    if (stats) *stats = ctx->aov_stats;
+    return RT_OK;
 }
 
 int rt_gpu_readback_adaptive(rt_gpu_ctx *ctx, uint32_t *sample_counts, float *rel_error) {

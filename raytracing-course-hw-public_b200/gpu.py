@@ -17,7 +17,7 @@ SYMBOLS = ["rt_gpu_create", "rt_gpu_destroy", "rt_gpu_upload_scene", "rt_gpu_upl
            "rt_gpu_accum_device_ptr", "rt_gpu_readback_rgb8", "rt_gpu_set_profiling", "rt_gpu_debug_get_bvh", "rt_gpu_fp32_peak", "rt_gpu_last_error",
            "rt_gpu_device_count", "rt_gpu_abi_version", "rt_gpu_render_adaptive", "rt_gpu_readback_adaptive",
            "rt_gpu_render_views", "rt_gpu_render_views_adaptive", "rt_gpu_render_projected", "rt_gpu_update_geometry",
-           "rt_gpu_debug_light_pdf"]
+           "rt_gpu_debug_light_pdf", "rt_gpu_render_aov", "rt_gpu_readback_aov"]
 
 _lib = None
 
@@ -47,6 +47,8 @@ def lib():
         L.rt_gpu_debug_get_bvh.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_size_t)]
         L.rt_gpu_fp32_peak.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
         L.rt_gpu_debug_light_pdf.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+        L.rt_gpu_render_aov.argtypes = [C.c_void_p, C.POINTER(rt_render_params), C.POINTER(rt_views), C.POINTER(rt_projection)]
+        L.rt_gpu_readback_aov.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_gpu_last_error.restype = C.c_char_p
         _lib = L
     return _lib
@@ -76,6 +78,7 @@ class RtGpu:
         self._scene = None
         self._last = None
         self._views = None  # views of the last render when it was render_views: readbacks are [V, H, W, ...]
+        self._aov = None  # (width, height, views or None) of the last render_aov
 
     def close(self):
         if self._h:
@@ -184,6 +187,47 @@ class RtGpu:
         _check(lib().rt_gpu_render_projected(self._h, C.byref(p), C.byref(v), projs, a), "rt_gpu_render_projected")
         self._last = (width, height, mode)
         self._views = len(cameras)
+
+    def render_aov(self, width, height, samples, seed=0, cameras=None, projections=None, view_base=0, centre=False, pixel_begin=0,
+                   pixel_end=0, max_paths_in_flight=0):
+        """AOV render (rt_gpu_render_aov): per-pixel albedo, shading normal, emission, depth and coverage of the visible
+        surface of the camera samples [0, samples) that render / render_views / render_projected trace for the same
+        arguments (cameras=None: the scene camera; projections needs cameras).  centre=True takes the pixel-centre rays
+        of primary_ids instead (one sample, the whole image).  readback_aov() returns the means over all samples."""
+        if projections is not None and cameras is None:
+            raise ValueError("render_aov: projections need cameras")
+        if projections is not None and len(projections) != len(cameras):
+            raise ValueError(f"render_aov: {len(cameras)} cameras but {len(projections)} projections")
+        p = rt_render_params(width, height, samples, 0, 0, RT_MODE_PRIMARY_IDS if centre else RT_MODE_BEAUTY, seed, max_paths_in_flight,
+                             0, pixel_begin, pixel_end)
+        v = projs = None
+        if cameras is not None:
+            cams = (rt_camera * max(len(cameras), 1))(*[c.to_c() for c in cameras])
+            v = rt_views(len(cameras), view_base, cams)
+            v._cams = cams
+        if projections is not None:
+            projs = (rt_projection * max(len(projections), 1))(*[pj.to_c() for pj in projections])
+        _check(lib().rt_gpu_render_aov(self._h, C.byref(p), None if v is None else C.byref(v), projs), "rt_gpu_render_aov")
+        self._aov = (width, height, None if cameras is None else len(cameras))
+
+    def readback_aov(self):
+        """The last render_aov's means as float32 arrays: albedo, normal and emission [H, W, 3], depth and coverage [H, W]
+        ([V, H, W, ...] with cameras).  aov_stats() has its counters."""
+        if self._aov is None:  # the library's own RT_ERR_NO_RENDER
+            _check(lib().rt_gpu_readback_aov(self._h, None, None, None, None, None, None), "rt_gpu_readback_aov")
+        w, h, views = self._aov
+        lead = ((views,) if views is not None else ()) + (h, w)
+        out = {k: np.zeros(lead + (3,), np.float32) for k in ("albedo", "normal", "emission")}
+        out.update({k: np.zeros(lead, np.float32) for k in ("depth", "coverage")})
+        ptr = [out[k].ctypes.data_as(C.c_void_p) for k in ("albedo", "normal", "emission", "depth", "coverage")]
+        _check(lib().rt_gpu_readback_aov(self._h, *ptr, None), "rt_gpu_readback_aov")
+        return out
+
+    def aov_stats(self):
+        """Stats dict of the last render_aov: samples, extension rays, kernel launches, render_ms."""
+        st = rt_stats()
+        _check(lib().rt_gpu_readback_aov(self._h, None, None, None, None, None, C.byref(st)), "rt_gpu_readback_aov")
+        return st.as_dict()
 
     def readback_adaptive(self):
         """(sample counts uint32 [H, W], err float32 [H, W]) of the last adaptive render; [V, H, W] each after

@@ -25,6 +25,8 @@
 //             the maximum spp, min_samples = step_samples = max(2, ceil(samples / 16)); the samples traced on stderr
 //   RT_PROJECTION  projection of the scene camera (rt_gpu_render_projected, glTF scenes): thin_lens:<aperture>:<focus>,
 //             ortho:<half_w>:<half_h>, equirect or pinhole; combines with RT_ADAPTIVE
+//   RT_AOV    samples per pixel of an AOV render after the beauty render (rt_gpu_render_aov, glTF scenes; same camera,
+//             RT_PROJECTION and seed): <stem>_albedo.pfm, _normal, _emission, _depth and _coverage (aov_out.hpp)
 #define STB_IMAGE_IMPLEMENTATION
 
 #include <algorithm>
@@ -45,6 +47,7 @@
 #include "raytracer.h"
 #include "scene.h"
 
+#include "aov_out.hpp"
 #include "flatten_ref.hpp"
 #include "rt_gpu.h"
 #include "rt_host.h"
@@ -149,6 +152,7 @@ void write_image(Image &img, const char *path) {
 
 // course text scene: parser in librt_host, megakernel behind rt_gpu_upload_text_scene
 int run_text_scene(const char *path, unsigned width, unsigned height, unsigned samples, const char *out_path) {
+    if (rt_aov::parse_samples(std::getenv("RT_AOV"))) throw std::runtime_error("RT_AOV applies to glTF scenes only");
     rt_text_scene *ts = nullptr;
     if (int rc = rt_text_scene_parse(path, &ts))
         throw std::runtime_error(std::string("cannot parse text scene ") + path + " (" + std::to_string(rc) + ")");
@@ -180,6 +184,7 @@ int main(int argc, char **argv) try {
 
     if (std::filesystem::path(argv[1]).extension() == ".txt") return run_text_scene(argv[1], width, height, samples, argv[5]);
 
+    const unsigned aov_samples = rt_aov::parse_samples(std::getenv("RT_AOV"));  // refused before any work when malformed
     PhaseClock clock;
     Scene scene = parse_gltf_scene(std::filesystem::path(argv[1]), static_cast<float>(width) / height);
     clock.lap("parse_gltf_scene");
@@ -218,10 +223,20 @@ int main(int argc, char **argv) try {
         clock.lap("rt_gpu_upload_scene");
         render_into(gpu, width, height, samples, img, &flat.desc.camera);
         clock.lap("render + readback + set_pixel");
+        if (aov_samples) {  // RT_PROJECTION was validated by render_into
+            const char *projection = std::getenv("RT_PROJECTION");
+            rt_projection proj{};
+            const bool projected = projection && *projection && parse_projection(projection, proj);
+            rt_aov::render_and_write(gpu, width, height, aov_samples, env_uint("RT_SEED", 0), env_uint("RT_PATHS", 128u << 20), &flat.desc.camera,
+                                     projected ? &proj : nullptr, argv[5]);
+            clock.lap("AOV render + PFMs");
+        }
         rt_gpu_destroy(gpu);
         clock.lap("rt_gpu_destroy");
     }
 
+    if (scene.ray_depth == 0 && aov_samples)  // nothing is rendered: the buffers are 0
+        rt_aov::render_and_write(nullptr, width, height, aov_samples, 0, 0, nullptr, nullptr, argv[5]);
     write_image(img, argv[5]);
     clock.lap("Image::write");
     return EXIT_SUCCESS;
